@@ -52,7 +52,36 @@ def parse_args():
     ap.add_argument("--gather", default="peer", choices=["peer", "nccl"],
                     help="N > 1: 'peer' = every rank stores its final pixels straight into rank 0's frame over NVLink (CUDA IPC "
                          "mapping, the gather is fused into the last accumulate kernel); 'nccl' = shard buffers + one NCCL gather + de-interleave")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the frame of the last one to DIR as .npy (a fixed, seeded sample of its "
+                         "pixels when the whole frame exceeds 64 MB), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the frame of the GPU path; the reference arm has none")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory, frame, counts):
+    """frame: the H x W x 4 float32 frame of the last timed step (what a caller of RaylibB200_RenderShardToFrame receives);
+    counts: that frame's ray queries and pixel samples, summed over all ranks.  Frames above DUMP_LIMIT_BYTES are written
+    as the pixels at fixed indices drawn from a seeded generator (frame_pixel_index.npy, row-major pixel numbers, float64
+    holds them exactly)."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    pixels = frame.reshape(-1, frame.shape[-1])
+    if frame.nbytes <= DUMP_LIMIT_BYTES:
+        np.save(os.path.join(directory, "frame.npy"), frame.astype(np.float32))
+    else:
+        k = DUMP_LIMIT_BYTES // 2 // (pixels.shape[1] * 4 + 8)
+        idx = np.sort(np.random.default_rng(1337).choice(len(pixels), size=k, replace=False))
+        np.save(os.path.join(directory, "frame_pixels.npy"), pixels[idx].astype(np.float32))
+        np.save(os.path.join(directory, "frame_pixel_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(directory, "ray_queries_pixel_samples.npy"), np.asarray(counts, dtype=np.float64))
 
 
 class ClockSampler:
@@ -381,6 +410,19 @@ def main_b200(args):
         sampler.start()
     total_ms, stats = timed(step_device, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        last_counts = torch.tensor([stats[-1].rayQueries, stats[-1].pixelSamples], dtype=torch.float64, device="cuda")
+        if distributed:
+            dist.all_reduce(last_counts, op=dist.ReduceOp.SUM)
+    if args.dump_outputs and rank == 0:
+        if gather == "peer":
+            if not prod.lib.RaylibB200_FrameRead(frame, W, H, host_image.data_ptr(), stream):
+                raise RuntimeError("RaylibB200_FrameRead failed: " + prod.last_error())
+            torch.cuda.synchronize()
+            last_frame = host_image.numpy()
+        else:
+            last_frame = image.cpu().numpy()
+        dump_outputs(args.dump_outputs, last_frame, last_counts.tolist())
 
     counts = torch.tensor([sum(s.rayQueries for s in stats), sum(s.pixelSamples for s in stats),
                            sum(s.kernelLaunches for s in stats) + (args.steps if (rank == 0 and gather == "nccl") else 0)],

@@ -153,11 +153,14 @@ class Restatement:
         self.lib.rt_oracle_trace(desc, rays, len(rays), t_min, rank, t, C.byref(counts))
         return rank, t, list(counts)
 
-    def primary(self, desc, cam, width, height, t_min, seed=1337, rows=None):
+    def primary(self, desc, cam, width, height, t_min, seed=1337, rows=None, want_rays=False):
+        """want_rays: also return the n x 8 camera rays (bit-identical to the compiled reference's, tests/golden)."""
         n = width * height
         rank = np.full(n, -2, dtype=np.int32)
         t = np.zeros(n, dtype=np.float32)
+        rays = np.zeros((n, 8), dtype=np.float32) if want_rays else None
         counts = (C.c_uint64 * 4)()
         y0, y1 = rows if rows else (0, height)
-        self.lib.rt_oracle_primary(desc, C.byref(cam), width, height, y0, y1, t_min, seed, rank, t, None, C.byref(counts))
-        return rank, t, list(counts)
+        self.lib.rt_oracle_primary(desc, C.byref(cam), width, height, y0, y1, t_min, seed, rank, t,
+                                   rays.ctypes.data if want_rays else None, C.byref(counts))
+        return (rank, t, list(counts), rays) if want_rays else (rank, t, list(counts))

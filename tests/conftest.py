@@ -1,5 +1,8 @@
+import hashlib
 import os
+import re
 import sys
+import zlib
 import numpy as np
 import pytest
 
@@ -52,6 +55,50 @@ def ref(rl):
 def restate(rl):
     from oracle import bindings as ob
     return ob.Restatement()
+
+
+class RecordedOutputs:
+    """Stored outputs for the tests that compared the product with the compiled reference (oracle/_ref), so that they run
+    where the reference cannot be built: tests/golden/recorded/<test>.npz.  The reference's own outputs for these inputs
+    are not available, so what is stored is this library's output at the last commit that ran the same GPU tests against
+    the compiled reference and passed them within their bars (profiles/r02fin_tests.log); an earlier run of them printed
+    the radiance and debug-view comparisons bit-identical (profiles/r02z_tests.log).  The CPU tests' answers are those of
+    the restatement and the host library at that commit, which those tests held bit-identical to the compiled reference.
+    The tests hold the product to the stored outputs with the bars they held it to against the reference.  In the GPU
+    tests primary hits and traced rays are not stored: they are compared with the C restatement (oracle/rt_oracle.c,
+    pinned to the reference by tests/golden/config*.npz).
+
+    An array is kept as the SHA-256 of its bytes plus its elements (pixels, rays) at up to SAMPLE positions drawn by a
+    generator seeded from the key: the digest decides bit-for-bit equality of the whole array, the sample carries the
+    fraction / PSNR / outlier bars."""
+    SAMPLE = 1024
+
+    def __init__(self, path):
+        self.data = dict(np.load(path))
+
+    def sample(self, key, a):
+        """The elements of `a` at the positions `compare` draws for `key`."""
+        a = np.ascontiguousarray(a)
+        flat = a.reshape(-1, a.shape[-1]) if a.ndim == 3 else a
+        rng = np.random.default_rng([len(flat), zlib.crc32(key.encode())])
+        idx = np.sort(rng.choice(len(flat), size=min(len(flat), self.SAMPLE), replace=False))
+        return flat[idx][:, None] if a.ndim == 3 else flat[idx]
+
+    def compare(self, key, got):
+        """-> (sample of `got`, the stored sample at the same positions, whole array bit-identical to the stored one).
+        Image samples are shaped K x 1 x C, so the per-pixel reductions over axis 2 apply to them unchanged."""
+        digest = hashlib.sha256(np.ascontiguousarray(got).tobytes()).hexdigest()
+        return self.sample(key, got), self.data[key + "/sample"], digest == str(self.data[key + "/sha256"])
+
+    def value(self, key):
+        """A stored scalar or short vector (a ray count, scene sizes)."""
+        return self.data[key]
+
+
+@pytest.fixture
+def recorded(request):
+    name = re.sub(r"[^A-Za-z0-9_.-]+", "_", "%s.%s" % (request.module.__name__, request.node.name)).strip("_")
+    return RecordedOutputs(os.path.join(GOLDEN, "recorded", name + ".npz"))
 
 
 def load_golden(cfg):

@@ -1,7 +1,8 @@
 """GPU parity tests: every call goes through the C ABI of libraylib_b200.so (pyraylib is a ctypes shim).
 
-Oracle = tests/golden (vectors generated from the compiled reference) and, where it travelled with the
-repository, the compiled reference itself (oracle/_ref).
+Oracle = tests/golden (vectors generated from the compiled reference), the C restatement (oracle/rt_oracle.c, pinned to
+those vectors) for primary hits and traced rays, and tests/golden/recorded for the outputs the compiled reference is no
+longer at hand to produce (see conftest.RecordedOutputs).
 
 Bars (north star):
   * primary rays: hit primitive ids identical to the reference; t bit-identical when the lens is a pinhole
@@ -105,23 +106,35 @@ def test_debug_views_match_golden(gpu, cfg):
         gpu.destroy_demo(info)
 
 
-def test_against_compiled_reference_fresh_inputs(gpu, ref, rl):
-    """Sizes/seeds that are NOT in the golden set, straight against the compiled reference."""
+def restated_primary(gpu, restate, info, seed=1337, scene=None):
+    """Primary hits (rank, t) and camera rays of the C restatement (oracle/rt_oracle.c) for a demo scene's camera.  On the
+    golden inputs its rays, ids and t are the compiled reference's bit for bit (tests/test_cpu_oracle.py); on other
+    inputs it is an independent exhaustive implementation, and the device must trace the same rays to the same hits."""
+    s = info.settings
+    rank, t, _, rays = restate.primary(gpu.flat_desc(scene or info.scene), gpu.camera_block(info.camera), s.viewportWidth,
+                                       s.viewportHeight, s.rayTMin, seed=seed, want_rays=True)
+    return rank, t, rays
+
+
+def test_against_compiled_reference_fresh_inputs(gpu, recorded, restate, rl):
+    """Sizes/seeds that are NOT in the golden set: camera rays through the device traversal against the C restatement,
+    radiance against the stored outputs (conftest.RecordedOutputs)."""
     for cfg, size, (w, h), spp, seed in [(3, 96, (200, 120), 3, 99), (4, 40, (128, 128), 2, 7), (6, 0, (111, 77), 5, 2024)]:
-        pinfo, rinfo = gpu.create_demo(cfg, size), ref.create_demo(cfg, size)
+        pinfo = gpu.create_demo(cfg, size)
+        key = "config%d_" % cfg
         try:
-            gpu.set_viewport(pinfo, w, h); ref.set_viewport(rinfo, w, h)
+            gpu.set_viewport(pinfo, w, h)
             gpu.lib.RaylibB200_SetFrameSeed(seed)
-            rr, rt, rays, _ = ref.primary_hits(rinfo.settings, rinfo.scene, rinfo.camera, seed=seed, want_rays=True)
+            rr, rt, rays = restated_primary(gpu, restate, pinfo, seed)
             gr, gt = gpu.trace_rays(pinfo.scene, rays, pinfo.settings.rayTMin)
             assert np.array_equal(gr, rr) and np.array_equal(bits(gt), bits(rt))
-            rimg, rst = ref.render_deterministic(rinfo.settings.copy(samplesPerPixel=spp), rinfo.scene, rinfo.camera, seed=seed)
             gimg = gpu.render(pinfo.settings.copy(samplesPerPixel=spp), pinfo.scene, pinfo.camera)
-            assert rl.psnr(gimg, rimg) >= 40.0 and rel_outliers(gimg, rimg) <= 0.02
-            assert float((bits(gimg) == bits(rimg)).all(axis=2).mean()) >= EXACT_FLOOR
+            g, r, _ = recorded.compare(key + "radiance", gimg)
+            assert rl.psnr(g, r) >= 40.0 and rel_outliers(g, r) <= 0.02
+            assert float((bits(g) == bits(r)).all(axis=2).mean()) >= EXACT_FLOOR
         finally:
             gpu.lib.RaylibB200_SetFrameSeed(1337)
-            gpu.destroy_demo(pinfo); ref.destroy_demo(rinfo)
+            gpu.destroy_demo(pinfo)
 
 
 def test_incoherent_rays_against_restatement(gpu, restate):
@@ -397,17 +410,17 @@ def test_adversarial_rays_against_restatement(gpu, restate, cfg, size):
         gpu.destroy_demo(info)
 
 
-def test_full_size_scatter10M_against_compiled_reference(gpu, ref, rl):
+def test_full_size_scatter10M_against_compiled_reference(gpu, recorded, restate, rl):
     """The headline workload at FULL scene size (9,999,362 triangles, 7812 meshes, two-level BVH, 8 materials, sun + sky):
-    primary-hit ids / t against the compiled reference, the reference's own camera rays through the device traversal,
-    radiance at matched spp and seed, and shard-count independence of the device frame."""
+    primary-hit ids / t and the camera rays through the device traversal against the C restatement, radiance at matched
+    spp and seed against the stored outputs (conftest.RecordedOutputs), and shard-count independence of the device frame."""
     import torch
-    pinfo, rinfo = gpu.create_demo(4, 0), ref.create_demo(4, 0)
+    pinfo = gpu.create_demo(4, 0)
     try:
         W, H = 640, 360
-        gpu.set_viewport(pinfo, W, H); ref.set_viewport(rinfo, W, H)
-        rr, rt, rays, _ = ref.primary_hits(rinfo.settings, rinfo.scene, rinfo.camera, want_rays=True)
+        gpu.set_viewport(pinfo, W, H)
         gr, gt = gpu.primary_hits(pinfo.settings, pinfo.scene, pinfo.camera)
+        rr, rt, rays = restated_primary(gpu, restate, pinfo)
         print("scatter10M primary: id match %.6f, t bit match %.6f, hit fraction %.3f"
               % (float((gr == rr).mean()), float((bits(gt) == bits(rt)).mean()), float((rr >= 0).mean())))
         assert np.array_equal(gr, rr) and np.array_equal(bits(gt), bits(rt))          # pinhole camera: exact
@@ -415,14 +428,15 @@ def test_full_size_scatter10M_against_compiled_reference(gpu, ref, rl):
         assert np.array_equal(gr2, rr) and np.array_equal(bits(gt2), bits(rt))
         # radiance, 2 spp, depth 8
         s = pinfo.settings.copy(samplesPerPixel=2)
-        rimg, rst = ref.render_deterministic(rinfo.settings.copy(samplesPerPixel=2), rinfo.scene, rinfo.camera)
         gimg = gpu.render(s, pinfo.scene, pinfo.camera)
         st = gpu.last_stats()
-        psnr, out = rl.psnr(gimg, rimg), rel_outliers(gimg, rimg)
-        exact = float((bits(gimg) == bits(rimg)).all(axis=2).mean())
-        print("scatter10M radiance: PSNR %.2f dB, outliers %.4f, bit-identical pixels %.4f, rays %d vs %d" % (psnr, out, exact, st.rayQueries, rst.rayQueries))
+        g, r, _ = recorded.compare("radiance", gimg)
+        rays = int(recorded.value("radiance_rays"))
+        psnr, out = rl.psnr(g, r), rel_outliers(g, r)
+        exact = float((bits(g) == bits(r)).all(axis=2).mean())
+        print("scatter10M radiance (sample): PSNR %.2f dB, outliers %.4f, bit-identical pixels %.4f, rays %d vs %d" % (psnr, out, exact, st.rayQueries, rays))
         assert psnr >= 40.0 and out <= 0.02 and exact >= EXACT_FLOOR
-        assert abs(int(st.rayQueries) - int(rst.rayQueries)) <= 0.002 * int(rst.rayQueries) + 8
+        assert abs(int(st.rayQueries) - rays) <= 0.002 * rays + 8
         # 1 shard vs 8 shards, bit-identical
         cap = int(gpu.lib.RaylibB200_ShardPixelCapacity(W, H, 8))
         slabs = torch.zeros((8 * cap, 4), dtype=torch.float32, device="cuda")
@@ -432,7 +446,7 @@ def test_full_size_scatter10M_against_compiled_reference(gpu, ref, rl):
         assert gpu.lib.RaylibB200_AssembleShards(slabs.data_ptr(), 8, W, H, image.data_ptr(), None)
         assert np.array_equal(bits(image.cpu().numpy()[:, :, :3]), bits(gimg))
     finally:
-        gpu.destroy_demo(pinfo); ref.destroy_demo(rinfo)
+        gpu.destroy_demo(pinfo)
 
 
 def test_pipes_do_not_change_the_image(gpu):
@@ -555,44 +569,46 @@ def test_flattened_scene_cache_renders_identically(gpu, tmp_path):
 
 
 @pytest.mark.parametrize("cfg,name,psnr_floor", [(3, "grid1M", 60.0), (5, "textured2M", 40.0)])
-def test_full_size_scenes_against_compiled_reference(gpu, ref, rl, cfg, name, psnr_floor):
+def test_full_size_scenes_against_compiled_reference(gpu, recorded, restate, rl, cfg, name, psnr_floor):
     """BASELINE configurations 3 (1,002,528-triangle displaced grid, primary + AO) and 5 (~2 M textured microfacet
-    triangles with alpha cut-outs, mirror / dielectric / metal objects) at FULL scene size against the compiled
-    reference: primary-hit ids and t, the SurfaceNormal view (README "VertexNormal"), radiance at matched spp and seed."""
-    pinfo, rinfo = gpu.create_demo(cfg, 0), ref.create_demo(cfg, 0)
+    triangles with alpha cut-outs, mirror / dielectric / metal objects) at FULL scene size: primary-hit ids and t against
+    the C restatement; the SurfaceNormal view (README "VertexNormal") and radiance at matched spp and seed against the
+    stored outputs (conftest.RecordedOutputs)."""
+    pinfo = gpu.create_demo(cfg, 0)
     try:
         W, H = 480, 270
-        gpu.set_viewport(pinfo, W, H); ref.set_viewport(rinfo, W, H)
-        rr, rt, rays, _ = ref.primary_hits(rinfo.settings, rinfo.scene, rinfo.camera, want_rays=True)
+        gpu.set_viewport(pinfo, W, H)
         gr, gt = gpu.primary_hits(pinfo.settings, pinfo.scene, pinfo.camera)
+        rr, rt, rays = restated_primary(gpu, restate, pinfo)
         idm, tm = float((gr == rr).mean()), float((bits(gt) == bits(rt)).mean())
         print("%s primary: id match %.6f, t bit match %.6f, hit fraction %.3f" % (name, idm, tm, float((rr >= 0).mean())))
         assert np.array_equal(gr, rr) and np.array_equal(bits(gt), bits(rt))          # pinhole cameras: exact
         gr2, gt2 = gpu.trace_rays(pinfo.scene, rays, pinfo.settings.rayTMin)
         assert np.array_equal(gr2, rr) and np.array_equal(bits(gt2), bits(rt))
         # SurfaceNormal debug view: bit-identical (triangles only, no transcendental on the way)
-        rn, _ = ref.render_deterministic(rinfo.settings.copy(renderMode=2), rinfo.scene, rinfo.camera)
         gn = gpu.render(pinfo.settings.copy(renderMode=2), pinfo.scene, pinfo.camera)
-        assert np.array_equal(bits(gn), bits(rn))
+        assert recorded.compare("normal_view", gn)[2]
         # radiance, 2 spp at the configuration's own depth
         s = pinfo.settings.copy(samplesPerPixel=2)
-        rimg, rst = ref.render_deterministic(rinfo.settings.copy(samplesPerPixel=2), rinfo.scene, rinfo.camera)
         gimg = gpu.render(s, pinfo.scene, pinfo.camera)
         st = gpu.last_stats()
-        psnr, out = rl.psnr(gimg, rimg), rel_outliers(gimg, rimg)
-        exact = float((bits(gimg) == bits(rimg)).all(axis=2).mean())
-        print("%s radiance: PSNR %.2f dB, outliers %.4f, bit-identical pixels %.4f, rays %d vs %d" % (name, psnr, out, exact, st.rayQueries, rst.rayQueries))
+        g, r, _ = recorded.compare("radiance", gimg)
+        rays = int(recorded.value("radiance_rays"))
+        psnr, out = rl.psnr(g, r), rel_outliers(g, r)
+        exact = float((bits(g) == bits(r)).all(axis=2).mean())
+        print("%s radiance (sample): PSNR %.2f dB, outliers %.4f, bit-identical pixels %.4f, rays %d vs %d" % (name, psnr, out, exact, st.rayQueries, rays))
         assert psnr >= psnr_floor and out <= 0.02 and exact >= EXACT_FLOOR
-        assert abs(int(st.rayQueries) - int(rst.rayQueries)) <= 0.002 * int(rst.rayQueries) + 8
+        assert abs(int(st.rayQueries) - rays) <= 0.002 * rays + 8
     finally:
-        gpu.destroy_demo(pinfo); ref.destroy_demo(rinfo)
+        gpu.destroy_demo(pinfo)
 
 
 # ---- round 2: comparisons that used to be self-comparisons, now against the compiled reference ---------------------
 
-def test_gpu_postprocess_vs_compiled_reference(gpu, ref):
+def test_gpu_postprocess_vs_compiled_reference(gpu, recorded):
     """SURVEY 8(f) rank 3 against the ORACLE: the same HDR frame through the reference's own Raylib_PostProcess
-    (render/image.cc:44-103, compiled unmodified) and through RaylibB200_PostProcessGPU / _PostProcessDevice."""
+    (render/image.cc:44-103, compiled unmodified; its output is stored, see conftest.RecordedOutputs) and through
+    RaylibB200_PostProcessGPU / _PostProcessDevice."""
     import torch
     info = gpu.create_demo(2, 0)            # Cornell box: the light (15) is far above white
     try:
@@ -610,10 +626,11 @@ def test_gpu_postprocess_vs_compiled_reference(gpu, ref):
         finally:
             gpu.lib.Raylib_DestroyImage(img)
         assert raw[..., :3].max() > 1.0, "the test frame must exercise the max-white reduction"
-        want = ref.postprocess_rgba(raw)
+        assert recorded.compare("input", raw)[2], "the rendered input frame is not the one the reference post-processed"
+        out, want, _ = recorded.compare("postprocess", out)
         # identical arithmetic except powf (device libm vs glibc): report how many pixels are bit-identical
         exact = float((bits(out) == bits(want)).all(axis=2).mean())
-        print("GPU post-process vs reference: bit-identical pixels %.4f, max abs diff %.3g" % (exact, float(np.abs(out - want).max())))
+        print("GPU post-process vs reference (sample): bit-identical pixels %.4f, max abs diff %.3g" % (exact, float(np.abs(out - want).max())))
         assert np.allclose(out, want, rtol=2e-6, atol=1e-7)
         assert exact >= EXACT_FLOOR
         # device-resident form with the packed 8-bit output (Pixel::ToUint32, image.h:57-64)
@@ -621,8 +638,8 @@ def test_gpu_postprocess_vs_compiled_reference(gpu, ref):
         packed = torch.zeros((H, W), dtype=torch.int32, device="cuda")
         mw = C.c_float(0.0)
         assert gpu.lib.RaylibB200_PostProcessDevice(dev.data_ptr(), W, H, packed.data_ptr(), C.byref(mw), None), gpu.last_error()
-        assert np.allclose(dev.cpu().numpy(), want, rtol=2e-6, atol=1e-7)
-        p = packed.cpu().numpy().view(np.uint32)
+        assert np.allclose(recorded.sample("postprocess", dev.cpu().numpy()), want, rtol=2e-6, atol=1e-7)
+        p = recorded.sample("postprocess", packed.cpu().numpy()[..., None])[..., 0].view(np.uint32)
         w8 = (want * 255.0).astype(np.uint32) & 0xff
         expect = (w8[..., 3] << 24) | (w8[..., 0] << 16) | (w8[..., 1] << 8) | w8[..., 2]
         assert (p == expect).mean() >= 0.99 and np.abs(((p >> 8) & 0xff).astype(np.int32) - w8[..., 1].astype(np.int32)).max() <= 1
@@ -631,23 +648,23 @@ def test_gpu_postprocess_vs_compiled_reference(gpu, ref):
 
 
 @pytest.mark.parametrize("cfg,size", [(5, 40), (6, 0), (2, 0)])
-def test_microsurface_normal_and_reflectance_views_vs_compiled_reference(gpu, ref, cfg, size):
+def test_microsurface_normal_and_reflectance_views_vs_compiled_reference(gpu, recorded, cfg, size):
     """Render modes 3 (MicrosurfaceNormal) and 6 (Reflectance) -- deterministic in the reference after all: the debug path
     never builds the tangent frame, but a default-constructed HitResult holds ZERO tangent / bitangent (vec3() = 0,
     core/vec3.h:16), so mode 3 shows N.z * n and mode 6 scatters on the zero frame.  Also the normal half of
-    RaylibB200_RenderAux (SURVEY 8f rank 2), which is the same pass."""
-    pinfo, rinfo = gpu.create_demo(cfg, size), ref.create_demo(cfg, size)
+    RaylibB200_RenderAux (SURVEY 8f rank 2), which is the same pass.  Views compared with the stored outputs (conftest.RecordedOutputs)."""
+    pinfo = gpu.create_demo(cfg, size)
     try:
         W, H = 240, 136
-        gpu.set_viewport(pinfo, W, H); ref.set_viewport(rinfo, W, H)
+        gpu.set_viewport(pinfo, W, H)
         for mode in (3, 6):
             gimg = gpu.render(pinfo.settings.copy(renderMode=mode), pinfo.scene, pinfo.camera)
-            rimg, _ = ref.render_deterministic(rinfo.settings.copy(renderMode=mode), rinfo.scene, rinfo.camera)
-            exact = float((bits(gimg) == bits(rimg)).all(axis=2).mean())
-            close = float(np.isclose(gimg, rimg, rtol=1e-4, atol=2e-3).all(axis=2).mean())
-            print("config%d mode %d vs reference: bit-identical %.4f, close %.4f" % (cfg, mode, exact, close))
+            g, r, same = recorded.compare("mode%d" % mode, gimg)
+            exact = float((bits(g) == bits(r)).all(axis=2).mean())
+            close = float(np.isclose(g, r, rtol=1e-4, atol=2e-3).all(axis=2).mean())
+            print("config%d mode %d vs reference (sample): bit-identical %.4f, close %.4f" % (cfg, mode, exact, close))
             if cfg in PINHOLE:
-                assert exact == 1.0 if mode == 3 else exact >= EXACT_FLOOR
+                assert same if mode == 3 else exact >= EXACT_FLOOR
             else:
                 assert exact >= 0.98 and close >= 0.98      # a finite aperture can move a silhouette pixel onto another primitive
         a_img, n_img = gpu.lib.Raylib_CreateImage(W, H), gpu.lib.Raylib_CreateImage(W, H)
@@ -656,82 +673,79 @@ def test_microsurface_normal_and_reflectance_views_vs_compiled_reference(gpu, re
             aux_a, aux_n = gpu.dump_image(a_img, W, H), gpu.dump_image(n_img, W, H)
         finally:
             gpu.lib.Raylib_DestroyImage(a_img); gpu.lib.Raylib_DestroyImage(n_img)
-        ralb, _ = ref.render_deterministic(rinfo.settings.copy(renderMode=1), rinfo.scene, rinfo.camera)
-        rnrm, _ = ref.render_deterministic(rinfo.settings.copy(renderMode=3), rinfo.scene, rinfo.camera)
         if cfg in PINHOLE:
-            assert np.array_equal(bits(aux_a), bits(ralb)) and np.array_equal(bits(aux_n), bits(rnrm))
+            assert recorded.compare("mode1", aux_a)[2] and recorded.compare("mode3", aux_n)[2]
         else:
-            assert (bits(aux_n) == bits(rnrm)).all(axis=2).mean() >= 0.85
+            g, r, _ = recorded.compare("mode3", aux_n)
+            assert (bits(g) == bits(r)).all(axis=2).mean() >= 0.85
     finally:
-        gpu.destroy_demo(pinfo); ref.destroy_demo(rinfo)
+        gpu.destroy_demo(pinfo)
 
 
 @pytest.mark.parametrize("cfg,size", [(5, 40), (6, 0), (4, 24)])
-def test_shallow_paths_vs_compiled_reference(gpu, ref, rl, cfg, size):
+def test_shallow_paths_vs_compiled_reference(gpu, recorded, rl, cfg, size):
     """Where does the radiance start to differ?  maxPathLength 1 (emission + sky + sun visibility of the camera ray; no
     scattered direction is ever used) must be bit-identical on (nearly) every pixel; maxPathLength 2 adds ONE scattered ray
     whose direction went through sinf/cosf/powf on the device instead of glibc -- values agree to float rounding.  Deeper
     paths only amplify those last-bit differences (specular chains), which is what the 40 dB bar of the full-depth tests
-    absorbs; a first-bounce disagreement would show up here."""
-    pinfo, rinfo = gpu.create_demo(cfg, size), ref.create_demo(cfg, size)
+    absorbs; a first-bounce disagreement would show up here.  Frames compared with the stored outputs (conftest.RecordedOutputs)."""
+    pinfo = gpu.create_demo(cfg, size)
     try:
         W, H = 256, 144
-        gpu.set_viewport(pinfo, W, H); ref.set_viewport(rinfo, W, H)
+        gpu.set_viewport(pinfo, W, H)
         for depth, spp in ((1, 4), (2, 4)):
             s = pinfo.settings.copy(samplesPerPixel=spp, maxPathLength=depth)
             gimg = gpu.render(s, pinfo.scene, pinfo.camera)
             grays = gpu.last_stats().rayQueries
-            rimg, rst = ref.render_deterministic(rinfo.settings.copy(samplesPerPixel=spp, maxPathLength=depth), rinfo.scene, rinfo.camera)
-            exact = float((bits(gimg) == bits(rimg)).all(axis=2).mean())
-            off = rel_outliers(gimg, rimg, rel=1e-4, absolute=1e-5)
-            print("config%d depth %d: bit-identical pixels %.4f, pixels off by > 1e-4 rel: %.4f, PSNR %.1f dB, rays %d vs %d"
-                  % (cfg, depth, exact, off, rl.psnr(gimg, rimg), grays, rst.rayQueries))
+            g, r, _ = recorded.compare("depth%d" % depth, gimg)
+            rays = int(recorded.value("depth%d_rays" % depth))
+            exact = float((bits(g) == bits(r)).all(axis=2).mean())
+            off = rel_outliers(g, r, rel=1e-4, absolute=1e-5)
+            print("config%d depth %d (sample): bit-identical pixels %.4f, pixels off by > 1e-4 rel: %.4f, PSNR %.1f dB, rays %d vs %d"
+                  % (cfg, depth, exact, off, rl.psnr(g, r), grays, rays))
             assert exact >= EXACT_FLOOR and off <= 0.001
-            assert abs(int(grays) - int(rst.rayQueries)) <= 4
+            assert abs(int(grays) - rays) <= 4
     finally:
-        gpu.destroy_demo(pinfo); ref.destroy_demo(rinfo)
+        gpu.destroy_demo(pinfo)
 
 
-def test_lighting_is_read_at_every_render(gpu, ref, rl):
+def test_lighting_is_read_at_every_render(gpu, recorded, rl):
     """The reference reads Scene::GetSun and the sky panorama live on every miss (renderer.cc:160-191): a client may change
     them between frames of a finalized scene.  The uploaded copy must follow (the sun travels per frame, a changed sky
-    re-uploads)."""
-    from oracle import bindings as ob
-    pinfo, rinfo = gpu.create_demo(4, 16), ref.create_demo(4, 16)
+    re-uploads).  The frames after each change are compared with the stored outputs (conftest.RecordedOutputs)."""
+    pinfo = gpu.create_demo(4, 16)
     try:
         W, H = 160, 90
-        gpu.set_viewport(pinfo, W, H); ref.set_viewport(rinfo, W, H)
+        gpu.set_viewport(pinfo, W, H)
         s = pinfo.settings.copy(samplesPerPixel=2, maxPathLength=3)
         first = gpu.render(s, pinfo.scene, pinfo.camera)
-        for lib, info in ((gpu.lib, pinfo), (ref.lib, rinfo)):
-            lib.Raylib_SetSunIlluminance(info.scene, 1.5, 9.0, 0.25)
-            lib.Raylib_SetSunDirection(info.scene, 0.6, -1.0, 0.2)
+        gpu.lib.Raylib_SetSunIlluminance(pinfo.scene, 1.5, 9.0, 0.25)
+        gpu.lib.Raylib_SetSunDirection(pinfo.scene, 0.6, -1.0, 0.2)
         second = gpu.render(s, pinfo.scene, pinfo.camera)
-        want, _ = ref.render_deterministic(rinfo.settings.copy(samplesPerPixel=2, maxPathLength=3), rinfo.scene, rinfo.camera)
         assert not np.array_equal(first, second), "the new sun was ignored"
-        assert rl.psnr(second, want) >= 40.0 and rel_outliers(second, want) <= 0.02
+        g, r, _ = recorded.compare("new_sun", second)
+        assert rl.psnr(g, r) >= 40.0 and rel_outliers(g, r) <= 0.02
         # sun off (renderer.cc:191: no visibility rays at all), then a different sky image
-        for lib, info in ((gpu.lib, pinfo), (ref.lib, rinfo)):
-            lib.Raylib_SetSunIlluminance(info.scene, 0.0, 0.0, 0.0)
+        gpu.lib.Raylib_SetSunIlluminance(pinfo.scene, 0.0, 0.0, 0.0)
         third = gpu.render(s, pinfo.scene, pinfo.camera)
         rays3 = gpu.last_stats().rayQueries
-        want3, rst3 = ref.render_deterministic(rinfo.settings.copy(samplesPerPixel=2, maxPathLength=3), rinfo.scene, rinfo.camera)
-        assert rl.psnr(third, want3) >= 40.0 and abs(int(rays3) - int(rst3.rayQueries)) <= 0.002 * rst3.rayQueries + 8
+        g, r, _ = recorded.compare("sun_off", third)
+        want_rays3 = int(recorded.value("sun_off_rays"))
+        assert rl.psnr(g, r) >= 40.0 and abs(int(rays3) - want_rays3) <= 0.002 * want_rays3 + 8
         sky = np.zeros((8, 16, 4), dtype=np.float32); sky[..., 0] = 2.0; sky[..., 3] = 1.0      # a red sky
-        g_sky, r_sky = gpu.lib.Raylib_CreateImage(16, 8), ref.lib.Raylib_CreateImage(16, 8)
+        g_sky = gpu.lib.Raylib_CreateImage(16, 8)
         try:
             assert gpu.lib.RaylibB200_ImageSetRGBA(g_sky, 16, 8, sky) == 1
-            ref.lib.oracle_image_set_rgba(r_sky, 16, 8, sky)
-            gpu.lib.Raylib_SetSkyPanorama(pinfo.scene, g_sky); ref.lib.Raylib_SetSkyPanorama(rinfo.scene, r_sky)
+            gpu.lib.Raylib_SetSkyPanorama(pinfo.scene, g_sky)
             fourth = gpu.render(s, pinfo.scene, pinfo.camera)
-            want4, _ = ref.render_deterministic(rinfo.settings.copy(samplesPerPixel=2, maxPathLength=3), rinfo.scene, rinfo.camera)
             assert fourth[..., 0].mean() > 4.0 * fourth[..., 2].mean(), "the new sky was ignored"
-            assert rl.psnr(fourth, want4) >= 40.0 and rel_outliers(fourth, want4) <= 0.02
+            g, r, _ = recorded.compare("red_sky", fourth)
+            assert rl.psnr(g, r) >= 40.0 and rel_outliers(g, r) <= 0.02
         finally:
-            gpu.lib.Raylib_SetSkyPanorama(pinfo.scene, 0); ref.lib.Raylib_SetSkyPanorama(rinfo.scene, 0)
-            gpu.lib.Raylib_DestroyImage(g_sky); ref.lib.Raylib_DestroyImage(r_sky)
+            gpu.lib.Raylib_SetSkyPanorama(pinfo.scene, 0)
+            gpu.lib.Raylib_DestroyImage(g_sky)
     finally:
-        gpu.destroy_demo(pinfo); ref.destroy_demo(rinfo)
+        gpu.destroy_demo(pinfo)
 
 
 @pytest.mark.parametrize("cfg,size", [(6, 0), (5, 40), (1, 0)])
@@ -785,25 +799,26 @@ def test_all_devices_behind_plain_raylib_render(gpu, rl):
         gpu.destroy_demo(info)
 
 
-def test_raw_hitable_list_element_on_the_device(gpu, ref, rl):
+def test_raw_hitable_list_element_on_the_device(gpu, recorded, restate, rl):
     """SURVEY 8a row a13 on the GPU: config 7 (a raw HitableList scene element with duplicated members) -- primary ids and t
-    against the compiled reference (pinhole camera: exact), then radiance at matched spp and seed."""
-    pinfo, rinfo = gpu.create_demo(7), ref.create_demo(7)
+    against the C restatement (pinhole camera: exact), then radiance at matched spp and seed against the stored outputs
+    (conftest.RecordedOutputs)."""
+    pinfo = gpu.create_demo(7)
     try:
-        rr, rt, rays, st = ref.primary_hits(rinfo.settings, rinfo.scene, rinfo.camera, want_rays=True)
-        assert st.walkVsHitMismatches == 0
         gr, gt = gpu.primary_hits(pinfo.settings, pinfo.scene, pinfo.camera)
+        rr, rt, rays = restated_primary(gpu, restate, pinfo)
         assert np.array_equal(gr, rr) and np.array_equal(bits(gt), bits(rt))
         gr2, gt2 = gpu.trace_rays(pinfo.scene, rays, pinfo.settings.rayTMin)
         assert np.array_equal(gr2, rr) and np.array_equal(bits(gt2), bits(rt))
-        rimg, rst = ref.render_deterministic(rinfo.settings, rinfo.scene, rinfo.camera)
         gimg = gpu.render(pinfo.settings, pinfo.scene, pinfo.camera)
-        print("config7 radiance: PSNR %.2f dB, bit-identical pixels %.4f" % (rl.psnr(gimg, rimg), float((bits(gimg) == bits(rimg)).all(axis=2).mean())))
-        assert rl.psnr(gimg, rimg) >= 40.0 and rel_outliers(gimg, rimg) <= 0.02
-        assert float((bits(gimg) == bits(rimg)).all(axis=2).mean()) >= EXACT_FLOOR
-        assert abs(int(gpu.last_stats().rayQueries) - int(rst.rayQueries)) <= 0.002 * rst.rayQueries + 8
+        rays = int(recorded.value("radiance_rays"))
+        g, r, _ = recorded.compare("radiance", gimg)
+        print("config7 radiance (sample): PSNR %.2f dB, bit-identical pixels %.4f" % (rl.psnr(g, r), float((bits(g) == bits(r)).all(axis=2).mean())))
+        assert rl.psnr(g, r) >= 40.0 and rel_outliers(g, r) <= 0.02
+        assert float((bits(g) == bits(r)).all(axis=2).mean()) >= EXACT_FLOOR
+        assert abs(int(gpu.last_stats().rayQueries) - rays) <= 0.002 * rays + 8
     finally:
-        gpu.destroy_demo(pinfo); ref.destroy_demo(rinfo)
+        gpu.destroy_demo(pinfo)
 
 
 def test_device_transcendentals_equal_the_host_c_library(gpu):
@@ -842,36 +857,36 @@ def test_device_transcendentals_equal_the_host_c_library(gpu):
         assert same.all(), "%s: %d of %d differ, first at x=%r" % (name, int((~same).sum()), len(idx), x[idx[np.argmin(same)]])
 
 
-def test_obj_import_renders_like_the_reference_conversion(gpu, ref, rl, tmp_path):
+def test_obj_import_renders_like_the_reference_conversion(gpu, recorded, restate, rl, tmp_path):
     """Raylib_LoadOBJModel -> Raylib_AddOBJModelToScene -> Raylib_Render on the GPU against the compiled reference rendering
-    the same file imported through the object API with the reference's conversion rules (scene client config 8): primary
-    ids and t exact (pinhole camera), radiance at matched spp and seed, and bit-identical to the product's own object path."""
+    the same file imported through the object API with the reference's conversion rules (scene client config 8; its
+    frames are stored, see conftest.RecordedOutputs): primary ids and t exact against the C restatement (pinhole camera),
+    radiance at matched spp and seed, debug views, and bit-identical to the product's own object path."""
     import ctypes, os
     from test_cpu_oracle import write_test_obj, load_obj_scene
     libc = ctypes.CDLL(None)
     path = write_test_obj(str(tmp_path))
     os.environ["DEMO_OBJ_PATH"] = path; libc.setenv(b"DEMO_OBJ_PATH", path.encode(), 1)
     try:
-        rinfo, pinfo = ref.create_demo(8), gpu.create_demo(8)
+        pinfo = gpu.create_demo(8)
         model, scene = load_obj_scene(gpu.lib, path)
         try:
             s = pinfo.settings
-            rr, rt, _, _ = ref.primary_hits(rinfo.settings, rinfo.scene, rinfo.camera)
             gr, gt = gpu.primary_hits(s, scene, pinfo.camera)
+            rr, rt, _ = restated_primary(gpu, restate, pinfo, scene=scene)
             assert np.array_equal(gr, rr) and np.array_equal(bits(gt), bits(rt))
             img_import = gpu.render(s, scene, pinfo.camera)
             img_objects = gpu.render(s, pinfo.scene, pinfo.camera)
             assert np.array_equal(bits(img_import), bits(img_objects)), "importer and object path differ"
-            rimg, rst = ref.render_deterministic(rinfo.settings, rinfo.scene, rinfo.camera)
-            exact = float((bits(img_import) == bits(rimg)).all(axis=2).mean())
-            print("OBJ scene radiance vs reference: PSNR %.2f dB, bit-identical pixels %.4f" % (rl.psnr(img_import, rimg), exact))
-            assert rl.psnr(img_import, rimg) >= 40.0 and rel_outliers(img_import, rimg) <= 0.02 and exact >= EXACT_FLOOR
+            g, r, _ = recorded.compare("radiance", img_import)
+            exact = float((bits(g) == bits(r)).all(axis=2).mean())
+            print("OBJ scene radiance vs reference (sample): PSNR %.2f dB, bit-identical pixels %.4f" % (rl.psnr(g, r), exact))
+            assert rl.psnr(g, r) >= 40.0 and rel_outliers(g, r) <= 0.02 and exact >= EXACT_FLOOR
             for mode in (1, 2, 4, 5):
                 g = gpu.render(s.copy(renderMode=mode), scene, pinfo.camera)
-                r, _ = ref.render_deterministic(rinfo.settings.copy(renderMode=mode), rinfo.scene, rinfo.camera)
-                assert np.array_equal(bits(g), bits(r)), "debug view %d" % mode
+                assert recorded.compare("mode%d" % mode, g)[2], "debug view %d" % mode
         finally:
             gpu.lib.Raylib_DestroyScene(scene); gpu.lib.Raylib_UnloadOBJModel(model)
-            gpu.destroy_demo(pinfo); ref.destroy_demo(rinfo)
+            gpu.destroy_demo(pinfo)
     finally:
         os.environ.pop("DEMO_OBJ_PATH", None); libc.unsetenv(b"DEMO_OBJ_PATH")
