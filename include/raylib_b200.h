@@ -9,6 +9,7 @@
 //   RaylibB200_RenderShard / _RenderShardToFrame / _AssembleShards / _RenderToDevice  -> Raylib_Render (raylib/raylib.h:106-110)
 //   RaylibB200_TraceRays / _PrimaryHits                         -> BVHNode::Hit  (raylib/geom/bvh.cc:82-107)
 //   RaylibB200_SetFrameSeed / _SetBvhBuildKey                   -> std::random_device seeding (raylib/core/random.h:17-29, geom/bvh.cc:43)
+//   RaylibB200_RenderAccumulate / _Accumulator*                 -> Raylib_Render in installments (progressive rendering)
 #pragma once
 #include "raylib_types.h"
 
@@ -138,6 +139,44 @@ RAYLIB_API int32_t RaylibB200_PostProcessGPU(ImageHandle image);
 // SetRGBA resizes the image.  Both return 1 on success.
 RAYLIB_API int32_t RaylibB200_ImageSetRGBA(ImageHandle image, uint32_t width, uint32_t height, const float* rgba);
 RAYLIB_API int32_t RaylibB200_ImageGetRGBA(ImageHandle image, float* outRgba);
+
+// ---- progressive rendering: a frame in installments -----------------------------------------------
+// An accumulator holds, for every pixel of a W x H frame, the float sums {sum R, sum G, sum B, sum luminance^2} of the
+// samples rendered so far, on the device that was current when it was created, and their count n.  RenderAccumulate
+// renders samples [n, n + samples) of every pixel and adds them to the sums in sample order -- the float additions of
+// one Raylib_Render of n + samples samples -- so that a resolve after any installment is BIT-IDENTICAL to Raylib_Render
+// with samplesPerPixel = n at the same frame seed, whatever the installment sizes, pipes, passes or device count were.
+// The first installment binds the accumulator to what decides the image: viewport (= the accumulator's size),
+// maxPathLength, rayTMin, frame seed, camera, the sun the frame is rendered with, and the uploaded scene (a fingerprint of
+// its arrays: a scene and its RaylibB200_LoadFlattenedScene reload are the same scene, a swapped sky is not).  A later
+// installment that differs in any of them is refused (0; GetLastError names every differing field) and changes nothing: start a new
+// image with Reset.  Installments spread over the active GPUs like Raylib_Render (the sums live on the first one, which
+// must be the accumulator's device; without peer access they render there alone).  Functions returning int32_t return
+// 1 on success and 0 on failure (GetLastError).
+typedef struct RaylibB200Accumulator RaylibB200Accumulator;
+// NULL without a CUDA device.  Create: n = 0, unbound.  Reset zeroes the sums and drops the binding.
+RAYLIB_API RaylibB200Accumulator* RaylibB200_AccumulatorCreate(uint32_t width, uint32_t height);
+RAYLIB_API void    RaylibB200_AccumulatorDestroy(RaylibB200Accumulator* acc);
+RAYLIB_API int32_t RaylibB200_AccumulatorReset(RaylibB200Accumulator* acc);
+RAYLIB_API uint32_t RaylibB200_AccumulatorSamples(const RaylibB200Accumulator* acc);      // n
+// settings->samplesPerPixel is ignored; renderMode must be 0 (path tracing); n + samples <= 2^24 (the divisor stays exact).
+// GetLastStats reports this installment (its pixel-samples, ray queries, passes).
+RAYLIB_API int32_t RaylibB200_RenderAccumulate(const RendererSettings* settings, SceneHandle scene, CameraHandle camera,
+	RaylibB200Accumulator* acc, uint32_t samples);
+// The average of the n samples (alpha 1) into an Image2D (resized like Raylib_Render resizes it) or into a W x H RGBA float4
+// device image on the accumulator's device (cudaStream may be NULL; synchronous).
+RAYLIB_API int32_t RaylibB200_AccumulatorResolve(RaylibB200Accumulator* acc, ImageHandle outImage);
+RAYLIB_API int32_t RaylibB200_AccumulatorResolveDevice(RaylibB200Accumulator* acc, void* deviceImageOut, void* cudaStream);
+// The raw sums, W*H*4 floats {sum R, sum G, sum B, sum luminance^2}, row 0 on top.
+RAYLIB_API int32_t RaylibB200_AccumulatorRead(RaylibB200Accumulator* acc, float* outRgba);
+// Relative standard error of each pixel's mean luminance: with m = luminance(sum) / n and var = max(0, (sumY2 - n m^2) / (n - 1)),
+// sqrt(var / n) / max(m, 1e-4).  perPixel (nullable) receives W*H floats, mean (nullable) their average, summed in a fixed
+// order (the same sums give the same double).  Needs n >= 2.
+RAYLIB_API int32_t RaylibB200_AccumulatorNoise(RaylibB200Accumulator* acc, float* perPixel, double* mean);
+// Checkpoint file: header, binding, n, sums and a checksum.  Load validates the whole file before it touches a device (a
+// foreign, truncated or damaged file is refused even without a GPU) and creates the accumulator on the current device.
+RAYLIB_API int32_t RaylibB200_AccumulatorSave(const RaylibB200Accumulator* acc, const char* path);
+RAYLIB_API RaylibB200Accumulator* RaylibB200_AccumulatorLoad(const char* path);
 
 // ---- queries used by parity tests ---------------------------------------------------------------
 // Closest hit of caller-supplied rays (8 floats each: o.xyz, time, d.xyz, unused).  outRank = global

@@ -11,12 +11,15 @@
 //   k_miss        sky lookup, spawns the sun visibility ray          render/renderer.cc:156-193
 //   k_shadow      any-hit query toward the sun                       render/renderer.cc:194-198
 //   k_accumulate  accum += Li (sample order), /= SPP, SetPixel       render/renderer.cc:244-248
+//                 (or: continue and store back a running sum, rt_progressive.h)
 //   k_debug_view  TraceSceneDebugMode                                render/renderer.cc:62-111
 // Recursion is unrolled into a per-path bounce stack {reflectance, scatPdf, emitted, pdf} that is
 // folded tail-first when the path ends, reproducing the nested arithmetic of TraceScene exactly.
 //
 // Compile: nvcc -gencode arch=compute_100a,code=sm_100a --fmad=false -lineinfo (see Makefile).
 #include "rt_device_abi.h"
+#include "rt_progressive.h"
+#include "rt_checksum.h"
 #include "rt_shade.cuh"
 
 #include <cuda_runtime.h>
@@ -152,6 +155,8 @@ struct RtLaunch
 	uint32_t refillThreshold;  // a warp refills its idle lanes once fewer than this many lanes are traversing
 	uint32_t walkThreshold;    // the node phase yields to the leaf phase once fewer than this many lanes can step
 	float    tMin;
+	uint32_t runningSum;       // 1 = `image` holds the undivided per-pixel sums {sum RGB, sum luminance^2} of earlier samples:
+	                           //   the first pass continues them, the last pass stores them back (progressive rendering)
 };
 
 // ---- path-state accessors (one definition per layout) ------------------------------------------------------------
@@ -910,7 +915,13 @@ __global__ void __launch_bounds__(128, RT_EXTEND_MIN_BLOCKS) k_shadow(const __gr
 	shadow_stage(L, bounce, stack);
 }
 
+// Rec. 709 weights, as Image2D::PostProcess uses them (render/image.cc:44-103)
+RT_DEV float luminance3(float3 v) { return dot3(v, v3(0.2126f, 0.7152f, 0.0722f)); }
+
 // Grid-stride over the shard's pixel slots: every pixel sums its K samples in sample order (renderer.cc:244-246).
+// Running-sum mode continues the sums held in the row-major `image` and stores them back undivided, so that samples [a, b)
+// added to the stored sum of [0, a) take exactly the float additions of one frame of b samples; .w sums the squared
+// luminance of the samples (the noise estimate of RaylibB200_AccumulatorNoise).
 RT_DEV void accumulate_stage(const RtLaunch& L, int firstPass, int lastPass)
 {
 	if (blockIdx.x == 0 && threadIdx.x == 0)
@@ -932,15 +943,24 @@ RT_DEV void accumulate_stage(const RtLaunch& L, int firstPass, int lastPass)
 			if (lastPass && !L.image) L.out[lp] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);      // padding slot of the shard buffer
 			continue;
 		}
-		float3 a = firstPass ? v3(0.0f) : xyz(L.accum[lp]);
+		const size_t pixel = (size_t)y * L.width + x;
+		const float4 start = !firstPass ? L.accum[lp] : L.runningSum ? L.image[pixel] : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+		float3 a = xyz(start);
+		float y2 = start.w;
 		const uint32_t kValid = min(L.K, L.spp - L.passBase);
-		for (uint32_t k = 0; k < kValid; ++k) a = a + xyz(L.Li[(size_t)k * L.npix + lp]);
-		if (lastPass)
+		for (uint32_t k = 0; k < kValid; ++k)
+		{
+			const float3 li = xyz(L.Li[(size_t)k * L.npix + lp]);
+			a = a + li;
+			if (L.runningSum) { const float lum = luminance3(li); y2 += lum * lum; }
+		}
+		if (lastPass && L.runningSum) L.image[pixel] = make_float4(a.x, a.y, a.z, y2);
+		else if (lastPass)
 		{
 			a = div_assign3(a, (float)L.spp);
 			store_pixel(L, lp, x, y, make_float4(a.x, a.y, a.z, 1.0f));
 		}
-		else L.accum[lp] = make_float4(a.x, a.y, a.z, 0.0f);
+		else L.accum[lp] = make_float4(a.x, a.y, a.z, y2);
 	}
 }
 __global__ void __launch_bounds__(256) k_accumulate(const __grid_constant__ RtLaunch L, int firstPass, int lastPass) { accumulate_stage(L, firstPass, lastPass); }
@@ -1189,6 +1209,7 @@ struct RtDeviceScene
 	RtSceneView view;
 	std::vector<void*> allocations;
 	std::vector<size_t> allocationBytes;
+	std::vector<size_t> contentBytes;     // bytes of each allocation that hold uploaded data (an empty array still allocates)
 	uint32_t maxStackDepth = 0;
 	uint32_t materialTypeMask = 0;
 	uint32_t numLeaves = 0;
@@ -1241,6 +1262,7 @@ static int upload_array(RtDeviceScene* sc, const T* host, size_t count, const T*
 	RT_CUDA(cudaMalloc(&dev, bytes));
 	sc->allocations.push_back(dev);
 	sc->allocationBytes.push_back(bytes);
+	sc->contentBytes.push_back(count * sizeof(T));
 	sc->bytes += bytes;
 	if (count) RT_CUDA(cudaMemcpy(dev, host, count * sizeof(T), cudaMemcpyHostToDevice));
 	*outDev = reinterpret_cast<const T*>(dev);
@@ -1595,7 +1617,25 @@ static void fill_scene(RtLaunch& L, const RtDeviceScene* sc, const RtCamera* cam
 extern "C" int rt_render_shard(RtRenderContext* ctx, const RtDeviceScene* sc, const RtCamera* cam,
                                const RtRenderParams* p, void* deviceShardOut, void* streamPtr, RtRenderStats* stats)
 {
-	if (!ctx || !sc || !cam || !p || (!deviceShardOut && !p->imageOut)) { g_lastError = "rt_render_shard: null argument"; return -1; }
+	if (!p) { g_lastError = "rt_render_shard: null argument"; return -1; }
+	return rt_render_window(ctx, sc, cam, p, 0u, (uint32_t)std::max(1, p->samplesPerPixel), nullptr, deviceShardOut, streamPtr, stats);
+}
+
+extern "C" int rt_render_window(RtRenderContext* ctx, const RtDeviceScene* sc, const RtCamera* cam, const RtRenderParams* params,
+                                uint32_t sampleBegin, uint32_t sampleEnd, void* runningSum, void* deviceShardOut, void* streamPtr,
+                                RtRenderStats* stats)
+{
+	if (!ctx || !sc || !cam || !params || (!deviceShardOut && !params->imageOut && !runningSum)) { g_lastError = "rt_render_shard: null argument"; return -1; }
+	if (sampleBegin >= sampleEnd || sampleEnd > (uint32_t)INT32_MAX) { g_lastError = "rt_render_window: empty sample window"; return -1; }
+	if (runningSum ? params->renderMode != 0u : sampleBegin != 0u)
+	{
+		g_lastError = "rt_render_window: a running sum needs path tracing, a window not starting at sample 0 a running sum";
+		return -1;
+	}
+	// the window's end is the frame's sample count of the kernels (raygen skips samples >= spp); its length sizes the passes
+	RtRenderParams windowParams = *params;
+	windowParams.samplesPerPixel = (int32_t)sampleEnd;
+	const RtRenderParams* p = &windowParams;
 	if (p->imageOut && p->renderMode == RT_RENDERMODE_AUX) { g_lastError = "rt_render_shard: the fused denoiser-input pass writes shard buffers only"; return -1; }
 	if (sc->device != ctx->device) { g_lastError = "rt_render_shard: scene and context live on different devices"; return -1; }
 	if (p->width == 0 || p->height == 0) { g_lastError = "rt_render_shard: empty viewport"; return -1; }
@@ -1610,6 +1650,7 @@ extern "C" int rt_render_shard(RtRenderContext* ctx, const RtDeviceScene* sc, co
 	memset(&probe, 0, sizeof(probe));
 	fill_scene(probe, sc, cam, p, levels);
 	const uint32_t npix = probe.npix, spp = probe.spp;
+	const uint32_t win = spp - sampleBegin;      // samples per pixel this call renders
 	const bool pathTrace = p->renderMode == 0u;
 	if (p->renderMode == RT_RENDERMODE_AUX && !p->auxShardOut) { g_lastError = "rt_render_shard: RT_RENDERMODE_AUX needs auxShardOut"; return -1; }
 
@@ -1623,7 +1664,7 @@ extern "C" int rt_render_shard(RtRenderContext* ctx, const RtDeviceScene* sc, co
 	if (pathTrace && !p->collectStats && !p->timeStages && !p->samplesPerPass && p->tuning.fusedPass != 1u && !p->tuning.pooledTraversal && ctx->cooperative)
 	{
 		const uint64_t limit = (uint64_t)(p->tuning.fusedPathsK ? p->tuning.fusedPathsK : RT_DEFAULT_FUSED_PATHS_K) << 10;
-		const uint64_t paths = (uint64_t)spp * npix;
+		const uint64_t paths = (uint64_t)win * npix;
 		fused = p->tuning.fusedPass == 2u ? paths <= (32ull << 20) : paths <= limit;
 	}
 	if (fused) pipes = 1;
@@ -1636,16 +1677,16 @@ extern "C" int rt_render_shard(RtRenderContext* ctx, const RtDeviceScene* sc, co
 		// launches (measured: +5 % on scatter10M, +10 % on grid1M going from 4 M to 32 M).
 		const uint64_t targetPaths = (uint64_t)(p->tuning.pathsM ? p->tuning.pathsM : RT_DEFAULT_PATHS_M) << 20;
 		const uint64_t perPass = std::max<uint64_t>(1, targetPaths / std::max(1u, npix));
-		if (fused) K = spp;
-		else if (p->samplesPerPass) { K = std::min<uint32_t>(p->samplesPerPass, spp); if (K >= spp) pipes = 1; }
-		else if (pipes > 1 && spp >= 2u)
+		if (fused) K = win;
+		else if (p->samplesPerPass) { K = std::min<uint32_t>(p->samplesPerPass, win); if (K >= win) pipes = 1; }
+		else if (pipes > 1 && win >= 2u)
 		{
-			K = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(1, perPass / pipes), (spp + pipes - 1) / pipes);
+			K = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(1, perPass / pipes), (win + pipes - 1) / pipes);
 			// few samples per pixel: prefer two passes per pipe (more overlap) while a pass still fills the machine
-			const uint32_t finer = (spp + 2u * pipes - 1u) / (2u * pipes);
+			const uint32_t finer = (win + 2u * pipes - 1u) / (2u * pipes);
 			if (finer < K && (uint64_t)finer * npix >= (4ull << 20)) K = finer;
 		}
-		else { K = (uint32_t)std::min<uint64_t>(perPass, spp); pipes = 1; }
+		else { K = (uint32_t)std::min<uint64_t>(perPass, win); pipes = 1; }
 	}
 	// path slots are 32-bit indices: never more than 2^31 paths in one pass, whatever the caller asks for
 	if (pathTrace) K = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(K, (1ull << 31) / std::max(1u, npix)));
@@ -1668,7 +1709,7 @@ extern "C" int rt_render_shard(RtRenderContext* ctx, const RtDeviceScene* sc, co
 		}
 		else if (grows) cudaGetLastError();
 	}
-	uint32_t numPasses = pathTrace ? (spp + K - 1) / K : 1u;
+	uint32_t numPasses = pathTrace ? (win + K - 1) / K : 1u;
 	if (numPasses < 2u) pipes = 1;
 
 	int rc;
@@ -1687,7 +1728,7 @@ extern "C" int rt_render_shard(RtRenderContext* ctx, const RtDeviceScene* sc, co
 		if (!outOfMemory) break;
 		for (RtPipe& pipe : ctx->pipe) free_arena(pipe);
 		K = std::max(1u, K / 2u);
-		numPasses = (spp + K - 1) / K;
+		numPasses = (win + K - 1) / K;
 	}
 	for (int q = 0; q < pipes; ++q)
 	{
@@ -1698,13 +1739,14 @@ extern "C" int rt_render_shard(RtRenderContext* ctx, const RtDeviceScene* sc, co
 		L.K = K;
 		L.accum = ctx->accum;
 		L.out = reinterpret_cast<float4*>(deviceShardOut);
-		L.image = reinterpret_cast<float4*>(p->imageOut);
+		L.image = reinterpret_cast<float4*>(runningSum ? runningSum : p->imageOut);
+		L.runningSum = runningSum ? 1u : 0u;
 		L.out2 = reinterpret_cast<float4*>(p->auxShardOut);
 		L.ctl = pipe.ctl;
 		if (fused) { L.binBits = 0; L.numBins = 0; }
 	}
 	// memory pressure may have cut the samples in flight: the fused pass wants them all at once
-	if (fused && (K < spp || numPasses != 1u)) fused = false;
+	if (fused && (K < win || numPasses != 1u)) fused = false;
 
 	uint32_t launches = 0, passes = 0, extendLaunches[RT_MAX_PIPES] = { 0 };
 	const bool timeStages = p->timeStages != 0 && stats != nullptr;
@@ -1727,7 +1769,7 @@ extern "C" int rt_render_shard(RtRenderContext* ctx, const RtDeviceScene* sc, co
 	{
 		RtPipe& pipe = ctx->pipe[0];
 		RtLaunch& L = pipe.L;
-		L.passBase = 0;
+		L.passBase = sampleBegin;
 		int grid = 0;
 		if ((rc = persistent_grid(ctx, k_pass_fused, 128, smem, &grid))) return rc;
 		RT_CUDA(cudaMemsetAsync(L.bounceCtl, 0, ((size_t)std::max(0, p->maxPathLength) + 2) * sizeof(RtBounceCtl), stream));
@@ -1808,7 +1850,7 @@ extern "C" int rt_render_shard(RtRenderContext* ctx, const RtDeviceScene* sc, co
 				RtPipe& pipe = ctx->pipe[q];
 				RtLaunch& L = pipe.L;
 				cudaStream_t ps = pipes > 1 ? pipe.stream : stream;
-				L.passBase = (group + (uint32_t)q) * K;
+				L.passBase = sampleBegin + (group + (uint32_t)q) * K;
 				RT_CUDA(cudaMemsetAsync(L.bounceCtl, 0, ((size_t)std::max(0, p->maxPathLength) + 2) * sizeof(RtBounceCtl), ps));
 				const uint32_t total = K * npix;
 				k_raygen<<<std::min<uint32_t>((total + 255) / 256, (uint32_t)ctx->numSMs * 8u), 256, 0, ps>>>(L);
@@ -1930,7 +1972,7 @@ extern "C" int rt_render_shard(RtRenderContext* ctx, const RtDeviceScene* sc, co
 			px += (uint64_t)w * hgt;
 			stats->tilesRendered++;
 		}
-		stats->pixelSamples = px * (pathTrace ? spp : 1u);
+		stats->pixelSamples = px * (pathTrace ? win : 1u);
 	}
 	return 0;
 }
@@ -1999,7 +2041,6 @@ extern "C" int rt_trace_closest(RtRenderContext* ctx, const RtDeviceScene* sc, c
 }
 
 // ---- Image2D::PostProcess on the device (render/image.cc:44-103) -----------------------------------------
-RT_DEV float luminance3(float3 v) { return dot3(v, v3(0.2126f, 0.7152f, 0.0722f)); }
 
 // Luminance is never negative where it matters (the maximum starts at 1.0), so the float order equals the order of
 // the bit patterns and one atomicMax per block on the raw bits is exact.
@@ -2075,6 +2116,142 @@ extern "C" int rt_postprocess(int device, void* deviceImage, uint32_t width, uin
 		RT_CUDA(cudaStreamSynchronize(stream));
 	}
 	RT_CUDA(cudaFreeAsync(maxBits, stream));
+	return 0;
+}
+
+// ---- progressive rendering: resolve of a running sum, scene fingerprint (rt_progressive.h) ------------------------------
+// One pixel per thread; the noise figure's sum is reduced by a fixed tree in each block and the blocks are added in index
+// order on the host, so the same sums give the same double every time.
+__global__ void __launch_bounds__(256) k_resolve(const float4* sums, uint32_t count, float n, float4* image, float* noise, double* blockSums)
+{
+	__shared__ double part[256];
+	const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+	double rel = 0.0;
+	if (i < count)
+	{
+		const float4 s = sums[i];
+		if (image)
+		{
+			const float3 a = div_assign3(xyz(s), n);      // the last pass of a one-shot frame of n samples
+			image[i] = make_float4(a.x, a.y, a.z, 1.0f);
+		}
+		if (noise || blockSums)
+		{
+			// relative standard error of the mean luminance: sqrt(var / n) / mean, var the unbiased sample variance
+			const float m = luminance3(xyz(s)) / n;
+			const float var = fmaxf(0.0f, (s.w - n * m * m) / (n - 1.0f));
+			const float r = sqrtf(var / n) / fmaxf(m, 1e-4f);
+			if (noise) noise[i] = r;
+			rel = r;
+		}
+	}
+	if (!blockSums) return;
+	part[threadIdx.x] = rel;
+	__syncthreads();
+	for (uint32_t half = blockDim.x / 2u; half > 0u; half >>= 1)
+	{
+		if (threadIdx.x < half) part[threadIdx.x] += part[threadIdx.x + half];
+		__syncthreads();
+	}
+	if (threadIdx.x == 0) blockSums[blockIdx.x] = part[0];
+}
+
+extern "C" int rt_resolve(int device, const void* sums, uint32_t count, uint32_t n, void* deviceImageOut, float* deviceNoiseOut,
+                          double* hostNoiseSum, void* streamPtr)
+{
+	if (!sums || count == 0 || n == 0) { g_lastError = "rt_resolve: empty accumulator"; return -1; }
+	if ((deviceNoiseOut || hostNoiseSum) && n < 2) { g_lastError = "rt_resolve: the noise figure needs at least 2 samples"; return -1; }
+	RT_CUDA(cudaSetDevice(device));
+	cudaStream_t stream = (cudaStream_t)streamPtr;
+	const uint32_t blocks = (count + 255u) / 256u;
+	double* blockSums = nullptr;
+	if (hostNoiseSum) RT_CUDA(cudaMallocAsync((void**)&blockSums, blocks * sizeof(double), stream));
+	k_resolve<<<blocks, 256, 0, stream>>>(reinterpret_cast<const float4*>(sums), count, (float)n,
+	                                      reinterpret_cast<float4*>(deviceImageOut), deviceNoiseOut, blockSums);
+	RT_CUDA(cudaGetLastError());
+	if (hostNoiseSum)
+	{
+		std::vector<double> host(blocks);
+		RT_CUDA(cudaMemcpyAsync(host.data(), blockSums, blocks * sizeof(double), cudaMemcpyDeviceToHost, stream));
+		RT_CUDA(cudaFreeAsync(blockSums, stream));
+		RT_CUDA(cudaStreamSynchronize(stream));
+		double total = 0.0;
+		for (double b : host) total += b;
+		*hostNoiseSum = total;
+	}
+	else RT_CUDA(cudaStreamSynchronize(stream));
+	return 0;
+}
+
+// Each thread hashes one RT_HASH_CHUNK-byte chunk with RtChecksum (allocations are 256-byte aligned, so the words are
+// aligned 8-byte loads); the host combines the chunk values in order.
+#define RT_HASH_CHUNK 4096u
+__global__ void __launch_bounds__(256) k_hash_chunks(const unsigned char* data, uint64_t bytes, uint64_t* chunkHash)
+{
+	const uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+	const uint64_t begin = c * RT_HASH_CHUNK;
+	if (begin >= bytes) return;
+	const uint64_t len = bytes - begin < RT_HASH_CHUNK ? bytes - begin : RT_HASH_CHUNK;
+	const uint64_t* words = reinterpret_cast<const uint64_t*>(data + begin);
+	RtChecksum sum;
+	uint64_t i = 0;
+	for (; i + 8u <= len; i += 8u) sum.Mix(words[i / 8u]);
+	if (i < len)
+	{
+		uint64_t w = 0;
+		for (uint64_t b = i; b < len; ++b) w |= (uint64_t)data[begin + b] << (8u * (b - i));
+		sum.Mix(w);
+	}
+	sum.Mix(len);
+	chunkHash[c] = sum.h;
+}
+
+extern "C" int rt_scene_fingerprint(const RtDeviceScene* sc, uint64_t* out)
+{
+	if (!sc || !out) { g_lastError = "rt_scene_fingerprint: null argument"; return -1; }
+	RT_CUDA(cudaSetDevice(sc->device));
+	RtChecksum sum;
+	uint64_t* chunkHash = nullptr;
+	size_t capacity = 0;
+	std::vector<uint64_t> host;
+	int rc = 0;
+	for (size_t a = 0; a < sc->allocations.size() && rc == 0; ++a)
+	{
+		if (sc->allocations[a] == (const void*)sc->view.refNodes) continue;      // statistics frames only
+		const uint64_t bytes = sc->contentBytes[a];
+		const uint64_t chunks = (bytes + RT_HASH_CHUNK - 1u) / RT_HASH_CHUNK;
+		sum.Mix(bytes);
+		if (!chunks) continue;
+		if (chunks > capacity)
+		{
+			if (chunkHash) cudaFree(chunkHash);
+			chunkHash = nullptr; capacity = 0;
+			cudaError_t e = cudaMalloc((void**)&chunkHash, chunks * sizeof(uint64_t));
+			if (e != cudaSuccess) { g_lastError = std::string("rt_scene_fingerprint: ") + cudaGetErrorString(e); cudaGetLastError(); rc = (int)e; break; }
+			capacity = chunks;
+		}
+		k_hash_chunks<<<(unsigned)((chunks + 255u) / 256u), 256>>>(reinterpret_cast<const unsigned char*>(sc->allocations[a]), bytes, chunkHash);
+		host.resize(chunks);
+		cudaError_t e = cudaMemcpy(host.data(), chunkHash, chunks * sizeof(uint64_t), cudaMemcpyDeviceToHost);
+		if (e != cudaSuccess) { g_lastError = std::string("rt_scene_fingerprint: ") + cudaGetErrorString(e); cudaGetLastError(); rc = (int)e; break; }
+		for (uint64_t h : host) sum.Mix(h);
+	}
+	if (chunkHash) cudaFree(chunkHash);
+	if (rc) return rc;
+	// the scalars of the view that decide the image (pointers differ per upload; the sun is a per-frame value)
+	const RtSceneView& v = sc->view;
+	sum.Add(v.rootMin, sizeof(v.rootMin)); sum.Add(v.rootMax, sizeof(v.rootMax)); sum.Mix(v.rootRef);
+	sum.Add(v.refRootMin, sizeof(v.refRootMin)); sum.Add(v.refRootMax, sizeof(v.refRootMax)); sum.Mix(v.refRootRef); sum.Mix(v.refRootBoxTests);
+	sum.Mix(v.flags); sum.Mix((uint32_t)v.skyTexture); sum.Add(v.skyRotation, sizeof(v.skyRotation));
+	sum.Mix(sc->maxStackDepth); sum.Mix(sc->materialTypeMask); sum.Mix(sc->numLeaves);
+	*out = sum.h;
+	return 0;
+}
+
+extern "C" int rt_device_zero(int device, void* ptr, uint64_t bytes)
+{
+	RT_CUDA(cudaSetDevice(device));
+	RT_CUDA(cudaMemset(ptr, 0, bytes));
 	return 0;
 }
 

@@ -8,6 +8,7 @@
 #include "render/material.h"
 #include "render/camera.h"
 #include "render/image.h"
+#include "rt_checksum.h"
 
 #include <algorithm>
 #include <atomic>
@@ -795,30 +796,15 @@ namespace
 		r[4] = sizeof(RtSphere); r[5] = sizeof(RtCube); r[6] = sizeof(RtMaterial); r[7] = sizeof(RtTexture);
 	}
 
-	// 64-bit multiply-xorshift over 8-byte words (tail bytes zero-padded): catches truncation and bit rot, runs at memory speed
-	struct Checksum
-	{
-		uint64_t h = 0x9E3779B97F4A7C15ull;
-		void Add(const void* data, size_t bytes)
-		{
-			const unsigned char* p = (const unsigned char*)data;
-			size_t i = 0;
-			for (; i + 8 <= bytes; i += 8) { uint64_t w; memcpy(&w, p + i, 8); Mix(w); }
-			if (i < bytes) { uint64_t w = 0; memcpy(&w, p + i, bytes - i); Mix(w); }
-			Mix((uint64_t)bytes);
-		}
-		void Mix(uint64_t w) { h ^= w; h *= 0xD6E8FEB86659FD93ull; h ^= h >> 32; }
-	};
-
 	struct FlatWriter
 	{
-		FILE* f; Checksum sum; uint64_t bytes = 0; bool ok = true;
+		FILE* f; RtChecksum sum; uint64_t bytes = 0; bool ok = true;
 		void Raw(const void* data, size_t n) { if (n && fwrite(data, 1, n, f) != n) ok = false; sum.Add(data, n); bytes += n; }
 		template<typename T, typename A> void Array(const std::vector<T, A>& v) { const uint64_t n = v.size(); Raw(&n, 8); Raw(v.data(), v.size() * sizeof(T)); }
 	};
 	struct FlatReader
 	{
-		FILE* f; Checksum sum; bool ok = true;
+		FILE* f; RtChecksum sum; bool ok = true;
 		void Raw(void* data, size_t n) { if (n && fread(data, 1, n, f) != n) ok = false; else sum.Add(data, n); }
 		template<typename T, typename A> void Array(std::vector<T, A>& v, uint64_t limitBytes)
 		{

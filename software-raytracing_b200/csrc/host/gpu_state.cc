@@ -4,6 +4,8 @@
 #include "gpu_state.h"
 #include "flatten.h"
 #include "host_internal.h"
+#include "rt_checksum.h"
+#include "rt_progressive.h"
 #include "geom/scene.h"
 #include "render/camera.h"
 #include "render/image.h"
@@ -35,6 +37,8 @@ namespace
 		// sky changed is flattened again; the sun is passed per frame (RtRenderParams.lightingOverride)
 		ImageHandle skyHandle = 0;
 		uint64_t skySignature = 0;
+		uint64_t fingerprint = 0;        // rt_scene_fingerprint of this upload, computed when an accumulator first binds to it
+		bool fingerprinted = false;
 	};
 
 	std::recursive_mutex g_mutex;
@@ -468,7 +472,8 @@ namespace RtGpu
 
 	bool Render(const RendererSettings* settings, const Scene* scene, const Camera* camera,
 	            Image2D* hostImage, void* deviceImage, void* deviceShard,
-	            uint32_t shardRank, uint32_t shardCount, uint32_t renderModeOverride, void* stream, bool pinHostImage)
+	            uint32_t shardRank, uint32_t shardCount, uint32_t renderModeOverride, void* stream, bool pinHostImage,
+	            const SampleWindow* window)
 	{
 		std::lock_guard<std::recursive_mutex> lock(g_mutex);
 		const auto wall0 = std::chrono::steady_clock::now();
@@ -515,12 +520,17 @@ namespace RtGpu
 		// ---- which devices render this frame -------------------------------------------------------------
 		// A whole frame (read back into a host image, or left in a row-major device image on the primary device) is spread over the
 		// active devices by interleaved 16x16 tiles (SURVEY 8e); shards, debug views and statistics frames stay on the primary device.
-		const uint64_t pixelSamples = (uint64_t)params.width * params.height * (uint64_t)std::max(1, params.samplesPerPixel);
+		const uint64_t samples = window ? (uint64_t)(window->end - window->begin) : (uint64_t)std::max(1, params.samplesPerPixel);
+		const uint64_t pixelSamples = (uint64_t)params.width * params.height * samples;
 		std::vector<int> devices(1, primary);
-		const bool wholeFrame = hostImage || (deviceImage && !deviceShard && shardCount <= 1);
+		const bool wholeFrame = window || hostImage || (deviceImage && !deviceShard && shardCount <= 1);
 		if (wholeFrame && params.renderMode == 0u && !g_collectStats && !g_timeStages && g_devices.size() > 1 &&
 		    pixelSamples >= g_multiDeviceMinSamples)
 			devices = g_devices;
+		// the running sums of an installment live on the primary device: a device that cannot address them sits it out
+		if (window && devices.size() > 1)
+			for (size_t i = 1; i < devices.size(); ++i)
+				if (!PeerOk(devices[i], primary)) { devices.assign(1, primary); break; }
 		const uint32_t n = (uint32_t)devices.size();
 
 		// hostImage: always the whole frame; deviceShard / deviceImage: the tiles of (shardRank, shardCount)
@@ -561,7 +571,7 @@ namespace RtGpu
 		for (uint32_t i = 1; i < n; ++i) direct = direct && PeerOk(work[i].device, primary);
 		if (!deviceShard)
 		{
-			imageBuffer = deviceImage ? deviceImage : ScratchBuffer(primary, 1, imageBytes);
+			imageBuffer = window ? window->sums : deviceImage ? deviceImage : ScratchBuffer(primary, 1, imageBytes);
 			if (!imageBuffer) { SetLastError(std::string("device allocation failed: ") + rt_last_error()); return false; }
 		}
 		const uint64_t shardBytes = (uint64_t)rt_shard_tile_capacity(params.width, params.height, n) * RT_TILE_PIXELS * 16ull;
@@ -582,9 +592,10 @@ namespace RtGpu
 
 		// one host thread per device issues that device's launches (about ten thousand per 4K frame) and waits for it;
 		// they share nothing but the read-only camera block
-		auto renderOn = [&cam](PerDevice& w, void* onStream)
+		auto renderOn = [&cam, window](PerDevice& w, void* onStream)
 		{
-			w.rc = rt_render_shard(w.ctx, w.scene, &cam, &w.params, w.shard, onStream, &w.stats);
+			w.rc = window ? rt_render_window(w.ctx, w.scene, &cam, &w.params, window->begin, window->end, window->sums, w.shard, onStream, &w.stats)
+			              : rt_render_shard(w.ctx, w.scene, &cam, &w.params, w.shard, onStream, &w.stats);
 			if (w.rc != 0) w.error = rt_last_error();
 		};
 		{
@@ -757,6 +768,358 @@ namespace RtGpu
 		std::lock_guard<std::recursive_mutex> lock(g_mutex);
 		auto it = g_prebuilt.find(scene);
 		return it == g_prebuilt.end() ? nullptr : it->second;
+	}
+}
+
+// ---------------------------------------------------------------------------------------------
+// Progressive rendering: an accumulator is the running sum of a frame rendered in installments (DESIGN.md section 13)
+
+// What decides the image of an accumulated frame; recorded by the first installment, compared by every later one, and
+// stored in checkpoint files as is.
+struct RtAccumBinding
+{
+	uint32_t width, height;
+	int32_t  maxPathLength;
+	float    rayTMin;
+	uint64_t frameSeed;
+	RtCamera camera;
+	float    sunIlluminance[3], sunDirection[3];
+	uint64_t sceneFingerprint;
+};
+static_assert(sizeof(RtAccumBinding) == 152, "the binding record has no padding (it is compared and stored bytewise)");
+
+struct RaylibB200Accumulator
+{
+	int device = 0;
+	uint32_t width = 0, height = 0;
+	void* sums = nullptr;             // row-major W x H float4 {sum R, sum G, sum B, sum luminance^2}
+	uint32_t samples = 0;             // n
+	bool bound = false;
+	RtAccumBinding binding;
+};
+
+namespace
+{
+	const uint32_t kMaxAccumSamples = 1u << 24;       // every count up to here is exact as the float divisor
+	const char* kNoDevice = "no CUDA device is available; this library renders on the GPU only (no CPU path)";
+
+	struct AccumFileHeader
+	{
+		char     magic[8];            // "RTACCUM1"
+		uint32_t headerBytes;         // sizeof(AccumFileHeader)
+		uint32_t bindingBytes;        // sizeof(RtAccumBinding)
+		uint32_t width, height;
+		uint32_t samples;             // n
+		uint32_t bound;
+		uint64_t checksum;            // RtChecksum of this header (checksum = 0), the binding and the sums
+	};
+	static_assert(sizeof(AccumFileHeader) == 40, "accumulator file header is 40 bytes");
+
+	uint64_t AccumFileChecksum(const AccumFileHeader& h, const RtAccumBinding& b, const float* sums, uint64_t sumBytes)
+	{
+		AccumFileHeader zeroed = h;
+		zeroed.checksum = 0;
+		RtChecksum sum;
+		sum.Add(&zeroed, sizeof(zeroed));
+		sum.Add(&b, sizeof(b));
+		sum.Add(sums, (size_t)sumBytes);
+		return sum.h;
+	}
+
+	// the sun a frame of `scene` is rendered with: the Scene object's as it is now, or the stored one of a flattened-scene file
+	void FrameSun(const Scene* scene, float illuminance[3], float direction[3])
+	{
+		const auto pre = g_prebuilt.find(scene);
+		if (pre != g_prebuilt.end())
+		{
+			memcpy(illuminance, pre->second->desc.sunIlluminance, 12);
+			memcpy(direction, pre->second->desc.sunDirection, 12);
+			return;
+		}
+		vec3 i, d;
+		scene->GetSun(i, d);
+		illuminance[0] = i.x; illuminance[1] = i.y; illuminance[2] = i.z;
+		direction[0] = d.x; direction[1] = d.y; direction[2] = d.z;
+	}
+
+	bool SceneFingerprint(const Scene* scene, int device, uint64_t* out)
+	{
+		if (!SceneOn(scene, device)) return false;
+		SceneEntry& entry = g_scenes[{ scene, device }];
+		if (!entry.fingerprinted)
+		{
+			if (rt_scene_fingerprint(entry.device, &entry.fingerprint) != 0)
+			{
+				RtGpu::SetLastError(std::string("rt_scene_fingerprint: ") + rt_last_error());
+				return false;
+			}
+			entry.fingerprinted = true;
+		}
+		*out = entry.fingerprint;
+		return true;
+	}
+
+	// every field in which two bindings differ ("" = none): an installment for another scene usually has another sun, too
+	std::string BindingDifference(const RtAccumBinding& a, const RtAccumBinding& b)
+	{
+		std::string fields;
+		auto differs = [&fields](bool different, const char* field) { if (different) fields += (fields.empty() ? "" : ", ") + std::string(field); };
+		differs(a.width != b.width || a.height != b.height, "viewport");
+		differs(a.maxPathLength != b.maxPathLength, "maxPathLength");
+		differs(memcmp(&a.rayTMin, &b.rayTMin, 4) != 0, "rayTMin");
+		differs(a.frameSeed != b.frameSeed, "frame seed");
+		differs(memcmp(&a.camera, &b.camera, sizeof(a.camera)) != 0, "camera");
+		differs(memcmp(a.sunIlluminance, b.sunIlluminance, 12) != 0 || memcmp(a.sunDirection, b.sunDirection, 12) != 0, "sun");
+		differs(a.sceneFingerprint != b.sceneFingerprint, "scene");
+		return fields;
+	}
+
+	RaylibB200Accumulator* NewAccumulator(uint32_t width, uint32_t height, const char* fn)
+	{
+		if (rt_device_count() <= 0) { RtGpu::SetLastError(kNoDevice); return nullptr; }
+		ResolveDevices();
+		std::unique_ptr<RaylibB200Accumulator> acc(new RaylibB200Accumulator);
+		memset(&acc->binding, 0, sizeof(acc->binding));
+		acc->device = g_devices[0];
+		acc->width = width; acc->height = height;
+		const uint64_t bytes = (uint64_t)width * height * 16ull;
+		if (rt_device_alloc(acc->device, bytes, &acc->sums) != 0 || rt_device_zero(acc->device, acc->sums, bytes) != 0)
+		{
+			RtGpu::SetLastError(std::string(fn) + "device allocation failed: " + rt_last_error());
+			if (acc->sums) rt_device_free(acc->device, acc->sums);
+			return nullptr;
+		}
+		return acc.release();
+	}
+}
+
+namespace RtGpu
+{
+	RaylibB200Accumulator* AccumulatorCreate(uint32_t width, uint32_t height)
+	{
+		std::lock_guard<std::recursive_mutex> lock(g_mutex);
+		t_lastError.clear();
+		if (width == 0 || height == 0 || (uint64_t)width * height >= (1ull << 31))
+		{
+			SetLastError("RaylibB200_AccumulatorCreate: size must be non-empty and below 2^31 pixels");
+			return nullptr;
+		}
+		return NewAccumulator(width, height, "RaylibB200_AccumulatorCreate: ");
+	}
+
+	void AccumulatorDestroy(RaylibB200Accumulator* acc)
+	{
+		std::lock_guard<std::recursive_mutex> lock(g_mutex);
+		if (!acc) return;
+		rt_device_free(acc->device, acc->sums);
+		delete acc;
+	}
+
+	bool AccumulatorReset(RaylibB200Accumulator* acc)
+	{
+		std::lock_guard<std::recursive_mutex> lock(g_mutex);
+		t_lastError.clear();
+		if (!acc) { SetLastError("RaylibB200_AccumulatorReset: null accumulator"); return false; }
+		if (rt_device_zero(acc->device, acc->sums, (uint64_t)acc->width * acc->height * 16ull) != 0)
+		{
+			SetLastError(std::string("RaylibB200_AccumulatorReset: ") + rt_last_error());
+			return false;
+		}
+		acc->samples = 0;
+		acc->bound = false;
+		memset(&acc->binding, 0, sizeof(acc->binding));
+		return true;
+	}
+
+	uint32_t AccumulatorSamples(const RaylibB200Accumulator* acc) { return acc ? acc->samples : 0u; }
+
+	bool RenderAccumulate(const RendererSettings* settings, const Scene* scene, const Camera* camera, RaylibB200Accumulator* acc, uint32_t samples)
+	{
+		std::lock_guard<std::recursive_mutex> lock(g_mutex);
+		t_lastError.clear();
+		const std::string fn = "RaylibB200_RenderAccumulate: ";
+		if (!settings || !scene || !camera || !acc) { SetLastError(fn + "null argument"); return false; }
+		if (samples == 0) { SetLastError(fn + "an installment renders at least one sample"); return false; }
+		if (settings->renderMode != 0u) { SetLastError(fn + "only renderMode 0 (path tracing) accumulates"); return false; }
+		if ((uint64_t)acc->samples + samples > kMaxAccumSamples) { SetLastError(fn + "more than 2^24 samples per pixel"); return false; }
+		if (DeviceCount() <= 0) { SetLastError(kNoDevice); return false; }
+		ResolveDevices();
+		const int primary = g_devices[0];
+		if (primary != acc->device)
+		{
+			SetLastError(fn + "the accumulator lives on GPU " + std::to_string(acc->device) + ", the first active device is GPU " + std::to_string(primary));
+			return false;
+		}
+
+		RtAccumBinding b;
+		memset(&b, 0, sizeof(b));
+		b.width = settings->viewportWidth; b.height = settings->viewportHeight;
+		b.maxPathLength = settings->maxPathLength;
+		b.rayTMin = settings->rayTMin;
+		b.frameSeed = g_frameSeed;
+		RtFlattenCamera(camera, b.camera);
+		FrameSun(scene, b.sunIlluminance, b.sunDirection);
+		if (b.width != acc->width || b.height != acc->height)
+		{
+			SetLastError(fn + "viewport " + std::to_string(b.width) + "x" + std::to_string(b.height) + " differs from the accumulator's " +
+			             std::to_string(acc->width) + "x" + std::to_string(acc->height));
+			return false;
+		}
+		if (!SceneFingerprint(scene, primary, &b.sceneFingerprint)) return false;
+		if (acc->bound)
+		{
+			const std::string fields = BindingDifference(acc->binding, b);
+			if (!fields.empty())
+			{
+				SetLastError(fn + "the accumulated image's " + fields + (fields.find(',') == std::string::npos ? " differs" : " differ") +
+				             " from this installment's; Reset the accumulator to start a new image");
+				return false;
+			}
+		}
+
+		const SampleWindow window = { acc->samples, acc->samples + samples, acc->sums };
+		if (!Render(settings, scene, camera, nullptr, nullptr, nullptr, 0, 1, 0, nullptr, false, &window)) return false;
+		acc->binding = b;
+		acc->bound = true;
+		acc->samples += samples;
+		return true;
+	}
+
+	bool AccumulatorResolve(RaylibB200Accumulator* acc, Image2D* hostImage, void* deviceImage, void* stream)
+	{
+		std::lock_guard<std::recursive_mutex> lock(g_mutex);
+		t_lastError.clear();
+		const std::string fn = "RaylibB200_AccumulatorResolve: ";
+		if (!acc || (!hostImage && !deviceImage)) { SetLastError(fn + "null argument"); return false; }
+		if (acc->samples == 0) { SetLastError(fn + "the accumulator holds no samples"); return false; }
+		const uint64_t count = (uint64_t)acc->width * acc->height, bytes = count * 16ull;
+		if (deviceImage)
+		{
+			if (rt_resolve(acc->device, acc->sums, (uint32_t)count, acc->samples, deviceImage, nullptr, nullptr, stream) != 0)
+			{
+				SetLastError(fn + rt_last_error());
+				return false;
+			}
+			return true;
+		}
+		if (hostImage->GetWidth() != acc->width || hostImage->GetHeight() != acc->height) hostImage->Reallocate(acc->width, acc->height);
+		void* image = ScratchBuffer(acc->device, 1, bytes);
+		if (!image) { SetLastError(fn + "device allocation failed: " + rt_last_error()); return false; }
+		if (rt_resolve(acc->device, acc->sums, (uint32_t)count, acc->samples, image, nullptr, nullptr, nullptr) != 0 ||
+		    rt_copy_to_host(acc->device, hostImage->MutablePixels(), image, bytes, nullptr) != 0)
+		{
+			SetLastError(fn + rt_last_error());
+			return false;
+		}
+		return true;
+	}
+
+	bool AccumulatorRead(RaylibB200Accumulator* acc, float* rgba)
+	{
+		std::lock_guard<std::recursive_mutex> lock(g_mutex);
+		t_lastError.clear();
+		if (!acc || !rgba) { SetLastError("RaylibB200_AccumulatorRead: null argument"); return false; }
+		if (rt_copy_to_host(acc->device, rgba, acc->sums, (uint64_t)acc->width * acc->height * 16ull, nullptr) != 0)
+		{
+			SetLastError(std::string("RaylibB200_AccumulatorRead: ") + rt_last_error());
+			return false;
+		}
+		return true;
+	}
+
+	bool AccumulatorNoise(RaylibB200Accumulator* acc, float* perPixel, double* mean)
+	{
+		std::lock_guard<std::recursive_mutex> lock(g_mutex);
+		t_lastError.clear();
+		const std::string fn = "RaylibB200_AccumulatorNoise: ";
+		if (!acc) { SetLastError(fn + "null accumulator"); return false; }
+		if (acc->samples < 2) { SetLastError(fn + "the noise figure needs at least 2 samples per pixel"); return false; }
+		const uint64_t count = (uint64_t)acc->width * acc->height;
+		float* noise = nullptr;
+		if (perPixel && !(noise = (float*)ScratchBuffer(acc->device, 4, count * 4ull))) { SetLastError(fn + "device allocation failed: " + rt_last_error()); return false; }
+		double total = 0.0;
+		if (rt_resolve(acc->device, acc->sums, (uint32_t)count, acc->samples, nullptr, noise, mean ? &total : nullptr, nullptr) != 0 ||
+		    (perPixel && rt_copy_to_host(acc->device, perPixel, noise, count * 4ull, nullptr) != 0))
+		{
+			SetLastError(fn + rt_last_error());
+			return false;
+		}
+		if (mean) *mean = total / (double)count;
+		return true;
+	}
+
+	bool AccumulatorSave(const RaylibB200Accumulator* acc, const char* path)
+	{
+		std::lock_guard<std::recursive_mutex> lock(g_mutex);
+		t_lastError.clear();
+		const std::string fn = "RaylibB200_AccumulatorSave: ";
+		if (!acc || !path || !*path) { SetLastError(fn + "null accumulator or empty path"); return false; }
+		const uint64_t sumBytes = (uint64_t)acc->width * acc->height * 16ull;
+		std::vector<float> sums((size_t)(sumBytes / 4));
+		if (rt_copy_to_host(acc->device, sums.data(), acc->sums, sumBytes, nullptr) != 0) { SetLastError(fn + rt_last_error()); return false; }
+		AccumFileHeader h;
+		memset(&h, 0, sizeof(h));
+		memcpy(h.magic, "RTACCUM1", 8);
+		h.headerBytes = sizeof(h); h.bindingBytes = sizeof(RtAccumBinding);
+		h.width = acc->width; h.height = acc->height; h.samples = acc->samples; h.bound = acc->bound ? 1u : 0u;
+		h.checksum = AccumFileChecksum(h, acc->binding, sums.data(), sumBytes);
+		const std::string tmp = std::string(path) + ".tmp";
+		FILE* f = fopen(tmp.c_str(), "wb");
+		if (!f) { SetLastError(fn + "cannot create " + tmp); return false; }
+		bool ok = fwrite(&h, 1, sizeof(h), f) == sizeof(h) && fwrite(&acc->binding, 1, sizeof(acc->binding), f) == sizeof(acc->binding) &&
+		          fwrite(sums.data(), 1, (size_t)sumBytes, f) == (size_t)sumBytes;
+		ok = (fclose(f) == 0) && ok;
+		if (!ok || rename(tmp.c_str(), path) != 0) { remove(tmp.c_str()); SetLastError(fn + "write failed: " + path); return false; }
+		return true;
+	}
+
+	RaylibB200Accumulator* AccumulatorLoad(const char* path)
+	{
+		std::lock_guard<std::recursive_mutex> lock(g_mutex);
+		t_lastError.clear();
+		const std::string fn = std::string("RaylibB200_AccumulatorLoad: ") + (path ? path : "(null)") + ": ";
+		FILE* f = path ? fopen(path, "rb") : nullptr;
+		if (!f) { SetLastError(fn + "cannot open"); return nullptr; }
+		AccumFileHeader h;
+		RtAccumBinding b;
+		std::vector<float> sums;
+		std::string why;
+		if (fread(&h, 1, sizeof(h), f) != sizeof(h) || memcmp(h.magic, "RTACCUM1", 8) != 0) why = "not an accumulator checkpoint file";
+		else if (h.headerBytes != sizeof(h) || h.bindingBytes != sizeof(b)) why = "checkpoint written by a build with a different format";
+		else if (h.width == 0 || h.height == 0 || (uint64_t)h.width * h.height >= (1ull << 31) || h.bound > 1u ||
+		         h.samples > kMaxAccumSamples || (h.samples > 0u) != (h.bound != 0u))
+			why = "checkpoint header is inconsistent";
+		else
+		{
+			const uint64_t sumBytes = (uint64_t)h.width * h.height * 16ull;
+			const uint64_t expect = sizeof(h) + sizeof(b) + sumBytes;
+			long size = -1;
+			if (fseek(f, 0, SEEK_END) == 0) size = ftell(f);
+			if (size < 0 || fseek(f, (long)sizeof(h), SEEK_SET) != 0) why = "cannot read";
+			else if ((uint64_t)size < expect) why = "checkpoint is truncated";
+			else if ((uint64_t)size > expect) why = "checkpoint has trailing bytes";
+			else
+			{
+				sums.resize((size_t)(sumBytes / 4));
+				if (fread(&b, 1, sizeof(b), f) != sizeof(b) || fread(sums.data(), 1, (size_t)sumBytes, f) != (size_t)sumBytes) why = "checkpoint is truncated";
+				else if (AccumFileChecksum(h, b, sums.data(), sumBytes) != h.checksum) why = "checkpoint is corrupt (checksum mismatch)";
+				else if (h.bound && (b.width != h.width || b.height != h.height)) why = "checkpoint header is inconsistent";
+			}
+		}
+		fclose(f);
+		if (!why.empty()) { SetLastError(fn + why); return nullptr; }
+		RaylibB200Accumulator* acc = NewAccumulator(h.width, h.height, fn.c_str());
+		if (!acc) return nullptr;
+		if (rt_copy_to_device(acc->device, acc->sums, sums.data(), (uint64_t)sums.size() * 4ull, nullptr) != 0)
+		{
+			SetLastError(fn + rt_last_error());
+			AccumulatorDestroy(acc);
+			return nullptr;
+		}
+		acc->samples = h.samples;
+		acc->bound = h.bound != 0u;
+		acc->binding = b;
+		return acc;
 	}
 }
 

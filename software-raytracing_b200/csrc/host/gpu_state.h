@@ -47,11 +47,28 @@ namespace RtGpu
 	std::shared_ptr<RtFlatScene> Prebuilt(const Scene* scene);
 	void ReleaseAll();
 
+	// Samples [begin, end) of a whole frame added to the running sums of an accumulator (row-major W x H float4 on the
+	// primary device): rt_render_window of rt_progressive.h.
+	struct SampleWindow { uint32_t begin, end; void* sums; };
+
 	// Shared implementation of every render entry point.  Exactly one of hostImage / deviceImage /
-	// deviceShard is non-null.
+	// deviceShard / window is non-null.
 	bool Render(const RendererSettings* settings, const Scene* scene, const Camera* camera,
 	            Image2D* hostImage, void* deviceImage, void* deviceShard,
-	            uint32_t shardRank, uint32_t shardCount, uint32_t renderModeOverride, void* stream, bool pinHostImage = false);
+	            uint32_t shardRank, uint32_t shardCount, uint32_t renderModeOverride, void* stream, bool pinHostImage = false,
+	            const SampleWindow* window = nullptr);
+
+	// Progressive rendering (RaylibB200_Accumulator*, include/raylib_b200.h)
+	RaylibB200Accumulator* AccumulatorCreate(uint32_t width, uint32_t height);
+	void AccumulatorDestroy(RaylibB200Accumulator* acc);
+	bool AccumulatorReset(RaylibB200Accumulator* acc);
+	uint32_t AccumulatorSamples(const RaylibB200Accumulator* acc);
+	bool RenderAccumulate(const RendererSettings* settings, const Scene* scene, const Camera* camera, RaylibB200Accumulator* acc, uint32_t samples);
+	bool AccumulatorResolve(RaylibB200Accumulator* acc, Image2D* hostImage, void* deviceImage, void* stream);
+	bool AccumulatorRead(RaylibB200Accumulator* acc, float* rgba);
+	bool AccumulatorNoise(RaylibB200Accumulator* acc, float* perPixel, double* mean);
+	bool AccumulatorSave(const RaylibB200Accumulator* acc, const char* path);
+	RaylibB200Accumulator* AccumulatorLoad(const char* path);
 
 	// Denoiser inputs in one primary-hit pass (reference: the Albedo and MicrosurfaceNormal debug renders of
 	// src/main.cc:464-476, two extra Raylib_Render calls).  Host images are resized to the viewport.

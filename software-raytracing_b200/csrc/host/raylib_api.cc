@@ -390,6 +390,29 @@ SceneHandle RaylibB200_LoadFlattenedScene(const char* path)
 	return (SceneHandle)scene;
 }
 
+RaylibB200Accumulator* RaylibB200_AccumulatorCreate(uint32_t width, uint32_t height) { return RtGpu::AccumulatorCreate(width, height); }
+void RaylibB200_AccumulatorDestroy(RaylibB200Accumulator* acc) { RtGpu::AccumulatorDestroy(acc); }
+int32_t RaylibB200_AccumulatorReset(RaylibB200Accumulator* acc) { return RtGpu::AccumulatorReset(acc) ? 1 : 0; }
+uint32_t RaylibB200_AccumulatorSamples(const RaylibB200Accumulator* acc) { return RtGpu::AccumulatorSamples(acc); }
+int32_t RaylibB200_RenderAccumulate(const RendererSettings* settings, SceneHandle scene, CameraHandle camera, RaylibB200Accumulator* acc, uint32_t samples)
+{
+	return RtGpu::RenderAccumulate(settings, (const Scene*)scene, (const Camera*)camera, acc, samples) ? 1 : 0;
+}
+int32_t RaylibB200_AccumulatorResolve(RaylibB200Accumulator* acc, ImageHandle outImage)
+{
+	if (!outImage) { RtGpu::SetLastError("RaylibB200_AccumulatorResolve: null image"); return 0; }
+	return RtGpu::AccumulatorResolve(acc, (Image2D*)outImage, nullptr, nullptr) ? 1 : 0;
+}
+int32_t RaylibB200_AccumulatorResolveDevice(RaylibB200Accumulator* acc, void* deviceImageOut, void* cudaStream)
+{
+	if (!deviceImageOut) { RtGpu::SetLastError("RaylibB200_AccumulatorResolveDevice: null image"); return 0; }
+	return RtGpu::AccumulatorResolve(acc, nullptr, deviceImageOut, cudaStream) ? 1 : 0;
+}
+int32_t RaylibB200_AccumulatorRead(RaylibB200Accumulator* acc, float* outRgba) { return RtGpu::AccumulatorRead(acc, outRgba) ? 1 : 0; }
+int32_t RaylibB200_AccumulatorNoise(RaylibB200Accumulator* acc, float* perPixel, double* mean) { return RtGpu::AccumulatorNoise(acc, perPixel, mean) ? 1 : 0; }
+int32_t RaylibB200_AccumulatorSave(const RaylibB200Accumulator* acc, const char* path) { return RtGpu::AccumulatorSave(acc, path) ? 1 : 0; }
+RaylibB200Accumulator* RaylibB200_AccumulatorLoad(const char* path) { return RtGpu::AccumulatorLoad(path); }
+
 int32_t RaylibB200_CameraBlock(CameraHandle camera, RtCamera* out)
 {
 	if (!camera || !out) return 0;

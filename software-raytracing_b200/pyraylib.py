@@ -173,6 +173,17 @@ B200_C_API = {
     "RaylibB200_ReleaseInspection": (None, [H]),
     "RaylibB200_CameraBlock": (C.c_int32, [H, C.POINTER(RtCamera)]),
     "RaylibB200_SeedHostRandom": (None, [C.c_uint64]),
+    "RaylibB200_AccumulatorCreate": (C.c_void_p, [C.c_uint32, C.c_uint32]),
+    "RaylibB200_AccumulatorDestroy": (None, [C.c_void_p]),
+    "RaylibB200_AccumulatorReset": (C.c_int32, [C.c_void_p]),
+    "RaylibB200_AccumulatorSamples": (C.c_uint32, [C.c_void_p]),
+    "RaylibB200_RenderAccumulate": (C.c_int32, [C.POINTER(RendererSettings), H, H, C.c_void_p, C.c_uint32]),
+    "RaylibB200_AccumulatorResolve": (C.c_int32, [C.c_void_p, H]),
+    "RaylibB200_AccumulatorResolveDevice": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "RaylibB200_AccumulatorRead": (C.c_int32, [C.c_void_p, _F32P]),
+    "RaylibB200_AccumulatorNoise": (C.c_int32, [C.c_void_p, C.c_void_p, C.POINTER(C.c_double)]),
+    "RaylibB200_AccumulatorSave": (C.c_int32, [C.c_void_p, C.c_char_p]),
+    "RaylibB200_AccumulatorLoad": (C.c_void_p, [C.c_char_p]),
 }
 
 SCENES_API = {
@@ -288,6 +299,37 @@ class Product(_Base):
         cam = RtCamera()
         self.lib.RaylibB200_CameraBlock(camera, C.byref(cam))
         return cam
+
+    # ---- progressive rendering (RaylibB200_Accumulator*): acc is the handle of RaylibB200_AccumulatorCreate / _Load
+    def accumulate(self, settings, scene, camera, acc, samples):
+        """Renders `samples` more samples of every pixel into the accumulator; raises when the call is refused."""
+        if not self.lib.RaylibB200_RenderAccumulate(C.byref(settings), scene, camera, acc, samples):
+            raise RuntimeError("RaylibB200_RenderAccumulate failed: " + self.last_error())
+
+    def resolve(self, acc, width, height):
+        """The running average (RaylibB200_AccumulatorResolve): H x W x 3 float32, the bits Raylib_Render gives at n spp."""
+        img = self.lib.Raylib_CreateImage(1, 1)          # resized by the resolve, as Raylib_Render resizes its output
+        try:
+            if not self.lib.RaylibB200_AccumulatorResolve(acc, img):
+                raise RuntimeError("RaylibB200_AccumulatorResolve failed: " + self.last_error())
+            return self.dump_image(img, width, height)
+        finally:
+            self.lib.Raylib_DestroyImage(img)
+
+    def accumulator_sums(self, acc, width, height):
+        """Raw sums: H x W x 4 float32 {sum R, sum G, sum B, sum luminance^2}."""
+        out = np.empty((height, width, 4), dtype=np.float32)
+        if not self.lib.RaylibB200_AccumulatorRead(acc, out):
+            raise RuntimeError("RaylibB200_AccumulatorRead failed: " + self.last_error())
+        return out
+
+    def noise(self, acc, width, height):
+        """(H x W float32 relative standard error of each pixel's mean luminance, their mean as a float)."""
+        out = np.empty((height, width), dtype=np.float32)
+        mean = C.c_double()
+        if not self.lib.RaylibB200_AccumulatorNoise(acc, out.ctypes.data, C.byref(mean)):
+            raise RuntimeError("RaylibB200_AccumulatorNoise failed: " + self.last_error())
+        return out, mean.value
 
 
 def device_source_hash():
