@@ -178,6 +178,32 @@ RAYLIB_API int32_t RaylibB200_AccumulatorNoise(RaylibB200Accumulator* acc, float
 RAYLIB_API int32_t RaylibB200_AccumulatorSave(const RaylibB200Accumulator* acc, const char* path);
 RAYLIB_API RaylibB200Accumulator* RaylibB200_AccumulatorLoad(const char* path);
 
+// ---- denoising: the step between RenderAux and post-processing ------------------------------------------
+// An edge-avoiding a-trous filter guided by the albedo and normal views RaylibB200_RenderAux writes (spatial SVGF without
+// its temporal part; DESIGN.md section 14): the colour is divided by the albedo, filtered in five iterations weighted by
+// normal agreement and by luminance distance over the estimated noise, and multiplied back.  A null albedo image counts as
+// 1 everywhere; a null normal image makes every pixel a surface facing +z.  Normals are encoded 0.5 + 0.5 N, (0,0,0)
+// marking a miss.  The output (alpha 1) is a pure function of the inputs: the same inputs give the same bits on every
+// call.  All three calls are synchronous and return 1 on success or 0 (GetLastError); their arguments are checked before
+// a device is used.  GetLastStats reports the call (device and wall time, launches, copies; no rays).
+// Noise estimate: the image and device forms only have the image, so they estimate each pixel's variance spatially, over
+// its 7 x 7 neighbourhood.  That counts real high-frequency detail (fine geometry, texture, shadow edges) as noise and can
+// blur it, making such scenes worse than the raw frame (measured: scatter10M and the textured room, DESIGN.md section 14).
+// When the frame comes from an accumulator, prefer RaylibB200_AccumulatorDenoise: it uses each pixel's exact sample
+// variance and keeps that detail.
+// Raylib_Denoise's image arguments (raylib/raylib.h) without the HDR flag: the filter does not depend on the range.
+// outImage is resized to the main image's size; albedo and normal must have that size.  Raylib_Denoise keeps returning 0.
+RAYLIB_API int32_t RaylibB200_Denoise(ImageHandle mainImage, ImageHandle albedoImage, ImageHandle normalImage, ImageHandle outImage);
+// W x H RGBA float4 images in device memory of the current device (albedo and normal nullable), each 16-byte aligned
+// (a misaligned pointer is refused); cudaStream may be NULL.
+RAYLIB_API int32_t RaylibB200_DenoiseDevice(const void* deviceColor, const void* deviceAlbedo, const void* deviceNormal,
+	uint32_t width, uint32_t height, void* deviceOut, void* cudaStream);
+// The accumulator's resolved image, filtered with the exact per-pixel variance of its mean from the sums (divided by the
+// squared luminance of the albedo: exact for grey albedo, an approximation for coloured).  Reads the sums in place and
+// leaves them and n untouched.  Needs n >= 2; guides must have the accumulator's size.
+RAYLIB_API int32_t RaylibB200_AccumulatorDenoise(RaylibB200Accumulator* acc, ImageHandle albedoImage, ImageHandle normalImage,
+	ImageHandle outImage);
+
 // ---- queries used by parity tests ---------------------------------------------------------------
 // Closest hit of caller-supplied rays (8 floats each: o.xyz, time, d.xyz, unused).  outRank = global
 // in-order leaf rank of the hit primitive or -1; outT = hit distance or 0.

@@ -6,6 +6,7 @@
 #include "host_internal.h"
 #include "rt_checksum.h"
 #include "rt_progressive.h"
+#include "rt_denoise.h"
 #include "geom/scene.h"
 #include "render/camera.h"
 #include "render/image.h"
@@ -756,6 +757,126 @@ namespace RtGpu
 	}
 }
 
+// ---------------------------------------------------------------------------------------------
+// Denoising (DESIGN.md section 14): the filter of rt_denoise.h over device images, host images or an accumulator's sums
+
+namespace
+{
+	const int kDenoiseScratchSlot = 5;      // the filter's records (rt_denoise_scratch_bytes)
+	const int kDenoiseImageSlot = 6;        // device copies of a host call's images: colour, albedo, normal, output
+
+	// "" or why a guide image cannot go with a W x H colour image
+	std::string GuideSizeError(const Image2D* guide, const char* name, uint32_t width, uint32_t height, const char* against)
+	{
+		if (!guide || (guide->GetWidth() == width && guide->GetHeight() == height)) return "";
+		return std::string("the ") + name + " image is " + std::to_string(guide->GetWidth()) + "x" + std::to_string(guide->GetHeight()) +
+		       ", " + against + " is " + std::to_string(width) + "x" + std::to_string(height);
+	}
+
+	// Uploads the non-null host images of `images` into consecutive W x H float4 images of the slot buffer (which also
+	// holds the output, returned in *out); NULL stays NULL.
+	bool UploadDenoiseImages(const std::string& fn, int device, const Image2D* const images[3], uint64_t bytes, void* dev[3],
+	                         void** out, RaylibB200Stats& st)
+	{
+		char* base = (char*)ScratchBuffer(device, kDenoiseImageSlot, 4 * bytes);
+		if (!base) { RtGpu::SetLastError(fn + "device allocation failed: " + rt_last_error()); return false; }
+		for (int k = 0; k < 3; ++k)
+		{
+			dev[k] = nullptr;
+			if (!images[k]) continue;
+			dev[k] = base + k * bytes;
+			if (rt_copy_to_device(device, dev[k], images[k]->GetPixelArray().data(), bytes, nullptr) != 0)
+			{
+				RtGpu::SetLastError(fn + rt_last_error());
+				return false;
+			}
+			st.h2dBytes += bytes;
+		}
+		*out = base + 3 * bytes;
+		return true;
+	}
+
+	// rt_denoise (n == 0) or rt_denoise_sums on device images of `device`; fills the device part of the statistics
+	bool RunDenoise(const std::string& fn, int device, const void* color, uint32_t n, const void* albedo, const void* normal,
+	                uint32_t width, uint32_t height, void* out, void* stream, RaylibB200Stats& st)
+	{
+		void* scratch = ScratchBuffer(device, kDenoiseScratchSlot, rt_denoise_scratch_bytes(width, height));
+		if (!scratch) { RtGpu::SetLastError(fn + "device allocation failed: " + rt_last_error()); return false; }
+		const int rc = n ? rt_denoise_sums(device, color, n, albedo, normal, width, height, scratch, out, stream, &st.deviceMs)
+		                 : rt_denoise(device, color, albedo, normal, width, height, scratch, out, stream, &st.deviceMs);
+		if (rc != 0) { RtGpu::SetLastError(fn + rt_denoise_last_error()); return false; }
+		st.kernelLaunches = RT_DENOISE_LAUNCHES;
+		st.device = (uint32_t)device;
+		st.devicesUsed = 1;
+		return true;
+	}
+
+	// The result of a host call: read back into `out`, resized to W x H only now that the filter has run
+	bool ReadDenoised(const std::string& fn, int device, const void* image, uint32_t width, uint32_t height, Image2D* out, RaylibB200Stats& st)
+	{
+		if (out->GetWidth() != width || out->GetHeight() != height) out->Reallocate(width, height);
+		const uint64_t bytes = (uint64_t)width * height * 16ull;
+		if (rt_copy_to_host(device, out->MutablePixels(), image, bytes, nullptr) != 0) { RtGpu::SetLastError(fn + rt_last_error()); return false; }
+		st.d2hBytes += bytes;
+		return true;
+	}
+
+	double MsSince(std::chrono::steady_clock::time_point t0)
+	{
+		return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+	}
+}
+
+namespace RtGpu
+{
+	bool Denoise(const Image2D* color, const Image2D* albedo, const Image2D* normal, Image2D* out)
+	{
+		std::lock_guard<std::recursive_mutex> lock(g_mutex);
+		const auto wall0 = std::chrono::steady_clock::now();
+		t_lastError.clear();
+		const std::string fn = "RaylibB200_Denoise: ";
+		if (!color || !out) { SetLastError(fn + "null main or output image"); return false; }
+		const uint32_t W = color->GetWidth(), H = color->GetHeight();
+		if (W == 0 || H == 0 || (uint64_t)W * H >= (1ull << 31)) { SetLastError(fn + "the main image must be non-empty and below 2^31 pixels"); return false; }
+		for (const std::string& why : { GuideSizeError(albedo, "albedo", W, H, "the main image"), GuideSizeError(normal, "normal", W, H, "the main image") })
+			if (!why.empty()) { SetLastError(fn + why); return false; }
+		if (DeviceCount() <= 0) { SetLastError("no CUDA device is available; this library renders on the GPU only (no CPU path)"); return false; }
+		const int device = CurrentDevice();
+		RaylibB200Stats st;
+		memset(&st, 0, sizeof(st));
+		const Image2D* images[3] = { color, albedo, normal };
+		void* dev[3];
+		void* image = nullptr;
+		if (!UploadDenoiseImages(fn, device, images, (uint64_t)W * H * 16ull, dev, &image, st) ||
+		    !RunDenoise(fn, device, dev[0], 0, dev[1], dev[2], W, H, image, nullptr, st) ||
+		    !ReadDenoised(fn, device, image, W, H, out, st))
+			return false;
+		st.totalMs = MsSince(wall0);
+		SetLastStats(st);
+		return true;
+	}
+
+	bool DenoiseDevice(const void* color, const void* albedo, const void* normal, uint32_t width, uint32_t height, void* out, void* stream)
+	{
+		std::lock_guard<std::recursive_mutex> lock(g_mutex);
+		const auto wall0 = std::chrono::steady_clock::now();
+		t_lastError.clear();
+		const std::string fn = "RaylibB200_DenoiseDevice: ";
+		if (!color || !out) { SetLastError(fn + "null colour or output image"); return false; }
+		if (width == 0 || height == 0 || (uint64_t)width * height >= (1ull << 31)) { SetLastError(fn + "the image must be non-empty and below 2^31 pixels"); return false; }
+		// the kernels read and write whole float4 pixels: a misaligned view (a sliced tensor) is refused here, not faulted on
+		for (const void* p : { color, albedo, normal, (const void*)out })
+			if ((uintptr_t)p % 16u != 0) { SetLastError(fn + "device images must be 16-byte aligned (RGBA float4 pixels)"); return false; }
+		if (DeviceCount() <= 0) { SetLastError("no CUDA device is available; this library renders on the GPU only (no CPU path)"); return false; }
+		RaylibB200Stats st;
+		memset(&st, 0, sizeof(st));
+		if (!RunDenoise(fn, CurrentDevice(), color, 0, albedo, normal, width, height, out, stream, st)) return false;
+		st.totalMs = MsSince(wall0);
+		SetLastStats(st);
+		return true;
+	}
+}
+
 namespace RtGpu
 {
 	void AdoptPrebuilt(const Scene* scene, std::shared_ptr<RtFlatScene> flat)
@@ -1011,6 +1132,31 @@ namespace RtGpu
 			SetLastError(fn + rt_last_error());
 			return false;
 		}
+		return true;
+	}
+
+	bool AccumulatorDenoise(RaylibB200Accumulator* acc, const Image2D* albedo, const Image2D* normal, Image2D* out)
+	{
+		std::lock_guard<std::recursive_mutex> lock(g_mutex);
+		const auto wall0 = std::chrono::steady_clock::now();
+		t_lastError.clear();
+		const std::string fn = "RaylibB200_AccumulatorDenoise: ";
+		if (!acc || !out) { SetLastError(fn + "null accumulator or output image"); return false; }
+		if (acc->samples < 2) { SetLastError(fn + "the variance needs at least 2 samples per pixel"); return false; }
+		const uint32_t W = acc->width, H = acc->height;
+		for (const std::string& why : { GuideSizeError(albedo, "albedo", W, H, "the accumulator"), GuideSizeError(normal, "normal", W, H, "the accumulator") })
+			if (!why.empty()) { SetLastError(fn + why); return false; }
+		RaylibB200Stats st;
+		memset(&st, 0, sizeof(st));
+		const Image2D* images[3] = { nullptr, albedo, normal };
+		void* dev[3];
+		void* image = nullptr;
+		if (!UploadDenoiseImages(fn, acc->device, images, (uint64_t)W * H * 16ull, dev, &image, st) ||
+		    !RunDenoise(fn, acc->device, acc->sums, acc->samples, dev[1], dev[2], W, H, image, nullptr, st) ||
+		    !ReadDenoised(fn, acc->device, image, W, H, out, st))
+			return false;
+		st.totalMs = MsSince(wall0);
+		SetLastStats(st);
 		return true;
 	}
 

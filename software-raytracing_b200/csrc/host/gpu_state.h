@@ -65,6 +65,8 @@ namespace RtGpu
 	uint32_t AccumulatorSamples(const RaylibB200Accumulator* acc);
 	bool RenderAccumulate(const RendererSettings* settings, const Scene* scene, const Camera* camera, RaylibB200Accumulator* acc, uint32_t samples);
 	bool AccumulatorResolve(RaylibB200Accumulator* acc, Image2D* hostImage, void* deviceImage, void* stream);
+	// The denoiser (rt_denoise_sums of rt_denoise.h) on the sums, which it leaves as they are; n >= 2, guides nullable.
+	bool AccumulatorDenoise(RaylibB200Accumulator* acc, const Image2D* albedo, const Image2D* normal, Image2D* out);
 	bool AccumulatorRead(RaylibB200Accumulator* acc, float* rgba);
 	bool AccumulatorNoise(RaylibB200Accumulator* acc, float* perPixel, double* mean);
 	bool AccumulatorSave(const RaylibB200Accumulator* acc, const char* path);
@@ -78,4 +80,9 @@ namespace RtGpu
 	bool PostProcessDevice(void* deviceImage, uint32_t width, uint32_t height, void* deviceOutArgb8, float* outMaxWhite, void* stream);
 	// Same for a host Image2D (H2D, kernels, D2H); used for large frames.
 	bool PostProcessHostImage(Image2D* image);
+
+	// The denoiser (rt_denoise of rt_denoise.h) on host images (H2D, kernels, D2H; out is resized to the colour image) or on
+	// W x H RGBA float4 images on the current device.  Guides are nullable.  Arguments are checked before a device is used.
+	bool Denoise(const Image2D* color, const Image2D* albedo, const Image2D* normal, Image2D* out);
+	bool DenoiseDevice(const void* color, const void* albedo, const void* normal, uint32_t width, uint32_t height, void* out, void* stream);
 }

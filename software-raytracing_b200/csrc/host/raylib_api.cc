@@ -408,6 +408,10 @@ int32_t RaylibB200_AccumulatorResolveDevice(RaylibB200Accumulator* acc, void* de
 	if (!deviceImageOut) { RtGpu::SetLastError("RaylibB200_AccumulatorResolveDevice: null image"); return 0; }
 	return RtGpu::AccumulatorResolve(acc, nullptr, deviceImageOut, cudaStream) ? 1 : 0;
 }
+int32_t RaylibB200_AccumulatorDenoise(RaylibB200Accumulator* acc, ImageHandle albedoImage, ImageHandle normalImage, ImageHandle outImage)
+{
+	return RtGpu::AccumulatorDenoise(acc, (const Image2D*)albedoImage, (const Image2D*)normalImage, (Image2D*)outImage) ? 1 : 0;
+}
 int32_t RaylibB200_AccumulatorRead(RaylibB200Accumulator* acc, float* outRgba) { return RtGpu::AccumulatorRead(acc, outRgba) ? 1 : 0; }
 int32_t RaylibB200_AccumulatorNoise(RaylibB200Accumulator* acc, float* perPixel, double* mean) { return RtGpu::AccumulatorNoise(acc, perPixel, mean) ? 1 : 0; }
 int32_t RaylibB200_AccumulatorSave(const RaylibB200Accumulator* acc, const char* path) { return RtGpu::AccumulatorSave(acc, path) ? 1 : 0; }
@@ -602,6 +606,16 @@ int32_t RaylibB200_LibmEval(int32_t fn, const float* x, const float* y, float* o
 }
 
 int32_t RaylibB200_PostProcessGPU(ImageHandle image) { return RtGpu::PostProcessHostImage((Image2D*)image) ? 1 : 0; }
+
+int32_t RaylibB200_Denoise(ImageHandle mainImage, ImageHandle albedoImage, ImageHandle normalImage, ImageHandle outImage)
+{
+	return RtGpu::Denoise((const Image2D*)mainImage, (const Image2D*)albedoImage, (const Image2D*)normalImage, (Image2D*)outImage) ? 1 : 0;
+}
+
+int32_t RaylibB200_DenoiseDevice(const void* color, const void* albedo, const void* normal, uint32_t width, uint32_t height, void* out, void* cudaStream)
+{
+	return RtGpu::DenoiseDevice(color, albedo, normal, width, height, out, cudaStream) ? 1 : 0;
+}
 
 int32_t RaylibB200_TraceRays(SceneHandle scene, const float* rays, int64_t numRays, float tMin, int32_t* outRank, float* outT)
 {

@@ -184,6 +184,9 @@ B200_C_API = {
     "RaylibB200_AccumulatorNoise": (C.c_int32, [C.c_void_p, C.c_void_p, C.POINTER(C.c_double)]),
     "RaylibB200_AccumulatorSave": (C.c_int32, [C.c_void_p, C.c_char_p]),
     "RaylibB200_AccumulatorLoad": (C.c_void_p, [C.c_char_p]),
+    "RaylibB200_Denoise": (C.c_int32, [H, H, H, H]),
+    "RaylibB200_DenoiseDevice": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p]),
+    "RaylibB200_AccumulatorDenoise": (C.c_int32, [C.c_void_p, H, H, H]),
 }
 
 SCENES_API = {
@@ -330,6 +333,57 @@ class Product(_Base):
         if not self.lib.RaylibB200_AccumulatorNoise(acc, out.ctypes.data, C.byref(mean)):
             raise RuntimeError("RaylibB200_AccumulatorNoise failed: " + self.last_error())
         return out, mean.value
+
+    # ---- denoising (RaylibB200_Denoise, _DenoiseDevice, _AccumulatorDenoise): guides are the albedo and encoded-normal
+    # views of RaylibB200_RenderAux, or None
+    def image_from_array(self, a):
+        """A new image handle holding an H x W x 3 or 4 float32 array (alpha 1 when absent); destroy with Raylib_DestroyImage."""
+        a = np.asarray(a, dtype=np.float32)
+        rgba = np.ones(a.shape[:2] + (4,), dtype=np.float32)
+        rgba[:, :, :a.shape[2]] = a
+        img = self.lib.Raylib_CreateImage(1, 1)
+        self.lib.RaylibB200_ImageSetRGBA(img, a.shape[1], a.shape[0], rgba)
+        return img
+
+    def _denoise_host(self, call, name, height, width, guides):
+        handles = [self.image_from_array(g) if g is not None else 0 for g in guides]
+        out = self.lib.Raylib_CreateImage(1, 1)          # resized by the call
+        try:
+            if not call(*handles, out):
+                raise RuntimeError(name + " failed: " + self.last_error())
+            rgba = np.empty((height, width, 4), dtype=np.float32)
+            self.lib.RaylibB200_ImageGetRGBA(out, rgba)
+            return rgba[:, :, :3].copy()
+        finally:
+            for h in handles + [out]:
+                if h:
+                    self.lib.Raylib_DestroyImage(h)
+
+    def denoise(self, color, albedo=None, normal=None):
+        """RaylibB200_Denoise on H x W x 3 or 4 float32 arrays: H x W x 3 float32."""
+        color = np.asarray(color, dtype=np.float32)
+        main = self.image_from_array(color)
+        try:
+            return self._denoise_host(lambda a, n, out: self.lib.RaylibB200_Denoise(main, a, n, out), "RaylibB200_Denoise",
+                                      color.shape[0], color.shape[1], (albedo, normal))
+        finally:
+            self.lib.Raylib_DestroyImage(main)
+
+    def denoise_device(self, color, albedo=None, normal=None):
+        """RaylibB200_DenoiseDevice on H x W x 4 float32 CUDA tensors (torch) of the current device, on torch's current
+        stream: H x W x 3 float32 (numpy)."""
+        import torch
+        out = torch.empty_like(color)
+        ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+        if not self.lib.RaylibB200_DenoiseDevice(ptr(color), ptr(albedo), ptr(normal), color.shape[1], color.shape[0], ptr(out),
+                                                 C.c_void_p(torch.cuda.current_stream().cuda_stream)):
+            raise RuntimeError("RaylibB200_DenoiseDevice failed: " + self.last_error())
+        return out[:, :, :3].cpu().numpy()
+
+    def accumulator_denoise(self, acc, width, height, albedo=None, normal=None):
+        """RaylibB200_AccumulatorDenoise with H x W x 3 or 4 float32 guide arrays: H x W x 3 float32."""
+        return self._denoise_host(lambda a, n, out: self.lib.RaylibB200_AccumulatorDenoise(acc, a, n, out),
+                                  "RaylibB200_AccumulatorDenoise", height, width, (albedo, normal))
 
 
 def device_source_hash():
