@@ -7,7 +7,7 @@
 //
 // Reference interfaces they extend:
 //   RaylibB200_RenderShard / _RenderShardToFrame / _AssembleShards / _RenderToDevice  -> Raylib_Render (raylib/raylib.h:106-110)
-//   RaylibB200_TraceRays / _PrimaryHits                         -> BVHNode::Hit  (raylib/geom/bvh.cc:82-107)
+//   RaylibB200_TraceRays / _PrimaryHits / _TraceRaysStaged      -> BVHNode::Hit  (raylib/geom/bvh.cc:82-107)
 //   RaylibB200_SetFrameSeed / _SetBvhBuildKey                   -> std::random_device seeding (raylib/core/random.h:17-29, geom/bvh.cc:43)
 //   RaylibB200_RenderAccumulate / _Accumulator*                 -> Raylib_Render in installments (progressive rendering)
 #pragma once
@@ -212,6 +212,22 @@ RAYLIB_API int32_t RaylibB200_TraceRays(SceneHandle scene, const float* rays, in
 // Primary visibility through the device ray generator: one unjittered camera ray per pixel.
 RAYLIB_API int32_t RaylibB200_PrimaryHits(const RendererSettings* settings, SceneHandle scene, CameraHandle camera,
 	int32_t* outRank, float* outT);
+// The same rays through the traversal kernels a render runs (TraceRays uses a plain one-ray-per-thread kernel): one launch
+// of the closest-hit stage (mode 0: k_extend, 1: k_extend with statistics, 2: the pooled k_extend_pool) or of the
+// sun-visibility any-hit stage (mode 3: k_shadow), with `order` (a permutation of 0..numRays-1) as the queue it drains and
+// explicit scheduling: refill / walk thresholds (1..32, 0 = 20), the pooled kernel's node and refill thresholds (1..32 and
+// 1..64, 0 = 24) and the grid in CTAs (1..4096, 0 = the persistent grid of a render).
+//   Closest hit: outQueue[i] = the queue ray i was pushed to (material type 0..5 of the hit primitive, 6 = miss; -1 none,
+//   -2 more than one), outHit[4i..4i+3] = its hit record {t, bu, bv, primitive reference bits} (bu/bv: triangle
+//   barycentrics, bu = face 0..5 of a cube; a miss leaves all-ones bits), outQueueCounts[0..6] (nullable) = the counters.
+//   Any hit: every ray is a sun-visibility ray from its origin at its shutter time along -sunDirection (the scene's sun
+//   convention; the rays' own directions are not read): outQueue[i] = 0 visible, 1 occluded, -1 neither; outHit[4i..] =
+//   the path's radiance with a sun of illuminance (1, 1, 1) and no sky.  sunDirection must be finite and non-zero.
+// rays: 8 floats each (o.xyz, time, d.xyz, unused).  Arguments are checked before a device is used; GetLastStats reports the
+// call (mode 1 fills the work counters, as TraceRays does with RaylibB200_SetCollectStats).  Returns 1 on success.
+RAYLIB_API int32_t RaylibB200_TraceRaysStaged(SceneHandle scene, int32_t mode, const float* rays, const uint32_t* order,
+	int64_t numRays, float tMin, const float* sunDirection, uint32_t refillThreshold, uint32_t walkThreshold,
+	uint32_t poolNodeThreshold, uint32_t poolRefill, uint32_t gridCtas, int32_t* outQueue, float* outHit, uint32_t* outQueueCounts);
 
 // The device's own sinf / cosf / tanf / asinf / acosf / atanf / expf / logf / powf / atan2f (fn 0..9; include/rt_libm.h:
 // glibc's algorithms restated so that the GPU consumes the same bits as the reference's host build) evaluated on `count`

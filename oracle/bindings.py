@@ -153,6 +153,25 @@ class Restatement:
         self.lib.rt_oracle_trace(desc, rays, len(rays), t_min, rank, t, C.byref(counts))
         return rank, t, list(counts)
 
+    def trace_hits(self, desc, rays, t_min):
+        """trace() plus what a device hit record and queue hold: -> (rank, t, uv n x 2 (paramU / paramV of triangle hits,
+        else 0), face (0..5 of cube hits in the device's order, else -1), material type of the hit primitive (-1: miss),
+        counts)."""
+        rays = np.ascontiguousarray(rays, dtype=np.float32).reshape(-1, 8)
+        n = len(rays)
+        rank = np.empty(n, dtype=np.int32)
+        t = np.empty(n, dtype=np.float32)
+        uv = np.empty((n, 2), dtype=np.float32)
+        face = np.empty(n, dtype=np.int32)
+        mat = np.empty(n, dtype=np.int32)
+        counts = (C.c_uint64 * 4)()
+        fn = self.lib.rt_oracle_trace_hits
+        fn.restype = None
+        fn.argtypes = [C.POINTER(RtSceneDesc), _F32P, C.c_int64, C.c_float, _I32P, _F32P, _F32P, _I32P, _I32P,
+                       C.POINTER(C.c_uint64 * 4)]
+        fn(desc, rays, n, t_min, rank, t, uv, face, mat, C.byref(counts))
+        return rank, t, uv, face, mat, list(counts)
+
     def primary(self, desc, cam, width, height, t_min, seed=1337, rows=None, want_rays=False):
         """want_rays: also return the n x 8 camera rays (bit-identical to the compiled reference's, tests/golden)."""
         n = width * height

@@ -36,7 +36,9 @@ static V3 normalize(V3 a) { float k = 1.0f / sqrtf(a.x * a.x + a.y * a.y + a.z *
 static int g_useTraversalTree = 0;
 
 typedef struct { V3 o, d; float time; } Ray;
-typedef struct { int hit; float t; uint32_t rank; } Hit;
+/* u, v: paramU / paramV of a triangle hit (triangle.cc:42-43); face: 0..5 of a cube hit, in the device's order (t1..t6 of
+ * cube.cc, csrc/device/rt_traverse.cuh cube_test); mat: RtMaterialType of the hit primitive's material */
+typedef struct { int hit; float t; uint32_t rank; float u, v; int32_t face, mat; } Hit;
 typedef struct { uint64_t box, tri, sphere, cube; } Counts;
 
 /* aabb.h:41-53 */
@@ -80,7 +82,7 @@ static int gate_ok(const RtSceneDesc* S, uint32_t gate, const Ray* r, float t_mi
 	return box_hit(g, g + 4, r, t_min, FLT_MAX);
 }
 
-static int triangle_hit(const RtSceneDesc* S, uint32_t idx, const Ray* r, float t_min, float t_max, float* outT)
+static int triangle_hit(const RtSceneDesc* S, uint32_t idx, const Ray* r, float t_min, float t_max, float* outT, float* outU, float* outV)
 {
 	const float* q = S->triHot[idx].q;
 	const V3 v0 = v3p(q), n = v3p(q + 3), u = v3p(q + 6), v = v3p(q + 9);
@@ -107,7 +109,7 @@ static int triangle_hit(const RtSceneDesc* S, uint32_t idx, const Ray* r, float 
 		}
 		/* device traversal tree only: the triangle's reference gate box (see rt_scene_format.h) must pass */
 		if (!gate_ok(S, S->triGate[idx], r, t_min)) return 0;
-		*outT = t;
+		*outT = t; *outU = paramU; *outV = paramV;
 		return 1;
 	}
 	return 0;
@@ -136,7 +138,7 @@ static float fmax_std(float a, float b) { return (a < b) ? b : a; }   /* std::ma
 static float fmin_std(float a, float b) { return (b < a) ? b : a; }   /* std::min */
 
 /* cube.cc:3-43 */
-static int cube_hit(const RtSceneDesc* S, uint32_t idx, const Ray* r, float t_min, float t_max, float* outT)
+static int cube_hit(const RtSceneDesc* S, uint32_t idx, const Ray* r, float t_min, float t_max, float* outT, int32_t* outFace)
 {
 	const RtCube* cb = &S->cubes[idx];
 	V3 move = muls(v3p(cb->velocity), fmax_std(0.0f, r->time - cb->timeStartMove));
@@ -148,19 +150,38 @@ static int cube_hit(const RtSceneDesc* S, uint32_t idx, const Ray* r, float t_mi
 	t[7] = fmax_std(fmax_std(fmin_std(t[1], t[2]), fmin_std(t[3], t[4])), fmin_std(t[5], t[6]));
 	t[8] = fmin_std(fmin_std(fmax_std(t[1], t[2]), fmax_std(t[3], t[4])), fmax_std(t[5], t[6]));
 	if (t[8] < 0 || t[7] > t[8]) return 0;
-	if (t_min <= t[7] && t[7] <= t_max) { *outT = t[7]; return gate_ok(S, S->cubeGate[idx], r, t_min); }
+	if (t_min <= t[7] && t[7] <= t_max)
+	{
+		*outT = t[7];
+		*outFace = 6;
+		for (int k = 6; k >= 1; --k) if (t[7] == t[k]) *outFace = k - 1;       /* the first of t1..t6 equal to the entry */
+		return gate_ok(S, S->cubeGate[idx], r, t_min);
+	}
 	return 0;
 }
 
-static Hit miss(void) { Hit h = { 0, 0.0f, 0 }; return h; }
+static Hit miss(void) { Hit h = { 0, 0.0f, 0, 0.0f, 0.0f, -1, -1 }; return h; }
 
 static Hit prim_hit(const RtSceneDesc* S, uint32_t kind, uint32_t idx, const Ray* r, float tMin, float tMax, Counts* c)
 {
 	Hit h = miss();
-	float t;
-	if (kind == RT_REF_TRI) { c->tri++; if (triangle_hit(S, idx, r, tMin, tMax, &t)) { h.hit = 1; h.t = t; h.rank = S->triRank[idx]; } }
-	else if (kind == RT_REF_SPHERE) { c->sphere++; if (sphere_hit(S, idx, r, tMin, tMax, &t)) { h.hit = 1; h.t = t; h.rank = S->sphereRank[idx]; } }
-	else { c->cube++; if (cube_hit(S, idx, r, tMin, tMax, &t)) { h.hit = 1; h.t = t; h.rank = S->cubeRank[idx]; } }
+	float t, u = 0.0f, v = 0.0f;
+	int32_t face = -1;
+	if (kind == RT_REF_TRI)
+	{
+		c->tri++;
+		if (triangle_hit(S, idx, r, tMin, tMax, &t, &u, &v)) { h.hit = 1; h.t = t; h.rank = S->triRank[idx]; h.u = u; h.v = v; h.mat = (int32_t)S->materials[S->triCold[idx].material].type; }
+	}
+	else if (kind == RT_REF_SPHERE)
+	{
+		c->sphere++;
+		if (sphere_hit(S, idx, r, tMin, tMax, &t)) { h.hit = 1; h.t = t; h.rank = S->sphereRank[idx]; h.mat = (int32_t)S->materials[S->sphereMaterial[idx]].type; }
+	}
+	else
+	{
+		c->cube++;
+		if (cube_hit(S, idx, r, tMin, tMax, &t, &face)) { h.hit = 1; h.t = t; h.rank = S->cubeRank[idx]; h.face = face; h.mat = (int32_t)S->materials[S->cubes[idx].material].type; }
+	}
 	return h;
 }
 
@@ -355,6 +376,27 @@ void rt_oracle_trace(const RtSceneDesc* S, const float* rays, int64_t numRays, f
 		Hit h = closest(S, &r, tMin, &c);
 		outRank[i] = h.hit ? (int32_t)h.rank : -1;
 		outT[i] = h.hit ? h.t : 0.0f;
+	}
+	if (counts4) { counts4[0] = c.box; counts4[1] = c.tri; counts4[2] = c.sphere; counts4[3] = c.cube; }
+}
+
+/* rt_oracle_trace plus what the hit record of a device path holds and where the path goes next (nullable outputs, n each):
+ * outUV (2 floats per ray) = paramU, paramV of a triangle hit, else 0; outFace = 0..5 of a cube hit (device order), else -1;
+ * outMat = RtMaterialType of the hit primitive's material, -1 on a miss. */
+void rt_oracle_trace_hits(const RtSceneDesc* S, const float* rays, int64_t numRays, float tMin,
+                          int32_t* outRank, float* outT, float* outUV, int32_t* outFace, int32_t* outMat, uint64_t* counts4)
+{
+	Counts c = { 0, 0, 0, 0 };
+	for (int64_t i = 0; i < numRays; ++i)
+	{
+		const float* q = rays + 8 * i;
+		Ray r; r.o = v3(q[0], q[1], q[2]); r.time = q[3]; r.d = v3(q[4], q[5], q[6]);
+		Hit h = closest(S, &r, tMin, &c);
+		outRank[i] = h.hit ? (int32_t)h.rank : -1;
+		outT[i] = h.hit ? h.t : 0.0f;
+		if (outUV) { outUV[2 * i] = h.hit ? h.u : 0.0f; outUV[2 * i + 1] = h.hit ? h.v : 0.0f; }
+		if (outFace) outFace[i] = h.hit ? h.face : -1;
+		if (outMat) outMat[i] = h.hit ? h.mat : -1;
 	}
 	if (counts4) { counts4[0] = c.box; counts4[1] = c.tri; counts4[2] = c.sphere; counts4[3] = c.cube; }
 }

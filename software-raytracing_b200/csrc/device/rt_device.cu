@@ -19,6 +19,7 @@
 // Compile: nvcc -gencode arch=compute_100a,code=sm_100a --fmad=false -lineinfo (see Makefile).
 #include "rt_device_abi.h"
 #include "rt_progressive.h"
+#include "rt_trace_stage.h"
 #include "rt_checksum.h"
 #include "rt_shade.cuh"
 
@@ -2038,6 +2039,168 @@ extern "C" int rt_trace_closest(RtRenderContext* ctx, const RtDeviceScene* sc, c
 		stats->kernelLaunches = 1;
 	}
 	return 0;
+}
+
+// ---- the traversal stage kernels of a render on caller rays (parity tests, rt_trace_stage.h) --------------------------
+// One of k_extend / k_extend_pool / k_shadow at bounce 0 on an arena prepared by hand: the caller's rays in the path
+// records, the caller's order as the queue.
+extern "C" int rt_trace_stage(RtRenderContext* ctx, const RtDeviceScene* sc, int mode, const float* hostRays, const uint32_t* hostOrder,
+                              int64_t numRays, float tMin, const float* sunDirection, const RtStageSchedule* schedule,
+                              int32_t* hostOutQueue, float* hostOutHit, uint32_t* hostOutQueueCounts, RtRenderStats* stats)
+{
+	if (!ctx || !sc || !hostRays || !hostOrder || !schedule || !hostOutQueue || !hostOutHit) { g_lastError = "rt_trace_stage: null argument"; return -1; }
+	if (mode < RT_STAGE_EXTEND || mode > RT_STAGE_SHADOW) { g_lastError = "rt_trace_stage: unknown mode"; return -1; }
+	if (mode == RT_STAGE_SHADOW && !sunDirection) { g_lastError = "rt_trace_stage: the any-hit mode needs a sun direction"; return -1; }
+	if (numRays <= 0 || numRays >= ((int64_t)1 << 31)) { g_lastError = "rt_trace_stage: the ray count must be in [1, 2^31)"; return -1; }
+	if (sc->device != ctx->device) { g_lastError = "rt_trace_stage: scene and context live on different devices"; return -1; }
+	const uint32_t n = (uint32_t)numRays;
+	{
+		// the kernels index the path records with the queue's entries: anything but a permutation would address outside them
+		std::vector<uint8_t> seen(n, 0);
+		for (uint32_t i = 0; i < n; ++i)
+		{
+			if (hostOrder[i] >= n || seen[hostOrder[i]]) { g_lastError = "rt_trace_stage: the order is not a permutation of the rays"; return -1; }
+			seen[hostOrder[i]] = 1;
+		}
+	}
+#if !RT_PACKED_STATE
+	g_lastError = "rt_trace_stage: needs the packed path-state layout (RT_PACKED_STATE 1)";
+	return -1;
+#else
+	RT_CUDA(cudaSetDevice(ctx->device));
+	const uint32_t levels = stack_levels(sc);
+	if (!stack_fits(levels)) { g_lastError = "rt_trace_stage: BVH too deep for the traversal stack"; return -1; }
+	RtPipe& pipe = ctx->pipe[0];
+	int rc;
+	if ((rc = ensure_arena(pipe, n, 1))) return rc;
+
+	// one bounce of a 1 x 1 frame: no pixels are touched, only the scene, tMin and the scheduling thresholds matter
+	RtRenderParams p;
+	memset(&p, 0, sizeof(p));
+	p.width = 1; p.height = 1; p.samplesPerPixel = 1; p.maxPathLength = 1; p.rayTMin = tMin; p.shardCount = 1;
+	p.tuning.refillThreshold = schedule->refillThreshold;
+	p.tuning.walkThreshold = schedule->walkThreshold;
+	p.tuning.binOriginBits = 0; p.tuning.binDirBits = 0;      // no ray binning (bounce 0 reads extQ[0] either way)
+	RtCamera cam;
+	memset(&cam, 0, sizeof(cam));
+	RtLaunch L = pipe.L;         // the arena's pointers
+	fill_scene(L, sc, &cam, &p, levels);
+	L.capacity = pipe.capacity;
+	L.K = 1;
+	L.ctl = pipe.ctl;
+	L.accum = nullptr; L.out = nullptr; L.image = nullptr; L.out2 = nullptr; L.runningSum = 0u;
+	if (mode == RT_STAGE_SHADOW)
+	{
+		// a sun of illuminance 1 and no sky term: a path's radiance is (1, 1, 1) if its sun ray is unoccluded, 0 otherwise
+		for (int i = 0; i < 3; ++i) { L.S.sunDirection[i] = sunDirection[i]; L.S.sunIlluminance[i] = 1.0f; }
+		L.S.hasSun = 1u;
+	}
+
+	int grid = 0;
+	const size_t smem = 0;
+	if (mode == RT_STAGE_EXTEND) rc = persistent_grid(ctx, k_extend<false>, 128, smem, &grid);
+	else if (mode == RT_STAGE_EXTEND_STATS) rc = persistent_grid(ctx, k_extend<true>, 128, smem, &grid);
+	else if (mode == RT_STAGE_EXTEND_POOL) rc = persistent_grid(ctx, k_extend_pool, 128, 0, &grid);
+	else rc = persistent_grid(ctx, k_shadow, 128, smem, &grid);
+	if (rc) return rc;
+	if (schedule->gridCtas) grid = (int)schedule->gridCtas;
+	if (mode == RT_STAGE_EXTEND_POOL)
+	{
+		const size_t entries = (size_t)grid * 4u * RT_MAX_STACK * RT_POOL_RAYS;
+		if (pipe.poolStackEntries < entries)
+		{
+			if (pipe.poolStack) cudaFree(pipe.poolStack);
+			pipe.poolStack = nullptr; pipe.poolStackEntries = 0;
+			RT_CUDA(cudaMalloc((void**)&pipe.poolStack, entries * sizeof(uint2)));
+			pipe.poolStackEntries = entries;
+		}
+		pipe.L.poolStack = pipe.poolStack;
+		L.poolStack = pipe.poolStack;
+		L.poolNodeThreshold = schedule->poolNodeThreshold ? schedule->poolNodeThreshold : 24u;
+		L.poolRefill = schedule->poolRefill ? schedule->poolRefill : 24u;
+	}
+
+	// the rays into the path records ({o.xyz, time | d.xyz, -}, the caller's layout), the order into the queue the kernel
+	// drains, its counter set and every other counter of the bounce block zeroed; hit records, radiance and the output
+	// queues start as all-ones sentinels, so that a slot the kernel never wrote is seen as such
+	uint32_t* const queueIn = mode == RT_STAGE_SHADOW ? L.shadowQ : L.extQ[0];
+	RT_CUDA(cudaMemcpy(L.ray, hostRays, (size_t)n * sizeof(RtF8), cudaMemcpyHostToDevice));
+	RT_CUDA(cudaMemcpy(queueIn, hostOrder, (size_t)n * 4, cudaMemcpyHostToDevice));
+	RT_CUDA(cudaMemset(L.bounceCtl, 0, ((size_t)pipe.depthCapacity + 2) * sizeof(RtBounceCtl)));
+	RtBounceCtl bc;
+	memset(&bc, 0, sizeof(bc));
+	if (mode == RT_STAGE_SHADOW) bc.shadowCount = n; else bc.extCount = n;
+	RT_CUDA(cudaMemcpy(L.bounceCtl, &bc, sizeof(bc), cudaMemcpyHostToDevice));
+	RT_CUDA(cudaMemset(L.hitCtl, 0xFF, (size_t)n * sizeof(RtF8)));
+	RT_CUDA(cudaMemset(L.Li, 0xFF, (size_t)n * sizeof(float4)));
+	RT_CUDA(cudaMemset(L.missPartial, 0, (size_t)n * sizeof(float4)));
+	for (int k = 0; k < RT_NUM_HIT_QUEUES; ++k) RT_CUDA(cudaMemset(L.matQ[k], 0xFF, (size_t)n * 4));
+	RT_CUDA(cudaMemset(pipe.ctl, 0, sizeof(RtQueueCtl)));
+
+	RT_CUDA(cudaEventRecord(ctx->evStart, 0));
+	if (mode == RT_STAGE_EXTEND) k_extend<false><<<grid, 128, smem>>>(L, 0);
+	else if (mode == RT_STAGE_EXTEND_STATS) k_extend<true><<<grid, 128, smem>>>(L, 0);
+	else if (mode == RT_STAGE_EXTEND_POOL) k_extend_pool<<<grid, 128, 0>>>(L, 0);
+	else k_shadow<<<grid, 128, smem>>>(L, 0);
+	RT_CUDA(cudaEventRecord(ctx->evStop, 0));
+	RT_CUDA(cudaGetLastError());
+	RT_CUDA(cudaDeviceSynchronize());
+
+	if (hostOutQueueCounts) memset(hostOutQueueCounts, 0, RT_NUM_HIT_QUEUES * sizeof(uint32_t));
+	if (mode == RT_STAGE_SHADOW)
+	{
+		std::vector<float4> li(n);
+		RT_CUDA(cudaMemcpy(li.data(), L.Li, (size_t)n * sizeof(float4), cudaMemcpyDeviceToHost));
+		for (uint32_t i = 0; i < n; ++i)
+		{
+			const float4 v = li[i];
+			memcpy(hostOutHit + 4 * (size_t)i, &v, sizeof(v));
+			const bool visible = v.x == 1.0f && v.y == 1.0f && v.z == 1.0f && v.w == 0.0f;
+			const bool occluded = v.x == 0.0f && v.y == 0.0f && v.z == 0.0f && v.w == 0.0f;
+			hostOutQueue[i] = visible ? 0 : occluded ? 1 : -1;
+		}
+	}
+	else
+	{
+		RtBounceCtl done;
+		RT_CUDA(cudaMemcpy(&done, L.bounceCtl, sizeof(done), cudaMemcpyDeviceToHost));
+		std::vector<RtF8> rec(n);
+		RT_CUDA(cudaMemcpy(rec.data(), L.hitCtl, (size_t)n * sizeof(RtF8), cudaMemcpyDeviceToHost));
+		for (uint32_t i = 0; i < n; ++i)
+		{
+			memcpy(hostOutHit + 4 * (size_t)i, &rec[i].lo, sizeof(float4));
+			hostOutQueue[i] = -1;
+		}
+		std::vector<uint32_t> q;
+		for (int k = 0; k < RT_NUM_HIT_QUEUES; ++k)
+		{
+			if (hostOutQueueCounts) hostOutQueueCounts[k] = done.matCount[k];
+			q.resize(std::min(done.matCount[k], n));        // a counter above n fails the caller's sum check on its own
+			if (!q.empty()) RT_CUDA(cudaMemcpy(q.data(), L.matQ[k], q.size() * 4, cudaMemcpyDeviceToHost));
+			for (uint32_t s : q)
+				if (s < n) hostOutQueue[s] = hostOutQueue[s] == -1 ? k : -2;
+		}
+	}
+	if (stats)
+	{
+		RtQueueCtl h;
+		RT_CUDA(cudaMemcpy(&h, pipe.ctl, sizeof(h), cudaMemcpyDeviceToHost));
+		float ms = 0.0f;
+		RT_CUDA(cudaEventElapsedTime(&ms, ctx->evStart, ctx->evStop));
+		memset(stats, 0, sizeof(*stats));
+		stats->rayQueries = n;
+		stats->boxTests = h.boxTests; stats->triTests = h.triTests; stats->sphereTests = h.sphereTests; stats->nodeVisits = h.nodeVisits;
+		stats->gateTests = h.gateTests; stats->cubeTests = h.cubeTests;
+		stats->refBoxTests = h.refBoxTests; stats->refTriTests = h.refTriTests; stats->refSphereTests = h.refSphereTests;
+		stats->statRays = h.statRays;
+		stats->nodeIters = h.nodeIters; stats->nodeStep = h.nodeStep; stats->nodeAlive = h.nodeAlive;
+		stats->leafIters = h.leafIters; stats->leafBusy = h.leafBusy;
+		stats->deviceMs = ms;
+		stats->kernelLaunches = 1;
+		stats->extendLaunches = mode == RT_STAGE_SHADOW ? 0u : 1u;
+	}
+	return 0;
+#endif
 }
 
 // ---- Image2D::PostProcess on the device (render/image.cc:44-103) -----------------------------------------

@@ -17,6 +17,7 @@
 
 #include <algorithm>
 #include <chrono>
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 #include <map>
@@ -872,6 +873,65 @@ namespace RtGpu
 		memset(&st, 0, sizeof(st));
 		if (!RunDenoise(fn, CurrentDevice(), color, 0, albedo, normal, width, height, out, stream, st)) return false;
 		st.totalMs = MsSince(wall0);
+		SetLastStats(st);
+		return true;
+	}
+}
+
+// ---------------------------------------------------------------------------------------------
+// The traversal stage kernels on caller rays (RaylibB200_TraceRaysStaged, rt_trace_stage of rt_trace_stage.h)
+
+namespace RtGpu
+{
+	bool TraceRaysStaged(const Scene* scene, int mode, const float* rays, const uint32_t* order, int64_t numRays, float tMin,
+	                     const float* sunDirection, const RtStageSchedule& schedule, int32_t* outQueue, float* outHit,
+	                     uint32_t* outQueueCounts)
+	{
+		const auto wall0 = std::chrono::steady_clock::now();
+		t_lastError.clear();
+		const std::string fn = "RaylibB200_TraceRaysStaged: ";
+		if (!scene) { SetLastError(fn + "null scene"); return false; }
+		if (!rays || !order || !outQueue || !outHit) { SetLastError(fn + "null ray, order or output buffer"); return false; }
+		if (mode < RT_STAGE_EXTEND || mode > RT_STAGE_SHADOW) { SetLastError(fn + "unknown mode " + std::to_string(mode) + " (0..3)"); return false; }
+		if (numRays <= 0 || numRays >= ((int64_t)1 << 31)) { SetLastError(fn + "the ray count must be in [1, 2^31)"); return false; }
+		if (mode == RT_STAGE_SHADOW)
+		{
+			if (!sunDirection) { SetLastError(fn + "the any-hit mode needs a sun direction"); return false; }
+			bool finite = true, zero = true;
+			for (int i = 0; i < 3; ++i) { finite = finite && std::isfinite(sunDirection[i]); zero = zero && sunDirection[i] == 0.0f; }
+			if (!finite || zero) { SetLastError(fn + "the sun direction must be finite and non-zero"); return false; }
+		}
+		if (schedule.refillThreshold > 32u || schedule.walkThreshold > 32u || schedule.poolNodeThreshold > 32u ||
+		    schedule.poolRefill > 64u || schedule.gridCtas > 4096u)
+		{
+			SetLastError(fn + "scheduling out of range (refill, walk, pool node: 0..32; pool refill: 0..64; grid: 0..4096 CTAs)");
+			return false;
+		}
+		{
+			std::vector<uint8_t> seen((size_t)numRays, 0);
+			for (int64_t i = 0; i < numRays; ++i)
+			{
+				if ((int64_t)order[i] >= numRays || seen[order[i]]) { SetLastError(fn + "the order is not a permutation of 0..numRays-1"); return false; }
+				seen[order[i]] = 1;
+			}
+		}
+		const RtDeviceScene* ds = AcquireScene(scene);
+		RtRenderContext* ctx = ds ? AcquireContext() : nullptr;
+		if (!ds || !ctx) return false;
+		RtRenderStats rs;
+		if (rt_trace_stage(ctx, ds, mode, rays, order, numRays, tMin, sunDirection, &schedule, outQueue, outHit, outQueueCounts, &rs) != 0)
+		{
+			SetLastError(fn + rt_last_error());
+			return false;
+		}
+		RaylibB200Stats st;
+		memset(&st, 0, sizeof(st));
+		AddStats(st, rs);
+		st.totalMs = MsSince(wall0);
+		st.device = (uint32_t)CurrentDevice();
+		st.devicesUsed = 1;
+		st.h2dBytes = (uint64_t)numRays * 36u;                                   // rays + order
+		st.d2hBytes = (uint64_t)numRays * (mode == RT_STAGE_SHADOW ? 16u : 36u);   // records or radiance (+ queues)
 		SetLastStats(st);
 		return true;
 	}

@@ -2,6 +2,7 @@
 // (path-state arenas) and the uploaded copy of every finalized scene.
 #pragma once
 #include "rt_device_abi.h"
+#include "rt_trace_stage.h"
 #include "raylib_b200.h"
 #include <memory>
 #include <string>
@@ -85,4 +86,10 @@ namespace RtGpu
 	// W x H RGBA float4 images on the current device.  Guides are nullable.  Arguments are checked before a device is used.
 	bool Denoise(const Image2D* color, const Image2D* albedo, const Image2D* normal, Image2D* out);
 	bool DenoiseDevice(const void* color, const void* albedo, const void* normal, uint32_t width, uint32_t height, void* out, void* stream);
+
+	// One launch of a traversal stage kernel (k_extend, k_extend_pool, k_shadow) on caller rays in a caller order
+	// (rt_trace_stage of rt_trace_stage.h).  Arguments are checked before a device is used.
+	bool TraceRaysStaged(const Scene* scene, int mode, const float* rays, const uint32_t* order, int64_t numRays, float tMin,
+	                     const float* sunDirection, const RtStageSchedule& schedule, int32_t* outQueue, float* outHit,
+	                     uint32_t* outQueueCounts);
 }

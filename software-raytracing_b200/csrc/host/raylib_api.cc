@@ -638,6 +638,15 @@ int32_t RaylibB200_TraceRays(SceneHandle scene, const float* rays, int64_t numRa
 	return 1;
 }
 
+int32_t RaylibB200_TraceRaysStaged(SceneHandle scene, int32_t mode, const float* rays, const uint32_t* order, int64_t numRays,
+	float tMin, const float* sunDirection, uint32_t refillThreshold, uint32_t walkThreshold, uint32_t poolNodeThreshold,
+	uint32_t poolRefill, uint32_t gridCtas, int32_t* outQueue, float* outHit, uint32_t* outQueueCounts)
+{
+	const RtStageSchedule schedule = { refillThreshold, walkThreshold, poolNodeThreshold, poolRefill, gridCtas };
+	return RtGpu::TraceRaysStaged((const Scene*)scene, mode, rays, order, numRays, tMin, sunDirection, schedule, outQueue, outHit,
+		outQueueCounts) ? 1 : 0;
+}
+
 int32_t RaylibB200_PrimaryHits(const RendererSettings* settings, SceneHandle scene, CameraHandle camera, int32_t* outRank, float* outT)
 {
 	if (!settings || !outRank || !outT) { RtGpu::SetLastError("RaylibB200_PrimaryHits: null argument"); return 0; }

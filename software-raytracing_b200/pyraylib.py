@@ -167,6 +167,9 @@ B200_C_API = {
     "RaylibB200_ImageGetRGBA": (C.c_int32, [H, _F32P]),
     "RaylibB200_TraceRays": (C.c_int32, [H, _F32P, C.c_int64, C.c_float, _I32P, _F32P]),
     "RaylibB200_PrimaryHits": (C.c_int32, [C.POINTER(RendererSettings), H, H, _I32P, _F32P]),
+    "RaylibB200_TraceRaysStaged": (C.c_int32, [H, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64, C.c_float, C.c_void_p,
+                                               C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32,
+                                               C.c_void_p, C.c_void_p, C.c_void_p]),
     "RaylibB200_SaveFlattenedScene": (C.c_int32, [H, C.c_char_p]),
     "RaylibB200_LoadFlattenedScene": (H, [C.c_char_p]),
     "RaylibB200_FlattenForInspection": (C.POINTER(RtSceneDesc), [H]),
@@ -291,6 +294,33 @@ class Product(_Base):
         if not self.lib.RaylibB200_TraceRays(scene, rays, len(rays), t_min, rank, t):
             raise RuntimeError("RaylibB200_TraceRays failed: " + self.last_error())
         return rank, t
+
+    # RaylibB200_TraceRaysStaged modes: the traversal stage kernels of a render
+    STAGE_MODES = {"extend": 0, "extend_stats": 1, "extend_pool": 2, "shadow": 3}
+    STAGE_QUEUE_MISS = 6
+
+    def trace_rays_staged(self, scene, rays, t_min, mode="extend", order=None, sun_direction=None, refill=0, walk=0,
+                          pool_node=0, pool_refill=0, grid_ctas=0):
+        """RaylibB200_TraceRaysStaged: one launch of k_extend / k_extend_pool ("extend", "extend_stats", "extend_pool") or
+        k_shadow ("shadow") on n x 8 float32 rays, drained in `order` (default: identity).  Returns (queue int32[n],
+        record float32[n, 4], queue counts uint32[7]): for the closest-hit modes the queue each ray was pushed to (material
+        type 0..5, 6 = miss, -1 none, -2 several) and its hit record {t, bu, bv, ref bits}; for "shadow" 0 (sun visible) /
+        1 (occluded) / -1 and the path's radiance.  Scheduling values of 0 are the render's defaults."""
+        self.require_gpu()
+        rays = np.ascontiguousarray(rays, dtype=np.float32).reshape(-1, 8)
+        n = len(rays)
+        order = np.arange(n, dtype=np.uint32) if order is None else np.ascontiguousarray(order, dtype=np.uint32)
+        sun = None if sun_direction is None else np.ascontiguousarray(sun_direction, dtype=np.float32)
+        queue = np.empty(n, dtype=np.int32)
+        record = np.empty((n, 4), dtype=np.float32)
+        counts = np.zeros(7, dtype=np.uint32)
+        ok = self.lib.RaylibB200_TraceRaysStaged(scene, self.STAGE_MODES[mode], rays.ctypes.data, order.ctypes.data, n, t_min,
+                                                 None if sun is None else sun.ctypes.data, refill, walk, pool_node,
+                                                 pool_refill, grid_ctas, queue.ctypes.data, record.ctypes.data,
+                                                 counts.ctypes.data)
+        if not ok:
+            raise RuntimeError("RaylibB200_TraceRaysStaged failed: " + self.last_error())
+        return queue, record, counts
 
     def flat_desc(self, scene):
         p = self.lib.RaylibB200_FlattenForInspection(scene)
