@@ -32,10 +32,6 @@
 #include <map>
 #include <algorithm>
 
-#ifndef RT_PACKED_STATE
-#define RT_PACKED_STATE 1      // path state as 32-byte records (one sector per access); 0 = separate float4 arrays
-#endif
-
 // ------------------------------------------------------------------------------------------------
 // error plumbing
 
@@ -55,12 +51,7 @@ extern "C" const char* rt_last_error(void) { return g_lastError.c_str(); }
 	} while (0)
 
 // The traversal stack of a thread: RT_MAX_STACK {ref, entry t} entries in thread-local memory (rt_traverse.cuh).
-#if RT_STACK_SMEM_LEVELS > 0
-#define RT_DECLARE_STACK(name) uint2 localStack_[RT_MAX_STACK]; __shared__ uint2 sharedStack_[RT_STACK_SMEM_LEVELS * 128]; \
-	RtStack name; name.base = localStack_; name.stride = 1; name.sm = sharedStack_ + threadIdx.x
-#else
 #define RT_DECLARE_STACK(name) uint2 localStack_[RT_MAX_STACK]; RtStack name; name.base = localStack_; name.stride = 1
-#endif
 
 // ------------------------------------------------------------------------------------------------
 // device-side control block and launch descriptor
@@ -98,19 +89,11 @@ struct RtLaunch
 	RtCamera cam;
 	// path-state arena (SoA, indexed by path slot)
 	// Path state is read and written through queue indices, i.e. as per-slot gathers: every record a stage kernel touches
-	// is ONE 32-byte sector moved by one 256-bit load / store (RT_PACKED_STATE 0 keeps the round-1 layout of separate
-	// float4 arrays, where each access used half a sector: the stage kernels ran at ~50 % sector efficiency).
-#if RT_PACKED_STATE
+	// is ONE 32-byte sector moved by one 256-bit load / store (separate float4 arrays used half a sector per access: the
+	// frame ran 5.7-6 % slower, profiles/r02a_packed_state_variants.jsonl).
 	RtF8*   ray;           // {o.xyz, time | d.xyz, -}
 	RtF8*   hitCtl;        // {t, bu, bv, ref bits | rngCtr, slotKey (bin of the ray a shade kernel wrote into this slot), -, -}
 	RtF8*   stack;         // [bounce][slot] {reflectance.xyz, scatPdf | emitted.xyz, pdf}
-#else
-	float4* rayO;          // o.xyz, time
-	float4* rayD;          // d.xyz, -
-	float4* hit;           // t, bu, bv, ref bits
-	float4* stackA;        // [bounce][slot] reflectance.xyz, scatPdf
-	float4* stackB;        // [bounce][slot] emitted.xyz, pdf
-#endif
 	float4* Li;            // per path result
 	float4* missPartial;   // sky term while the sun ray is in flight
 	float4* accum;         // [shard pixel] running sample sum
@@ -118,16 +101,10 @@ struct RtLaunch
 	float4* image;         // optional: row-major W x H frame the final pixels go to DIRECTLY (may be another GPU's memory,
 	                       // mapped over NVLink): fuses the tile gather into the last accumulate; `out` is then unused
 	float4* out2;          // [shard pixel] second output of the fused denoiser-input pass (RT_RENDERMODE_AUX)
-#if !RT_PACKED_STATE
-	uint32_t* rngCtr;
-#endif
 	uint32_t* extQ[2];
 	uint32_t* matQ[RT_NUM_HIT_QUEUES];   // extend's output queues: material-sorted hits + misses
 	uint32_t* shadowQ;
 	// ray binning (counting sort of the next bounce's rays by origin cell + direction octant, see k_bin_*)
-#if !RT_PACKED_STATE
-	uint32_t* slotKey;     // [slot] bin of the ray a shade kernel wrote into this slot
-#endif
 	uint32_t* extKey;      // [queue position] bin of the ray at that position of the coming bounce's extend queue: written next
 	                       // to the queue entry (coalesced), so that the scatter pass streams instead of gathering per slot
 	uint32_t* extSorted;   // the extend queue of the coming bounce in bin order
@@ -160,7 +137,7 @@ struct RtLaunch
 	                           //   the first pass continues them, the last pass stores them back (progressive rendering)
 };
 
-// ---- path-state accessors (one definition per layout) ------------------------------------------------------------
+// ---- path-state accessors ------------------------------------------------------------------------------------------
 RT_DEV RtF8 ld8_state(const RtF8* p)
 {
 	RtF8 r;
@@ -173,7 +150,6 @@ RT_DEV void st8_state(RtF8* p, float4 lo, float4 hi)
 	asm volatile("st.global.v8.f32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
 		:: "l"(p), "f"(lo.x), "f"(lo.y), "f"(lo.z), "f"(lo.w), "f"(hi.x), "f"(hi.y), "f"(hi.z), "f"(hi.w) : "memory");
 }
-#if RT_PACKED_STATE
 RT_DEV void load_ray(const RtLaunch& L, uint32_t slot, float4& o, float4& d) { const RtF8 v = ld8_state(L.ray + slot); o = v.lo; d = v.hi; }
 RT_DEV float4 load_ray_origin(const RtLaunch& L, uint32_t slot) { return reinterpret_cast<const float4*>(L.ray + slot)[0]; }
 RT_DEV float4 load_ray_dir(const RtLaunch& L, uint32_t slot) { return reinterpret_cast<const float4*>(L.ray + slot)[1]; }
@@ -196,25 +172,6 @@ RT_DEV void load_bounce(const RtLaunch& L, int bounce, uint32_t slot, float4& a,
 	a = v.lo; b = v.hi;
 }
 RT_DEV void store_bounce(const RtLaunch& L, int bounce, uint32_t slot, float4 a, float4 b) { st8_state(L.stack + (size_t)bounce * L.capacity + slot, a, b); }
-#else
-RT_DEV void load_ray(const RtLaunch& L, uint32_t slot, float4& o, float4& d) { o = L.rayO[slot]; d = L.rayD[slot]; }
-RT_DEV float4 load_ray_origin(const RtLaunch& L, uint32_t slot) { return L.rayO[slot]; }
-RT_DEV float4 load_ray_dir(const RtLaunch& L, uint32_t slot) { return L.rayD[slot]; }
-RT_DEV void store_ray(const RtLaunch& L, uint32_t slot, float4 o, float4 d) { L.rayO[slot] = o; L.rayD[slot] = d; }
-RT_DEV void store_hit(const RtLaunch& L, uint32_t slot, float4 h) { L.hit[slot] = h; }
-RT_DEV void load_hit_and_counter(const RtLaunch& L, uint32_t slot, float4& h, uint32_t& ctr) { h = L.hit[slot]; ctr = L.rngCtr[slot]; }
-RT_DEV void store_counter(const RtLaunch& L, uint32_t slot, uint32_t ctr) { L.rngCtr[slot] = ctr; }
-RT_DEV void store_counter_and_key(const RtLaunch& L, uint32_t slot, uint32_t ctr, uint32_t key) { L.rngCtr[slot] = ctr; L.slotKey[slot] = key; }
-RT_DEV uint32_t load_slot_key(const RtLaunch& L, uint32_t slot) { return L.slotKey[slot]; }
-RT_DEV void load_bounce(const RtLaunch& L, int bounce, uint32_t slot, float4& a, float4& b)
-{
-	a = L.stackA[(size_t)bounce * L.capacity + slot]; b = L.stackB[(size_t)bounce * L.capacity + slot];
-}
-RT_DEV void store_bounce(const RtLaunch& L, int bounce, uint32_t slot, float4 a, float4 b)
-{
-	L.stackA[(size_t)bounce * L.capacity + slot] = a; L.stackB[(size_t)bounce * L.capacity + slot] = b;
-}
-#endif
 
 // shard pixel slot -> image pixel (tiles interleaved across shards, 8x4 sub-blocks per warp)
 RT_DEV bool slot_to_pixel(const RtLaunch& L, uint32_t lp, uint32_t& x, uint32_t& y)
@@ -380,16 +337,6 @@ enum { LANE_EMPTY = 0, LANE_ACTIVE = 1, LANE_DONE = 2 };
 #ifndef RT_DEFAULT_BIN_DBITS
 #define RT_DEFAULT_BIN_DBITS 2      // bits per side of the octahedral direction map
 #endif
-#ifndef RT_HIT_TO_MEMORY
-#define RT_HIT_TO_MEMORY 1          // k_extend writes an accepted hit to the path's hit record at once instead of carrying bu / bv (needs RT_PACKED_STATE)
-#endif
-#if !RT_PACKED_STATE
-#undef RT_HIT_TO_MEMORY
-#define RT_HIT_TO_MEMORY 0          // the separate-arrays layout keeps the round-1 flush
-#endif
-#ifndef RT_PARK_DIRECTION
-#define RT_PARK_DIRECTION 0         // k_extend keeps {d, time} of its rays in shared memory while they walk inner nodes (see trav_run)
-#endif
 #ifndef RT_EXTEND_MIN_BLOCKS
 #define RT_EXTEND_MIN_BLOCKS 9      // CTAs of 128 threads per SM the traversal kernels are compiled for (register cap = 65536 / (128 * N));
                                     // 9 = 56 registers: 42 bytes of spills, all outside the node/leaf loops (8: 64 registers, 10: spills in the loops)
@@ -398,9 +345,6 @@ enum { LANE_EMPTY = 0, LANE_ACTIVE = 1, LANE_DONE = 2 };
 template<bool STATS>
 RT_DEV void extend_stage(const RtLaunch& L, int bounce, RtStack stack)
 {
-#if RT_PARK_DIRECTION
-	__shared__ float4 parkedDir[128];     // {d.xyz, time} of every lane's ray while it walks inner nodes (trav_run)
-#endif
 	const uint32_t cur = bounce & 1;
 	RtBounceCtl& bc = L.bounceCtl[bounce];
 	const uint32_t count = bc.extCount;
@@ -419,9 +363,7 @@ RT_DEV void extend_stage(const RtLaunch& L, int bounce, RtStack stack)
 		int target = -1;
 		if (state == LANE_DONE)
 		{
-		#if !RT_HIT_TO_MEMORY
-			store_hit(L, slot, make_float4(ts.best.t, ts.best.bu, ts.best.bv, __uint_as_float(ts.best.ref)));
-		#endif      // else: every accepted hit went to the record when it was accepted (trav_leaf); nobody reads the record of a miss
+			// every accepted hit went to the record when it was accepted (trav_leaf); nobody reads the record of a miss
 			if (ts.found()) target = ts.hitType;        // recorded when the hit was accepted: no dependent loads here
 			else target = RT_Q_MISS;
 			state = LANE_EMPTY;
@@ -446,9 +388,6 @@ RT_DEV void extend_stage(const RtLaunch& L, int bounce, RtStack stack)
 					float4 o, d;
 					load_ray(L, slot, o, d);
 					r = make_ray(xyz(o), xyz(d), o.w);
-				#if RT_PARK_DIRECTION
-					parkedDir[threadIdx.x] = make_float4(d.x, d.y, d.z, o.w);
-				#endif
 					if (STATS) count_reference_work(L.S, r, L.tMin, stack, st);
 					state = trav_begin<STATS>(L.S, r, L.tMin, ts, st) ? LANE_ACTIVE : LANE_DONE;
 				}
@@ -465,14 +404,8 @@ RT_DEV void extend_stage(const RtLaunch& L, int bounce, RtStack stack)
 
 		// ---- traverse until too few lanes are busy ----
 		bool alive = state == LANE_ACTIVE;
-	#if RT_HIT_TO_MEMORY
-		trav_run<false, STATS>(L.S, r, L.tMin, stack, ts, alive, exhausted ? 1u : L.refillThreshold, L.walkThreshold, st, nullptr,
+		trav_run<false, STATS>(L.S, r, L.tMin, stack, ts, alive, exhausted ? 1u : L.refillThreshold, L.walkThreshold, st,
 		                       reinterpret_cast<float4*>(L.hitCtl), slot);
-	#elif RT_PARK_DIRECTION
-		trav_run<false, STATS>(L.S, r, L.tMin, stack, ts, alive, exhausted ? 1u : L.refillThreshold, L.walkThreshold, st, parkedDir + threadIdx.x);
-	#else
-		trav_run<false, STATS>(L.S, r, L.tMin, stack, ts, alive, exhausted ? 1u : L.refillThreshold, L.walkThreshold, st);
-	#endif
 		if (state == LANE_ACTIVE && !alive) state = LANE_DONE;
 	}
 	if (STATS)
@@ -1271,7 +1204,7 @@ static int upload_array(RtDeviceScene* sc, const T* host, size_t count, const T*
 }
 
 // sRGB textures are decoded ONCE, when the scene is uploaded: the reference applies pow(x, 2.2) to all four channels of every
-// texel it fetches (render/texture.cc:45-51 -> image.h:79-83), a pure function of the texel, so running the very same rt_m_powf
+// texel it fetches (render/texture.cc:45-51 -> image.h:79-83), a pure function of the texel, so running the very same rt_powf
 // over the uploaded copy gives the bits a fetch-time decode would -- and takes four double-precision pow evaluations out
 // of every microfacet texture fetch and one out of every cut-out test inside the traversal loop.  Every (image, sRGB flag)
 // pair owns its texel range (RtSceneFlattener::AddTexture), so the in-place rewrite cannot touch a linear view of the image.
@@ -1280,7 +1213,7 @@ __global__ void __launch_bounds__(256) k_linearize_texels(float4* texels, uint64
 	for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (uint64_t)gridDim.x * blockDim.x)
 	{
 		float4 px = texels[i];
-		px.x = rt_m_powf(px.x, 2.2f); px.y = rt_m_powf(px.y, 2.2f); px.z = rt_m_powf(px.z, 2.2f); px.w = rt_m_powf(px.w, 2.2f);
+		px.x = rt_powf(px.x, 2.2f); px.y = rt_powf(px.y, 2.2f); px.z = rt_powf(px.z, 2.2f); px.w = rt_powf(px.w, 2.2f);
 		texels[i] = px;
 	}
 }
@@ -1484,13 +1417,8 @@ static int arena_alloc(RtPipe& pipe, T** out, size_t count)
 // bytes of path state per slot at a given bounce-stack depth (everything ensure_arena allocates per slot)
 static uint64_t arena_slot_bytes(int32_t depth)
 {
-#if RT_PACKED_STATE
 	return 32ull * 2 /* ray hitCtl */ + 16ull * 2 /* Li missPartial */ + 32ull * (uint64_t)std::max(1, depth) /* stack */
 	     + 4ull * (2 + RT_NUM_HIT_QUEUES + 1 + 2) /* extQ[2] matQ[] shadowQ extSorted extKey */;
-#else
-	return 16ull * 5 /* rayO rayD hit Li missPartial */ + 32ull * (uint64_t)std::max(1, depth) /* stackA stackB */
-	     + 4ull * (1 + 2 + RT_NUM_HIT_QUEUES + 1 + 3) /* rngCtr extQ[2] matQ[] shadowQ slotKey extSorted extKey */;
-#endif
 }
 static int ensure_arena(RtPipe& pipe, uint32_t slots, int32_t depth)
 {
@@ -1499,28 +1427,14 @@ static int ensure_arena(RtPipe& pipe, uint32_t slots, int32_t depth)
 	free_arena(pipe);
 	RtLaunch& L = pipe.L;
 	int rc;
-#if RT_PACKED_STATE
 	if ((rc = arena_alloc(pipe, &L.ray, slots))) return rc;
 	if ((rc = arena_alloc(pipe, &L.hitCtl, slots))) return rc;
 	if ((rc = arena_alloc(pipe, &L.stack, (size_t)slots * depth))) return rc;
-#else
-	if ((rc = arena_alloc(pipe, &L.rayO, slots))) return rc;
-	if ((rc = arena_alloc(pipe, &L.rayD, slots))) return rc;
-	if ((rc = arena_alloc(pipe, &L.hit, slots))) return rc;
-	if ((rc = arena_alloc(pipe, &L.stackA, (size_t)slots * depth))) return rc;
-	if ((rc = arena_alloc(pipe, &L.stackB, (size_t)slots * depth))) return rc;
-#endif
 	if ((rc = arena_alloc(pipe, &L.Li, slots))) return rc;
 	if ((rc = arena_alloc(pipe, &L.missPartial, slots))) return rc;
-#if !RT_PACKED_STATE
-	if ((rc = arena_alloc(pipe, &L.rngCtr, slots))) return rc;
-#endif
 	for (int i = 0; i < 2; ++i) if ((rc = arena_alloc(pipe, &L.extQ[i], slots))) return rc;
 	for (int i = 0; i < RT_NUM_HIT_QUEUES; ++i) if ((rc = arena_alloc(pipe, &L.matQ[i], slots))) return rc;
 	if ((rc = arena_alloc(pipe, &L.shadowQ, slots))) return rc;
-#if !RT_PACKED_STATE
-	if ((rc = arena_alloc(pipe, &L.slotKey, slots))) return rc;
-#endif
 	if ((rc = arena_alloc(pipe, &L.extSorted, slots))) return rc;
 	if ((rc = arena_alloc(pipe, &L.extKey, slots))) return rc;
 	if ((rc = arena_alloc(pipe, &L.binCount, RT_MAX_BINS))) return rc;
@@ -1545,22 +1459,21 @@ static uint32_t stack_levels(const RtDeviceScene* sc) { return std::max(8u, (sc-
 static bool stack_fits(uint32_t levels) { return levels <= RT_MAX_STACK; }
 
 // Grid of a persistent kernel: resident CTAs per SM x SMs.  The occupancy query is made once per (context, kernel) -- a
-// dozen of them per render call were a measurable part of millisecond frames.
+// dozen of them per render call were a measurable part of millisecond frames.  No kernel takes dynamic shared memory.
 template<typename Kernel>
-static int persistent_grid(RtRenderContext* ctx, Kernel kernel, int blockSize, size_t smem, int* outGrid)
+static int persistent_grid(RtRenderContext* ctx, Kernel kernel, int blockSize, int* outGrid)
 {
 	const void* key = reinterpret_cast<const void*>(kernel);
 	auto it = ctx->gridCache.find(key);
 	if (it != ctx->gridCache.end()) { *outGrid = it->second; return 0; }
 	int perSM = 0;
-	if (smem > 48 * 1024) RT_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-	RT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, kernel, blockSize, smem));
+	RT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, kernel, blockSize, 0));
 	*outGrid = ctx->numSMs * std::max(1, perSM);
 	ctx->gridCache[key] = *outGrid;
 	return 0;
 }
 
-static void fill_scene(RtLaunch& L, const RtDeviceScene* sc, const RtCamera* cam, const RtRenderParams* p, uint32_t stackLevels)
+static void fill_scene(RtLaunch& L, const RtDeviceScene* sc, const RtCamera* cam, const RtRenderParams* p)
 {
 	L.S = sc->view;
 	L.cam = *cam;
@@ -1615,6 +1528,31 @@ static void fill_scene(RtLaunch& L, const RtDeviceScene* sc, const RtCamera* cam
 	L.numBins = L.binBits ? (1u << L.binBits) : 0u;
 }
 
+// k_extend_pool's traversal stacks for a launch of `grid` CTAs, grown when a larger grid needs more
+static int ensure_pool_stack(RtPipe& pipe, int grid)
+{
+	const size_t entries = (size_t)grid * 4u * RT_MAX_STACK * RT_POOL_RAYS;
+	if (pipe.poolStackEntries < entries)
+	{
+		if (pipe.poolStack) cudaFree(pipe.poolStack);
+		pipe.poolStack = nullptr; pipe.poolStackEntries = 0;
+		RT_CUDA(cudaMalloc((void**)&pipe.poolStack, entries * sizeof(uint2)));
+		pipe.poolStackEntries = entries;
+	}
+	pipe.L.poolStack = pipe.poolStack;
+	return 0;
+}
+
+// Adds the traversal counters of a control block to `stats` (the ray counts and launch fields are the caller's).
+static void add_counters(RtRenderStats* stats, const RtQueueCtl& h)
+{
+	stats->boxTests += h.boxTests; stats->triTests += h.triTests; stats->sphereTests += h.sphereTests; stats->nodeVisits += h.nodeVisits;
+	stats->gateTests += h.gateTests; stats->cubeTests += h.cubeTests;
+	stats->refBoxTests += h.refBoxTests; stats->refTriTests += h.refTriTests; stats->refSphereTests += h.refSphereTests;
+	stats->nodeIters += h.nodeIters; stats->nodeStep += h.nodeStep; stats->nodeAlive += h.nodeAlive;
+	stats->leafIters += h.leafIters; stats->leafBusy += h.leafBusy;
+}
+
 extern "C" int rt_render_shard(RtRenderContext* ctx, const RtDeviceScene* sc, const RtCamera* cam,
                                const RtRenderParams* p, void* deviceShardOut, void* streamPtr, RtRenderStats* stats)
 {
@@ -1643,13 +1581,11 @@ extern "C" int rt_render_window(RtRenderContext* ctx, const RtDeviceScene* sc, c
 	RT_CUDA(cudaSetDevice(ctx->device));
 	cudaStream_t stream = (cudaStream_t)streamPtr;
 
-	const uint32_t levels = stack_levels(sc);
-	const size_t smem = 0;      // no dynamic shared memory: the traversal stack is thread-local
-	if (!stack_fits(levels)) { g_lastError = "rt_render_shard: BVH too deep for the traversal stack"; return -1; }
+	if (!stack_fits(stack_levels(sc))) { g_lastError = "rt_render_shard: BVH too deep for the traversal stack"; return -1; }
 
 	RtLaunch probe;
 	memset(&probe, 0, sizeof(probe));
-	fill_scene(probe, sc, cam, p, levels);
+	fill_scene(probe, sc, cam, p);
 	const uint32_t npix = probe.npix, spp = probe.spp;
 	const uint32_t win = spp - sampleBegin;      // samples per pixel this call renders
 	const bool pathTrace = p->renderMode == 0u;
@@ -1735,7 +1671,7 @@ extern "C" int rt_render_window(RtRenderContext* ctx, const RtDeviceScene* sc, c
 	{
 		RtPipe& pipe = ctx->pipe[q];
 		RtLaunch& L = pipe.L;
-		fill_scene(L, sc, cam, p, levels);
+		fill_scene(L, sc, cam, p);
 		L.capacity = pipe.capacity;
 		L.K = K;
 		L.accum = ctx->accum;
@@ -1762,8 +1698,8 @@ extern "C" int rt_render_window(RtRenderContext* ctx, const RtDeviceScene* sc, c
 	if (!pathTrace)
 	{
 		int grid = 0;
-		if ((rc = persistent_grid(ctx, k_debug_view, 128, smem, &grid))) return rc;
-		k_debug_view<<<grid, 128, smem, stream>>>(ctx->pipe[0].L);
+		if ((rc = persistent_grid(ctx, k_debug_view, 128, &grid))) return rc;
+		k_debug_view<<<grid, 128, 0, stream>>>(ctx->pipe[0].L);
 		launches++;
 	}
 	if (pathTrace && fused)
@@ -1772,12 +1708,12 @@ extern "C" int rt_render_window(RtRenderContext* ctx, const RtDeviceScene* sc, c
 		RtLaunch& L = pipe.L;
 		L.passBase = sampleBegin;
 		int grid = 0;
-		if ((rc = persistent_grid(ctx, k_pass_fused, 128, smem, &grid))) return rc;
+		if ((rc = persistent_grid(ctx, k_pass_fused, 128, &grid))) return rc;
 		RT_CUDA(cudaMemsetAsync(L.bounceCtl, 0, ((size_t)std::max(0, p->maxPathLength) + 2) * sizeof(RtBounceCtl), stream));
 		uint32_t materialMask = sc->materialTypeMask;
 		int firstPass = 1, lastPass = 1;
 		void* args[] = { (void*)&L, (void*)&materialMask, (void*)&firstPass, (void*)&lastPass };
-		const cudaError_t e = cudaLaunchCooperativeKernel((const void*)k_pass_fused, dim3((unsigned)grid), dim3(128), args, smem, stream);
+		const cudaError_t e = cudaLaunchCooperativeKernel((const void*)k_pass_fused, dim3((unsigned)grid), dim3(128), args, 0, stream);
 		if (e == cudaSuccess) { launches++; passes++; }
 		else
 		{
@@ -1790,38 +1726,30 @@ extern "C" int rt_render_window(RtRenderContext* ctx, const RtDeviceScene* sc, c
 	}
 	if (pathTrace && !fused)
 	{
+		// the shade kernels, indexed by RtMaterialType
+		void (*const shadeKernels[RT_MAT_NUM_TYPES])(RtLaunch, int) = {
+			k_shade<RT_MAT_LAMBERTIAN>, k_shade<RT_MAT_METAL>, k_shade<RT_MAT_DIELECTRIC>,
+			k_shade<RT_MAT_MIRROR>, k_shade<RT_MAT_LIGHT>, k_shade<RT_MAT_MICROFACET> };
 		int gridExtend = 0, gridShadow = 0, gridMiss = 0, gridShade[RT_MAT_NUM_TYPES];
 		const bool st = p->collectStats != 0;
-		if (st) { if ((rc = persistent_grid(ctx, k_extend<true>, 128, smem, &gridExtend))) return rc; }
-		else    { if ((rc = persistent_grid(ctx, k_extend<false>, 128, smem, &gridExtend))) return rc; }
-		if ((rc = persistent_grid(ctx, k_shadow, 128, smem, &gridShadow))) return rc;
-		if ((rc = persistent_grid(ctx, k_miss, 128, 0, &gridMiss))) return rc;
-		if ((rc = persistent_grid(ctx, k_shade<RT_MAT_LAMBERTIAN>, 128, 0, &gridShade[RT_MAT_LAMBERTIAN]))) return rc;
-		if ((rc = persistent_grid(ctx, k_shade<RT_MAT_METAL>, 128, 0, &gridShade[RT_MAT_METAL]))) return rc;
-		if ((rc = persistent_grid(ctx, k_shade<RT_MAT_DIELECTRIC>, 128, 0, &gridShade[RT_MAT_DIELECTRIC]))) return rc;
-		if ((rc = persistent_grid(ctx, k_shade<RT_MAT_MIRROR>, 128, 0, &gridShade[RT_MAT_MIRROR]))) return rc;
-		if ((rc = persistent_grid(ctx, k_shade<RT_MAT_LIGHT>, 128, 0, &gridShade[RT_MAT_LIGHT]))) return rc;
-		if ((rc = persistent_grid(ctx, k_shade<RT_MAT_MICROFACET>, 128, 0, &gridShade[RT_MAT_MICROFACET]))) return rc;
+		if (st) { if ((rc = persistent_grid(ctx, k_extend<true>, 128, &gridExtend))) return rc; }
+		else    { if ((rc = persistent_grid(ctx, k_extend<false>, 128, &gridExtend))) return rc; }
+		if ((rc = persistent_grid(ctx, k_shadow, 128, &gridShadow))) return rc;
+		if ((rc = persistent_grid(ctx, k_miss, 128, &gridMiss))) return rc;
+		for (int m = 0; m < RT_MAT_NUM_TYPES; ++m)
+			if ((rc = persistent_grid(ctx, shadeKernels[m], 128, &gridShade[m]))) return rc;
 		// opt-in: the pooled traversal kernel (a warp regroups its rays at every step) instead of k_extend
 		const bool pooled = p->tuning.pooledTraversal != 0 && !st;
 		int gridPool = 0;
 		if (pooled)
 		{
-			if ((rc = persistent_grid(ctx, k_extend_pool, 128, 0, &gridPool))) return rc;
+			if ((rc = persistent_grid(ctx, k_extend_pool, 128, &gridPool))) return rc;
 			if (p->tuning.poolCtas) gridPool = std::min(gridPool, ctx->numSMs * (int)p->tuning.poolCtas);
 			else if (pipes > 1) gridPool = std::min(gridPool, ctx->numSMs * (p->tuning.traversalCtas ? (int)p->tuning.traversalCtas : RT_DUAL_PIPE_TRAVERSAL_CTAS));
-			const size_t entries = (size_t)gridPool * 4u * RT_MAX_STACK * RT_POOL_RAYS;
 			for (int q = 0; q < pipes; ++q)
 			{
 				RtPipe& pipe = ctx->pipe[q];
-				if (pipe.poolStackEntries < entries)
-				{
-					if (pipe.poolStack) cudaFree(pipe.poolStack);
-					pipe.poolStack = nullptr; pipe.poolStackEntries = 0;
-					RT_CUDA(cudaMalloc((void**)&pipe.poolStack, entries * sizeof(uint2)));
-					pipe.poolStackEntries = entries;
-				}
-				pipe.L.poolStack = pipe.poolStack;
+				if ((rc = ensure_pool_stack(pipe, gridPool))) return rc;
 				pipe.L.poolNodeThreshold = p->tuning.poolNodeThreshold ? p->tuning.poolNodeThreshold : 24u;
 				pipe.L.poolRefill = p->tuning.poolRefill ? p->tuning.poolRefill : 24u;
 			}
@@ -1873,23 +1801,18 @@ extern "C" int rt_render_window(RtRenderContext* ctx, const RtDeviceScene* sc, c
 					}
 					RT_CUDA(cudaEventRecord(pipe.stageEvents[2 * ext], ps));
 				}
-				if (st) k_extend<true><<<gridExtend, 128, smem, ps>>>(L, b);
+				if (st) k_extend<true><<<gridExtend, 128, 0, ps>>>(L, b);
 				else if (pooled) k_extend_pool<<<gridPool, 128, 0, ps>>>(L, b);
-				else    k_extend<false><<<gridExtend, 128, smem, ps>>>(L, b);
+				else    k_extend<false><<<gridExtend, 128, 0, ps>>>(L, b);
 				if (timeStages) RT_CUDA(cudaEventRecord(pipe.stageEvents[2 * ext + 1], ps));
 				if (ring) { RT_CUDA(cudaEventRecord(pipe.evExtend, ps)); lastExtend = pipe.evExtend; }
 				ext++;
 				launches++;
-				const uint32_t mask = sc->materialTypeMask;
-				if (mask & (1u << RT_MAT_LAMBERTIAN)) { k_shade<RT_MAT_LAMBERTIAN><<<gridShade[RT_MAT_LAMBERTIAN], 128, 0, ps>>>(L, b); launches++; }
-				if (mask & (1u << RT_MAT_METAL))      { k_shade<RT_MAT_METAL><<<gridShade[RT_MAT_METAL], 128, 0, ps>>>(L, b); launches++; }
-				if (mask & (1u << RT_MAT_DIELECTRIC)) { k_shade<RT_MAT_DIELECTRIC><<<gridShade[RT_MAT_DIELECTRIC], 128, 0, ps>>>(L, b); launches++; }
-				if (mask & (1u << RT_MAT_MIRROR))     { k_shade<RT_MAT_MIRROR><<<gridShade[RT_MAT_MIRROR], 128, 0, ps>>>(L, b); launches++; }
-				if (mask & (1u << RT_MAT_LIGHT))      { k_shade<RT_MAT_LIGHT><<<gridShade[RT_MAT_LIGHT], 128, 0, ps>>>(L, b); launches++; }
-				if (mask & (1u << RT_MAT_MICROFACET)) { k_shade<RT_MAT_MICROFACET><<<gridShade[RT_MAT_MICROFACET], 128, 0, ps>>>(L, b); launches++; }
+				for (int m = 0; m < RT_MAT_NUM_TYPES; ++m)
+					if (sc->materialTypeMask & (1u << m)) { shadeKernels[m]<<<gridShade[m], 128, 0, ps>>>(L, b); launches++; }
 				k_miss<<<gridMiss, 128, 0, ps>>>(L, b);
 				launches++;
-				if (sc->view.hasSun) { k_shadow<<<gridShadow, 128, smem, ps>>>(L, b); launches++; }
+				if (sc->view.hasSun) { k_shadow<<<gridShadow, 128, 0, ps>>>(L, b); launches++; }
 				if (L.binBits && b + 1 < L.maxDepth)
 				{
 					k_bin_scan<<<1, 1024, 0, ps>>>(L.binCount, L.binCursor, L.numBins);
@@ -1924,13 +1847,9 @@ extern "C" int rt_render_window(RtRenderContext* ctx, const RtDeviceScene* sc, c
 		{
 			RtQueueCtl h;
 			RT_CUDA(cudaMemcpy(&h, ctx->pipe[q].ctl, sizeof(h), cudaMemcpyDeviceToHost));
+			add_counters(stats, h);
 			stats->rayQueries += h.rayQueries;
-			stats->boxTests += h.boxTests; stats->triTests += h.triTests; stats->sphereTests += h.sphereTests; stats->nodeVisits += h.nodeVisits;
-			stats->gateTests += h.gateTests; stats->cubeTests += h.cubeTests;
-			stats->refBoxTests += h.refBoxTests; stats->refTriTests += h.refTriTests; stats->refSphereTests += h.refSphereTests;
 			stats->statRays += h.statRays;
-			stats->nodeIters += h.nodeIters; stats->nodeStep += h.nodeStep; stats->nodeAlive += h.nodeAlive;
-			stats->leafIters += h.leafIters; stats->leafBusy += h.leafBusy;
 			stats->extendLaunches += extendLaunches[q];
 			if (timeStages)
 			{
@@ -2008,17 +1927,15 @@ extern "C" int rt_trace_closest(RtRenderContext* ctx, const RtDeviceScene* sc, c
 	RT_CUDA(cudaMemcpy(dRays, hostRays, (size_t)numRays * 32, cudaMemcpyHostToDevice));
 	RtQueueCtl* ctl = ctx->pipe[0].ctl;
 	RT_CUDA(cudaMemset(ctl, 0, sizeof(RtQueueCtl)));
-	const uint32_t levels = stack_levels(sc);
-	const size_t smem = 0;      // no dynamic shared memory: the traversal stack is thread-local
-	if (!stack_fits(levels)) { g_lastError = "rt_trace_closest: BVH too deep for the traversal stack"; return -1; }
+	if (!stack_fits(stack_levels(sc))) { g_lastError = "rt_trace_closest: BVH too deep for the traversal stack"; return -1; }
 	int grid = 0, rc;
 	const bool st = stats != nullptr;
-	if (st) { if ((rc = persistent_grid(ctx, k_trace_rays<true>, 128, smem, &grid))) return rc; }
-	else    { if ((rc = persistent_grid(ctx, k_trace_rays<false>, 128, smem, &grid))) return rc; }
+	if (st) { if ((rc = persistent_grid(ctx, k_trace_rays<true>, 128, &grid))) return rc; }
+	else    { if ((rc = persistent_grid(ctx, k_trace_rays<false>, 128, &grid))) return rc; }
 	grid = (int)std::min<int64_t>(grid, (numRays + 127) / 128);
 	RT_CUDA(cudaEventRecord(ctx->evStart, 0));
-	if (st) k_trace_rays<true><<<grid, 128, smem>>>(sc->view, dRays, numRays, tMin, dRank, dT, ctl);
-	else    k_trace_rays<false><<<grid, 128, smem>>>(sc->view, dRays, numRays, tMin, dRank, dT, ctl);
+	if (st) k_trace_rays<true><<<grid, 128>>>(sc->view, dRays, numRays, tMin, dRank, dT, ctl);
+	else    k_trace_rays<false><<<grid, 128>>>(sc->view, dRays, numRays, tMin, dRank, dT, ctl);
 	RT_CUDA(cudaEventRecord(ctx->evStop, 0));
 	RT_CUDA(cudaGetLastError());
 	RT_CUDA(cudaMemcpy(hostOutRank, dRank, (size_t)numRays * 4, cudaMemcpyDeviceToHost));
@@ -2030,10 +1947,8 @@ extern "C" int rt_trace_closest(RtRenderContext* ctx, const RtDeviceScene* sc, c
 		float ms = 0.0f;
 		RT_CUDA(cudaEventElapsedTime(&ms, ctx->evStart, ctx->evStop));
 		memset(stats, 0, sizeof(*stats));
+		add_counters(stats, h);
 		stats->rayQueries = (uint64_t)numRays;
-		stats->boxTests = h.boxTests; stats->triTests = h.triTests; stats->sphereTests = h.sphereTests; stats->nodeVisits = h.nodeVisits;
-		stats->gateTests = h.gateTests; stats->cubeTests = h.cubeTests;
-		stats->refBoxTests = h.refBoxTests; stats->refTriTests = h.refTriTests; stats->refSphereTests = h.refSphereTests;
 		stats->statRays = (uint64_t)numRays;
 		stats->deviceMs = ms;
 		stats->kernelLaunches = 1;
@@ -2063,13 +1978,8 @@ extern "C" int rt_trace_stage(RtRenderContext* ctx, const RtDeviceScene* sc, int
 			seen[hostOrder[i]] = 1;
 		}
 	}
-#if !RT_PACKED_STATE
-	g_lastError = "rt_trace_stage: needs the packed path-state layout (RT_PACKED_STATE 1)";
-	return -1;
-#else
 	RT_CUDA(cudaSetDevice(ctx->device));
-	const uint32_t levels = stack_levels(sc);
-	if (!stack_fits(levels)) { g_lastError = "rt_trace_stage: BVH too deep for the traversal stack"; return -1; }
+	if (!stack_fits(stack_levels(sc))) { g_lastError = "rt_trace_stage: BVH too deep for the traversal stack"; return -1; }
 	RtPipe& pipe = ctx->pipe[0];
 	int rc;
 	if ((rc = ensure_arena(pipe, n, 1))) return rc;
@@ -2084,7 +1994,7 @@ extern "C" int rt_trace_stage(RtRenderContext* ctx, const RtDeviceScene* sc, int
 	RtCamera cam;
 	memset(&cam, 0, sizeof(cam));
 	RtLaunch L = pipe.L;         // the arena's pointers
-	fill_scene(L, sc, &cam, &p, levels);
+	fill_scene(L, sc, &cam, &p);
 	L.capacity = pipe.capacity;
 	L.K = 1;
 	L.ctl = pipe.ctl;
@@ -2097,24 +2007,15 @@ extern "C" int rt_trace_stage(RtRenderContext* ctx, const RtDeviceScene* sc, int
 	}
 
 	int grid = 0;
-	const size_t smem = 0;
-	if (mode == RT_STAGE_EXTEND) rc = persistent_grid(ctx, k_extend<false>, 128, smem, &grid);
-	else if (mode == RT_STAGE_EXTEND_STATS) rc = persistent_grid(ctx, k_extend<true>, 128, smem, &grid);
-	else if (mode == RT_STAGE_EXTEND_POOL) rc = persistent_grid(ctx, k_extend_pool, 128, 0, &grid);
-	else rc = persistent_grid(ctx, k_shadow, 128, smem, &grid);
+	if (mode == RT_STAGE_EXTEND) rc = persistent_grid(ctx, k_extend<false>, 128, &grid);
+	else if (mode == RT_STAGE_EXTEND_STATS) rc = persistent_grid(ctx, k_extend<true>, 128, &grid);
+	else if (mode == RT_STAGE_EXTEND_POOL) rc = persistent_grid(ctx, k_extend_pool, 128, &grid);
+	else rc = persistent_grid(ctx, k_shadow, 128, &grid);
 	if (rc) return rc;
 	if (schedule->gridCtas) grid = (int)schedule->gridCtas;
 	if (mode == RT_STAGE_EXTEND_POOL)
 	{
-		const size_t entries = (size_t)grid * 4u * RT_MAX_STACK * RT_POOL_RAYS;
-		if (pipe.poolStackEntries < entries)
-		{
-			if (pipe.poolStack) cudaFree(pipe.poolStack);
-			pipe.poolStack = nullptr; pipe.poolStackEntries = 0;
-			RT_CUDA(cudaMalloc((void**)&pipe.poolStack, entries * sizeof(uint2)));
-			pipe.poolStackEntries = entries;
-		}
-		pipe.L.poolStack = pipe.poolStack;
+		if ((rc = ensure_pool_stack(pipe, grid))) return rc;
 		L.poolStack = pipe.poolStack;
 		L.poolNodeThreshold = schedule->poolNodeThreshold ? schedule->poolNodeThreshold : 24u;
 		L.poolRefill = schedule->poolRefill ? schedule->poolRefill : 24u;
@@ -2138,10 +2039,10 @@ extern "C" int rt_trace_stage(RtRenderContext* ctx, const RtDeviceScene* sc, int
 	RT_CUDA(cudaMemset(pipe.ctl, 0, sizeof(RtQueueCtl)));
 
 	RT_CUDA(cudaEventRecord(ctx->evStart, 0));
-	if (mode == RT_STAGE_EXTEND) k_extend<false><<<grid, 128, smem>>>(L, 0);
-	else if (mode == RT_STAGE_EXTEND_STATS) k_extend<true><<<grid, 128, smem>>>(L, 0);
-	else if (mode == RT_STAGE_EXTEND_POOL) k_extend_pool<<<grid, 128, 0>>>(L, 0);
-	else k_shadow<<<grid, 128, smem>>>(L, 0);
+	if (mode == RT_STAGE_EXTEND) k_extend<false><<<grid, 128>>>(L, 0);
+	else if (mode == RT_STAGE_EXTEND_STATS) k_extend<true><<<grid, 128>>>(L, 0);
+	else if (mode == RT_STAGE_EXTEND_POOL) k_extend_pool<<<grid, 128>>>(L, 0);
+	else k_shadow<<<grid, 128>>>(L, 0);
 	RT_CUDA(cudaEventRecord(ctx->evStop, 0));
 	RT_CUDA(cudaGetLastError());
 	RT_CUDA(cudaDeviceSynchronize());
@@ -2188,19 +2089,14 @@ extern "C" int rt_trace_stage(RtRenderContext* ctx, const RtDeviceScene* sc, int
 		float ms = 0.0f;
 		RT_CUDA(cudaEventElapsedTime(&ms, ctx->evStart, ctx->evStop));
 		memset(stats, 0, sizeof(*stats));
+		add_counters(stats, h);
 		stats->rayQueries = n;
-		stats->boxTests = h.boxTests; stats->triTests = h.triTests; stats->sphereTests = h.sphereTests; stats->nodeVisits = h.nodeVisits;
-		stats->gateTests = h.gateTests; stats->cubeTests = h.cubeTests;
-		stats->refBoxTests = h.refBoxTests; stats->refTriTests = h.refTriTests; stats->refSphereTests = h.refSphereTests;
 		stats->statRays = h.statRays;
-		stats->nodeIters = h.nodeIters; stats->nodeStep = h.nodeStep; stats->nodeAlive = h.nodeAlive;
-		stats->leafIters = h.leafIters; stats->leafBusy = h.leafBusy;
 		stats->deviceMs = ms;
 		stats->kernelLaunches = 1;
 		stats->extendLaunches = mode == RT_STAGE_SHADOW ? 0u : 1u;
 	}
 	return 0;
-#endif
 }
 
 // ---- Image2D::PostProcess on the device (render/image.cc:44-103) -----------------------------------------
@@ -2244,7 +2140,7 @@ __global__ void __launch_bounds__(256) k_tonemap(float4* image, uint32_t count, 
 		}
 		rgb = v3(fminf(1.0f, rgb.x), fminf(1.0f, rgb.y), fminf(1.0f, rgb.z));
 		const float g = 1.0f / 2.2f;
-		rgb = v3(rt_m_powf(rgb.x, g), rt_m_powf(rgb.y, g), rt_m_powf(rgb.z, g));
+		rgb = v3(rt_powf(rgb.x, g), rt_powf(rgb.y, g), rt_powf(rgb.z, g));
 		px.x = rgb.x; px.y = rgb.y; px.z = rgb.z;
 		image[i] = px;
 		if (outArgb8)
@@ -2521,16 +2417,16 @@ __global__ void __launch_bounds__(256) k_libm_eval(int fn, const float* x, const
 		float r;
 		switch (fn)
 		{
-		case 0: r = rt_m_sinf(a); break;
-		case 1: r = rt_m_cosf(a); break;
-		case 2: r = rt_m_tanf(a); break;
-		case 3: r = rt_m_asinf(a); break;
-		case 4: r = rt_m_acosf(a); break;
-		case 5: r = rt_m_atanf(a); break;
-		case 6: r = rt_m_expf(a); break;
-		case 7: r = rt_m_logf(a); break;
-		case 8: r = rt_m_powf(a, b); break;
-		default: r = rt_m_atan2f(a, b); break;
+		case 0: r = rt_sinf(a); break;
+		case 1: r = rt_cosf(a); break;
+		case 2: r = rt_tanf(a); break;
+		case 3: r = rt_asinf(a); break;
+		case 4: r = rt_acosf(a); break;
+		case 5: r = rt_atanf(a); break;
+		case 6: r = rt_expf(a); break;
+		case 7: r = rt_logf(a); break;
+		case 8: r = rt_powf(a, b); break;
+		default: r = rt_atan2f(a, b); break;
 		}
 		out[i] = r;
 	}

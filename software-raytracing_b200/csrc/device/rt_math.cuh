@@ -8,37 +8,10 @@
 
 #define RT_DEV __device__ __forceinline__
 
-// Transcendentals.  RT_EXACT_LIBM 1 (default): include/rt_libm.h, glibc's float algorithms restated operation for operation
-// (double-precision polynomials, the library's own tables): the shaders consume the SAME BITS as the reference's host build,
-// so the only remaining differences from the oracle are the documented epsilon ties of the traversal.  0: CUDA's libdevice
-// functions (1-2 ulp away from glibc; what round 1 shipped).
-#ifndef RT_EXACT_LIBM
-#define RT_EXACT_LIBM 1
-#endif
-#if RT_EXACT_LIBM
+// Transcendentals: include/rt_libm.h, glibc's float algorithms restated operation for operation (double-precision
+// polynomials, the library's own tables), so the shaders consume the SAME BITS as the reference's host build; CUDA's
+// libdevice functions are 1-2 ulp away from glibc, enough to change images (profiles/r02c_exact_libm_variants.jsonl).
 #include "rt_libm.h"
-#define rt_m_sinf rt_sinf
-#define rt_m_cosf rt_cosf
-#define rt_m_tanf rt_tanf
-#define rt_m_asinf rt_asinf
-#define rt_m_acosf rt_acosf
-#define rt_m_atanf rt_atanf
-#define rt_m_atan2f rt_atan2f
-#define rt_m_expf rt_expf
-#define rt_m_logf rt_logf
-#define rt_m_powf rt_powf
-#else
-#define rt_m_sinf sinf
-#define rt_m_cosf cosf
-#define rt_m_tanf tanf
-#define rt_m_asinf asinf
-#define rt_m_acosf acosf
-#define rt_m_atanf atanf
-#define rt_m_atan2f atan2f
-#define rt_m_expf expf
-#define rt_m_logf logf
-#define rt_m_powf powf
-#endif
 
 RT_DEV float3 v3(float x, float y, float z) { return make_float3(x, y, z); }
 RT_DEV float3 v3(float s) { return make_float3(s, s, s); }
@@ -78,26 +51,12 @@ RT_DEV float4 ldg4(const float4* p) { return __ldg(p); }
 // triangle put half as many wavefronts through L1TEX as four 128-bit loads -- the traversal kernels are bound
 // by that pipe, not by DRAM or issue slots (profiles/README.md).  `p` must be 32-byte aligned.
 struct __align__(32) RtF8 { float4 lo, hi; };
-#define RT_LDG8_ASM(hint, r, p) asm volatile("ld.global.nc" hint ".v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];" \
-		: "=f"(r.lo.x), "=f"(r.lo.y), "=f"(r.lo.z), "=f"(r.lo.w), "=f"(r.hi.x), "=f"(r.hi.y), "=f"(r.hi.z), "=f"(r.hi.w) : "l"(p))
-RT_DEV RtF8 ldg8(const void* p) { RtF8 r; RT_LDG8_ASM("", r, p); return r; }
-// The same load with an L1 policy.  The traversal stack lives in thread-local memory, i.e. in L1 next to the scene data:
-// ncu shows 40 % of the stack pops missing L1 when every triangle record a ray ever tests is allocated there too.
-// Inner nodes (re-used by the other lanes and warps of the SM) are kept with evict_last; triangle records (hardly ever
-// re-used before eviction) are streamed.  RT_NODE_LOAD_HINT / RT_TRI_LOAD_HINT: 0 plain, 1 no_allocate, 2 evict_first, 3 evict_last.
-#ifndef RT_NODE_LOAD_HINT
-#define RT_NODE_LOAD_HINT 0
-#endif
-#ifndef RT_TRI_LOAD_HINT
-#define RT_TRI_LOAD_HINT 0
-#endif
-template<int HINT> RT_DEV RtF8 ldg8_hint(const void* p)
+// No L1 eviction policy: hints on the node and triangle loads measured within +-0.5 % (profiles/README.md).
+RT_DEV RtF8 ldg8(const void* p)
 {
 	RtF8 r;
-	if (HINT == 1) RT_LDG8_ASM(".L1::no_allocate", r, p);
-	else if (HINT == 2) RT_LDG8_ASM(".L1::evict_first", r, p);
-	else if (HINT == 3) RT_LDG8_ASM(".L1::evict_last", r, p);
-	else RT_LDG8_ASM("", r, p);
+	asm volatile("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+		: "=f"(r.lo.x), "=f"(r.lo.y), "=f"(r.lo.z), "=f"(r.lo.w), "=f"(r.hi.x), "=f"(r.hi.y), "=f"(r.hi.z), "=f"(r.hi.w) : "l"(p));
 	return r;
 }
 // Two IEEE fused multiply-adds in one instruction (sm_100a: FFMA2, fma.rn.f32x2): {a.x*b.x+c.x, a.y*b.y+c.y}, each half
@@ -112,6 +71,3 @@ RT_DEV float2 fma2_rn(float2 a, float2 b, float2 c)
 	    : "=f"(d.x), "=f"(d.y) : "f"(a.x), "f"(a.y), "f"(b.x), "f"(b.y), "f"(c.x), "f"(c.y));
 	return d;
 }
-
-RT_DEV RtF8 ldg8_node(const void* p) { return ldg8_hint<RT_NODE_LOAD_HINT>(p); }
-RT_DEV RtF8 ldg8_tri(const void* p) { return ldg8_hint<RT_TRI_LOAD_HINT>(p); }

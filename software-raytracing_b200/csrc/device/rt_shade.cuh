@@ -36,7 +36,7 @@ RT_DEV float3 random_on_sphere(RtRng& rng)
 	const float z = 1.0f - 2.0f * u1;
 	const float r = sqrtf(fmaxf(0.0f, 1.0f - z * z));
 	const float phi = 2.0f * 3.141592f * u2;
-	return v3(r * rt_m_cosf(phi), r * rt_m_sinf(phi), z);
+	return v3(r * rt_cosf(phi), r * rt_sinf(phi), z);
 }
 
 // core/random.cc:44-50
@@ -46,7 +46,7 @@ RT_DEV float3 random_in_disk(RtRng& rng)
 	const float u2 = rng.next();
 	const float r = sqrtf(u1);
 	const float theta = 2.0f * 3.14159265358979323846f * u2;
-	return v3(r * rt_m_cosf(theta), r * rt_m_sinf(theta), 0.0f);
+	return v3(r * rt_cosf(theta), r * rt_sinf(theta), 0.0f);
 }
 
 // render/camera.h:44-53 (the derived block is computed on the host, camera.h:55-78)
@@ -96,8 +96,8 @@ RT_DEV void reconstruct_surface(const RtSceneView& S, const RtRay& r, const RtHi
 		const float4 s = ldg4(S.spheres + idx);
 		const float3 op = sf.p - v3(s.x, s.y, s.z);
 		sf.n = op / s.w;
-		sf.u = rt_m_atanf(op.y / op.x);
-		sf.v = rt_m_acosf(op.z / s.w);
+		sf.u = rt_atanf(op.y / op.x);
+		sf.v = rt_acosf(op.z / s.w);
 		sf.material = S.sphereMaterial[idx];
 	}
 	else
@@ -120,7 +120,7 @@ RT_DEV float erf_inv(float x)
 {
 	float w, p;
 	x = clampf(x, -.99999f, .99999f);
-	w = -rt_m_logf((1.0f - x) * (1.0f + x));
+	w = -rt_logf((1.0f - x) * (1.0f + x));
 	if (w < 5.0f)
 	{
 		w = w - 2.5f;
@@ -157,7 +157,7 @@ RT_DEV float erf_as(float x)
 	const int sign = (x < 0.0f) ? -1 : 1;
 	x = fabsf(x);
 	const float t = 1.0f / (1.0f + pp * x);
-	const float y = 1.0f - (((((a5 * t + a4) * t) + a3) * t + a2) * t + a1) * t * rt_m_expf(-x * x);
+	const float y = 1.0f - (((((a5 * t + a4) * t) + a3) * t + a2) * t + a1) * t * rt_expf(-x * x);
 	return (float)sign * y;
 }
 
@@ -170,9 +170,9 @@ RT_DEV void beckmann_sample11(float cosThetaI, float U1, float U2, float* slope_
 	const float Pi = RT_BRDF_PI;
 	if ((double)cosThetaI > .9999)
 	{
-		const float r = sqrtf(-rt_m_logf(1.0f - U1));
-		const float sinPhi = rt_m_sinf(2.0f * Pi * U2);
-		const float cosPhi = rt_m_cosf(2.0f * Pi * U2);
+		const float r = sqrtf(-rt_logf(1.0f - U1));
+		const float sinPhi = rt_sinf(2.0f * Pi * U2);
+		const float cosPhi = rt_cosf(2.0f * Pi * U2);
 		*slope_x = r * cosPhi;
 		*slope_y = r * sinPhi;
 		return;
@@ -184,19 +184,19 @@ RT_DEV void beckmann_sample11(float cosThetaI, float U1, float U2, float* slope_
 	float a = -1.0f, c = erf_as(cotThetaI);
 	const float sample_x = fmaxf(U1, 1e-6f);
 
-	const float thetaI = rt_m_acosf(cosThetaI);
+	const float thetaI = rt_acosf(cosThetaI);
 	const float fit = 1.0f + thetaI * (-0.876f + thetaI * (0.4265f - 0.0594f * thetaI));
-	float b = c - (1.0f + c) * rt_m_powf(1.0f - sample_x, fit);
+	float b = c - (1.0f + c) * rt_powf(1.0f - sample_x, fit);
 
 	const float SQRT_PI_INV = 1.f / sqrtf(Pi);
-	const float normalization = 1.0f / (1.0f + c + SQRT_PI_INV * tanThetaI * rt_m_expf(-cotThetaI * cotThetaI));
+	const float normalization = 1.0f / (1.0f + c + SQRT_PI_INV * tanThetaI * rt_expf(-cotThetaI * cotThetaI));
 
 	int it = 0;
 	while (++it < 10)
 	{
 		if (!(b >= a && b <= c)) b = 0.5f * (a + c);
 		const float invErf = erf_inv(b);
-		const float value = normalization * (1.0f + b + SQRT_PI_INV * tanThetaI * rt_m_expf(-invErf * invErf)) - sample_x;
+		const float value = normalization * (1.0f + b + SQRT_PI_INV * tanThetaI * rt_expf(-invErf * invErf)) - sample_x;
 		const float derivative = normalization * (1.0f - invErf * tanThetaI);
 		if (fabsf(value) < 1e-5f) break;
 		if (value > 0.0f) c = b; else a = b;
@@ -219,7 +219,7 @@ RT_DEV float3 beckmann_sample(float3 wi, float alpha_x, float alpha_y, float U1,
 	return normalize3(v3(-slope_x, -slope_y, 1.f));
 }
 
-RT_DEV float3 fresnel_schlick(float cosTheta, float3 F0) { return F0 + (1.0f - F0) * rt_m_powf(1.0f - cosTheta, 5.0f); }
+RT_DEV float3 fresnel_schlick(float cosTheta, float3 F0) { return F0 + (1.0f - F0) * rt_powf(1.0f - cosTheta, 5.0f); }
 
 RT_DEV float distribution_beckmann(float3 N, float3 H, float roughness)
 {
@@ -229,15 +229,15 @@ RT_DEV float distribution_beckmann(float3 N, float3 H, float roughness)
 	const float cosH2 = cosH * cosH;
 	const float rr = roughness * roughness;
 	const float exp_x = (1.0f - cosH2) / (rr * cosH);
-	const float num = (cosH > 0.0f ? 1.0f : 0.0f) * rt_m_expf(-exp_x);
+	const float num = (cosH > 0.0f ? 1.0f : 0.0f) * rt_expf(-exp_x);
 	const float denom = RT_BRDF_PI * rr * cosH2 * cosH2;
 	return num / denom;
 }
 
 RT_DEV float geometry_beckmann(float3 N, float3 H, float3 V, float roughness)
 {
-	const float thetaV = rt_m_acosf(dot3(N, V));
-	const float tanThetaV = rt_m_tanf(thetaV);
+	const float thetaV = rt_acosf(dot3(N, V));
+	const float tanThetaV = rt_tanf(thetaV);
 	const float a = 1.0f / (roughness * tanThetaV);
 	const float aa = a * a;
 	if (dot3(V, H) / dot3(V, N) <= 0.0f) return 0.0f;
@@ -365,7 +365,7 @@ RT_DEV void scatter(const RtSceneView& S, const RtMaterial& m, const RtRay& r, c
 			refracted = ni_over_nt * (unit - outward_normal * dt) - outward_normal * sqrtf(disc);
 			float r0 = (1.0f - ref_idx) / (1.0f + ref_idx);
 			r0 = r0 * r0;
-			reflect_prob = r0 + (1.0f - r0) * rt_m_powf(1.0f - cosine, 5.0f);
+			reflect_prob = r0 + (1.0f - r0) * rt_powf(1.0f - cosine, 5.0f);
 		}
 		else
 		{
@@ -433,7 +433,7 @@ RT_DEV float3 sky_radiance(const RtSceneView& S, float3 d)
 	{
 		const float3 dir = normalize3(d);
 		const float3 D = v3(dot3(v3(S.skyRotation + 0), dir), dot3(v3(S.skyRotation + 3), dir), dot3(v3(S.skyRotation + 6), dir));
-		float u = rt_m_atan2f(D.z, D.x), v = rt_m_asinf(D.y);
+		float u = rt_atan2f(D.z, D.x), v = rt_asinf(D.y);
 		u *= 0.1591f; v *= 0.3183f;
 		u += 0.5f; v += 0.5f;
 		const RtTexture tx = S.textures[S.skyTexture];

@@ -23,14 +23,6 @@
 #include <float.h>
 
 #define RT_PRUNE_SLACK 2.0e-3f
-#ifndef RT_BRANCHLESS_POP
-#define RT_BRANCHLESS_POP 1
-#endif
-// RT_PLANE_FMA2 1: the near and the far plane of a child on one axis are evaluated by ONE packed fma.rn.f32x2 (FFMA2):
-// 12 instead of 24 FFMA per inner node.  Same roundings (each half is an IEEE fma), same results.
-#ifndef RT_PLANE_FMA2
-#define RT_PLANE_FMA2 1
-#endif
 // stack-pop attempts per traversal step (an entry beyond the best hit is dropped; with one attempt the lane retries in its
 // next step, which the warp runs anyway for its other lanes)
 // RT_POP_HOISTED 1: the two stack entries a step may pop are loaded at the START of the step, next to the node fetch, instead
@@ -136,8 +128,8 @@ RT_DEV float4 sample_texture_impl(const RtSceneView& S, int32_t texIndex, float 
 	{
 		// SRGBToLinear decodes all four channels, alpha included (render/image.h:79-83); the cut-out test of the traversal
 		// loop only looks at alpha, so it skips the three powf it would throw away
-		if (!ALPHA_ONLY) { px.x = rt_m_powf(px.x, 2.2f); px.y = rt_m_powf(px.y, 2.2f); px.z = rt_m_powf(px.z, 2.2f); }
-		px.w = rt_m_powf(px.w, 2.2f);
+		if (!ALPHA_ONLY) { px.x = rt_powf(px.x, 2.2f); px.y = rt_powf(px.y, 2.2f); px.z = rt_powf(px.z, 2.2f); }
+		px.w = rt_powf(px.w, 2.2f);
 	}
 	return px;
 }
@@ -196,7 +188,7 @@ RT_DEV bool gate_passes(const RtSceneView& S, uint32_t gate, const RtRay& r, flo
 RT_DEV bool triangle_test(const RtSceneView& S, uint32_t idx, const RtRay& r, float tMin, float tLimit,
                           float& outT, float& outBu, float& outBv, int32_t& outMatType, uint32_t& gateTests)
 {
-	const RtF8 ta = ldg8_tri(S.triHot + 4u * (size_t)idx), tb = ldg8_tri(S.triHot + 4u * (size_t)idx + 2);
+	const RtF8 ta = ldg8(S.triHot + 4u * (size_t)idx), tb = ldg8(S.triHot + 4u * (size_t)idx + 2);
 	const float4 q0 = ta.lo, q1 = ta.hi, q2 = tb.lo;
 	const float3 v0 = v3(q0.x, q0.y, q0.z);
 	const float3 n  = v3(q0.w, q1.x, q1.y);
@@ -293,28 +285,12 @@ RT_DEV bool cube_test(const RtSceneView& S, uint32_t idx, const RtRay& r, float 
 // alternatives that lost (profiles/README.md): all of it in shared memory, a shared-memory window for the newest
 // entries, the newest entry in registers.
 #define RT_MAX_STACK 96
-// RT_STACK_SMEM_LEVELS > 0: the lowest N levels of every thread's stack live in shared memory (a stack pop is on the
-// critical path of the walk -- pop, node address, node load -- and ncu shows 40 % of the local-memory pops missing L1);
-// deeper levels fall back to local memory.  CTAs of the traversal kernels have 128 threads.
-#ifndef RT_STACK_SMEM_LEVELS
-#define RT_STACK_SMEM_LEVELS 0
-#endif
 struct RtStack
 {
 	uint2*   base;
 	uint32_t stride;
-#if RT_STACK_SMEM_LEVELS > 0
-	uint2*   sm;        // this thread's column of the CTA's shared block: level i at sm[i * 128]
-	RT_DEV void push(uint32_t level, uint32_t ref, float entry)
-	{
-		const uint2 e = make_uint2(ref, __float_as_uint(entry));
-		if (level < RT_STACK_SMEM_LEVELS) sm[level * 128u] = e; else base[level * stride] = e;
-	}
-	RT_DEV uint2 at(uint32_t level) const { return level < RT_STACK_SMEM_LEVELS ? sm[level * 128u] : base[level * stride]; }
-#else
 	RT_DEV void push(uint32_t level, uint32_t ref, float entry) { base[level * stride] = make_uint2(ref, __float_as_uint(entry)); }
 	RT_DEV uint2 at(uint32_t level) const { return base[level * stride]; }
-#endif
 };
 
 // Resumable traversal state of one ray, so that a warp can swap finished rays for fresh ones while the
@@ -358,7 +334,7 @@ RT_DEV bool trav_begin(const RtSceneView& S, const RtRay& r, float tMin, RtTrav&
 // reference's rule: minimum t, ties to the highest in-order rank.  Returns true if an any-hit query is done.
 // `hitRecords` (optional): when given, an accepted hit is written straight to record `hitSlot` there ({t, bu, bv, ref}: the first
 // half of the path's 32-byte hit record) instead of being carried in ts.best.bu / .bv until the ray is done: two registers
-// less across the node loop of k_extend (RT_HIT_TO_MEMORY); a ray accepts one or two hits in its life.
+// less across the node loop of k_extend (+1-2.5 %, profiles/README.md); a ray accepts one or two hits in its life.
 template<bool ANY_HIT, bool STATS>
 RT_DEV bool trav_leaf(const RtSceneView& S, const RtRay& r, float tMin, uint32_t leaf, RtTrav& ts, RtTravStats& st,
                       float4* hitRecords = nullptr, uint32_t hitSlot = 0u)
@@ -440,7 +416,7 @@ RT_DEV void trav_step(const RtSceneView& S, const RtRay& r, float tMin, RtStack 
 	{
 		// 64-byte RtNodeQ4 in two 256-bit loads: {base.xyz Sx qlo.xyz qhi.x} {qhi.yz ref[4] Sy Sz}
 		const float4* np = S.nodes + 4u * (size_t)RT_REF_INDEX(cur);
-		const RtF8 A = ldg8_node(np), B = ldg8_node(np + 2);
+		const RtF8 A = ldg8(np), B = ldg8(np + 2);
 		if (STATS) { st.nodes++; }
 		uint32_t r0 = __float_as_uint(B.lo.z), r1 = __float_as_uint(B.lo.w), r2 = __float_as_uint(B.hi.x), r3 = __float_as_uint(B.hi.y);
 		// Conservative slab test in ray space.  A child plane is p = m*S + base (m in [0.5, 2) from the stored byte), so
@@ -464,8 +440,8 @@ RT_DEV void trav_step(const RtSceneView& S, const RtRay& r, float tMin, RtStack 
 		const uint32_t nwz = nz ? whz : wlz, fwz = nz ? wlz : whz;
 		float e0, e1, e2, e3;
 		#define RT_Q4_M(word, k) __uint_as_float(rt_prmt(word, S.q4magic, 0x7044u | ((k) << 8)))
-		#define RT_Q4_T(word, k, a, b) __fmaf_rn(RT_Q4_M(word, k), a, b)
-	#if RT_PLANE_FMA2
+		// the near and the far plane of a child on one axis in ONE packed fma.rn.f32x2 (FFMA2): 12 instead of 24 FFMA per
+		// inner node, same roundings (+0.3-0.5 %, profiles/README.md)
 		#define RT_Q4_CHILD(k, e, p) { \
 			const float2 tx = fma2_rn(make_float2(RT_Q4_M(nwx, k), RT_Q4_M(fwx, k)), make_float2(ax, ax), make_float2(bnx, bfx)); \
 			const float2 ty = fma2_rn(make_float2(RT_Q4_M(nwy, k), RT_Q4_M(fwy, k)), make_float2(ay, ay), make_float2(bny, bfy)); \
@@ -474,17 +450,9 @@ RT_DEV void trav_step(const RtSceneView& S, const RtRay& r, float tMin, RtStack 
 			const float tf = fminf(fminf(tx.y, ty.y), tz.y); \
 			e = fmaxf(__fmaf_rn(-kSlack, fabsf(tn), tn), tMin); \
 			p = e <= fminf(__fmaf_rn(kSlack, fabsf(tf), tf) + tMin, ts.limit); }
-	#else
-		#define RT_Q4_CHILD(k, e, p) { \
-			const float tn = fmaxf(fmaxf(RT_Q4_T(nwx, k, ax, bnx), RT_Q4_T(nwy, k, ay, bny)), RT_Q4_T(nwz, k, az, bnz)); \
-			const float tf = fminf(fminf(RT_Q4_T(fwx, k, ax, bfx), RT_Q4_T(fwy, k, ay, bfy)), RT_Q4_T(fwz, k, az, bfz)); \
-			e = fmaxf(__fmaf_rn(-kSlack, fabsf(tn), tn), tMin); \
-			p = e <= fminf(__fmaf_rn(kSlack, fabsf(tf), tf) + tMin, ts.limit); }
-	#endif
 		bool p0, p1, p2, p3;
 		RT_Q4_CHILD(0, e0, p0); RT_Q4_CHILD(1, e1, p1); RT_Q4_CHILD(2, e2, p2); RT_Q4_CHILD(3, e3, p3);
 		#undef RT_Q4_CHILD
-		#undef RT_Q4_T
 		#undef RT_Q4_M
 		// absent children carry an inverted box (lo at the top of the grid, hi at the bottom); the slack could let a
 		// ray through it, so they are masked explicitly
@@ -527,7 +495,7 @@ RT_DEV void trav_step(const RtSceneView& S, const RtRay& r, float tMin, RtStack 
 		cur = pop2 ? next2 : cur;
 		ts.sp = pop2 ? ts.sp - (has2 ? 1u : 0u) : ts.sp;
 	}
-#elif RT_BRANCHLESS_POP
+#else
 	// two pop attempts as straight-line code: the top entry is read whether or not this lane pops (slot 0 when the
 	// stack is empty: never used), the selects do the rest -- no divergent regions, ~16 instructions fewer per step
 	#pragma unroll
@@ -540,20 +508,6 @@ RT_DEV void trav_step(const RtSceneView& S, const RtRay& r, float tMin, RtStack 
 		const uint32_t next = !has ? RT_REF_DONE : ((__uint_as_float(e.y) > ts.limit) ? RT_REF_POP : e.x);
 		cur = pop ? next : cur;
 		ts.sp = pop ? idx : ts.sp;
-	}
-#else
-	#pragma unroll
-	for (int attempt = 0; attempt < 2; ++attempt)
-	{
-		if (cur == RT_REF_POP)
-		{
-			if (ts.sp == 0) cur = RT_REF_DONE;
-			else
-			{
-				const uint2 e = stack.at(--ts.sp);
-				cur = (__uint_as_float(e.y) > ts.limit) ? RT_REF_POP : e.x;
-			}
-		}
 	}
 #endif
 	ts.cur = cur;
@@ -579,12 +533,9 @@ RT_DEV bool trav_pending_leaf(const RtSceneView& S, const RtRay& r, float tMin, 
 // `walkThreshold` lanes can and at least one lane is blocked on leaves -- waiting for the slowest lane to
 // collect its leaves left 2/3 of the SIMD lanes idle (ncu: 9.8 active threads per warp).
 // Leaf phase: every lane with a pending leaf tests it (lanes blocked on two leaves become steppable again).
-// `parkedDir` (optional): where this lane parked {d.xyz, time} of its ray (shared memory).  The node phase only needs the origin and
-// the clamped 1/d; with the direction out of the register file during that phase the 56-register traversal kernels keep 1/d in
-// registers instead of reloading spilled copies at every node (the leaf phase reads the direction back, one LDS.128 per leaf).
 template<bool ANY_HIT, bool STATS>
 RT_DEV void trav_run(const RtSceneView& S, const RtRay& r, float tMin, RtStack stack, RtTrav& ts, bool& alive,
-                     uint32_t keepGoing, uint32_t walkThreshold, RtTravStats& st, const float4* parkedDir = nullptr,
+                     uint32_t keepGoing, uint32_t walkThreshold, RtTravStats& st,
                      float4* hitRecords = nullptr, uint32_t hitSlot = 0u)
 {
 	for (;;)
@@ -605,16 +556,7 @@ RT_DEV void trav_run(const RtSceneView& S, const RtRay& r, float tMin, RtStack s
 		if (STATS) { st.leafIters++; st.leafBusy += (alive && ts.leaf != RT_REF_DONE) ? 1u : 0u; }
 		if (alive && ts.leaf != RT_REF_DONE)
 		{
-			bool done;
-			if (parkedDir)
-			{
-				RtRay full;
-				const float4 dv = *parkedDir;
-				full.o = r.o; full.idc = r.idc; full.d = v3(dv.x, dv.y, dv.z); full.time = dv.w;
-				done = trav_pending_leaf<ANY_HIT, STATS>(S, full, tMin, ts, st, hitRecords, hitSlot);
-			}
-			else done = trav_pending_leaf<ANY_HIT, STATS>(S, r, tMin, ts, st, hitRecords, hitSlot);
-			if (done) alive = false;
+			if (trav_pending_leaf<ANY_HIT, STATS>(S, r, tMin, ts, st, hitRecords, hitSlot)) alive = false;
 			else if (trav_finished(ts)) alive = false;
 		}
 		if ((uint32_t)__popc(__ballot_sync(0xFFFFFFFFu, alive)) < keepGoing) return;
