@@ -58,8 +58,21 @@ namespace
 	std::map<int, RtRenderContext*> g_contexts;                      // per device
 	std::map<std::pair<const Scene*, int>, SceneEntry> g_scenes;     // (scene, device)
 	std::map<const Scene*, std::shared_ptr<RtFlatScene>> g_prebuilt; // scenes that came from RaylibB200_LoadFlattenedScene
+
+	// Device buffers a call needs only while it runs, kept per (device, slot) and grown on demand.  Calls run one at a time
+	// under g_mutex, so calls that name the same slot share its buffer; slots a call uses together are distinct.
+	enum class ScratchSlot
+	{
+		Shard = 0,             // Render: a device's tile-major shard (gather fall-back); RenderAux: the albedo shard
+		Image = 1,             // a W x H float4 image: Render (into a host image), RenderAux, PostProcessHostImage, AccumulatorResolve
+		AuxShard = 2,          // RenderAux: the normal shard
+		Gather = 3,            // Render: every device's shard, copied to the primary (gather fall-back)
+		Noise = 4,             // AccumulatorNoise: the per-pixel noise figures
+		DenoiseScratch = 5,    // Denoise, DenoiseDevice, AccumulatorDenoise: the filter's records (rt_denoise_scratch_bytes)
+		DenoiseImages = 6,     // Denoise, AccumulatorDenoise: device copies of the host images: colour, albedo, normal, output
+	};
 	struct Scratch { void* ptr = nullptr; uint64_t bytes = 0; };
-	std::map<std::pair<int, int>, Scratch> g_scratch;                // (device, slot)
+	std::map<std::pair<int, ScratchSlot>, Scratch> g_scratch;
 	std::map<std::pair<int, int>, bool> g_peerOk;                    // (device, peer) -> device can store into peer's memory
 	std::map<const Image2D*, std::pair<void*, uint64_t>> g_pinnedImages;   // library-created images whose storage is page-locked
 
@@ -115,6 +128,30 @@ namespace
 	thread_local std::string t_lastError;
 	thread_local RaylibB200Stats t_lastStats;
 	thread_local bool t_haveStats = false;
+
+	// The start of every device call: holds g_mutex for the whole call, clears this thread's error, and keeps the start time
+	// of the call's statistics and the prefix of its messages.
+	struct Call
+	{
+		std::lock_guard<std::recursive_mutex> lock{ g_mutex };
+		const std::chrono::steady_clock::time_point start = std::chrono::steady_clock::now();
+		const std::string prefix;
+
+		explicit Call(std::string messagePrefix = "") : prefix(std::move(messagePrefix)) { t_lastError.clear(); }
+		bool Fail(const std::string& why) const { RtGpu::SetLastError(prefix + why); return false; }
+		bool RequireDevice() const
+		{
+			if (rt_device_count() > 0) return true;
+			RtGpu::SetLastError(RtGpu::kNoDevice);
+			return false;
+		}
+		// stats.totalMs is the wall time since the call started
+		void Report(RaylibB200Stats& stats) const
+		{
+			stats.totalMs = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - start).count();
+			RtGpu::SetLastStats(stats);
+		}
+	};
 
 	const char* Env(const char* name) { const char* v = getenv(name); return (v && *v) ? v : nullptr; }
 
@@ -188,7 +225,7 @@ namespace
 		if (g_devices.empty()) for (int d = 0; d < n; ++d) g_devices.push_back(d);
 	}
 
-	void* ScratchBuffer(int device, int slot, uint64_t bytes)
+	void* ScratchBuffer(int device, ScratchSlot slot, uint64_t bytes)
 	{
 		Scratch& s = g_scratch[{device, slot}];
 		if (s.bytes >= bytes && s.ptr) return s.ptr;
@@ -239,6 +276,16 @@ namespace
 		return ok;
 	}
 
+	// Frees every device's copy of `scene`.
+	void DropSceneCopies(const Scene* scene)
+	{
+		for (auto e = g_scenes.begin(); e != g_scenes.end();)
+		{
+			if (e->first.first == scene) { rt_scene_free(e->second.device); e = g_scenes.erase(e); }
+			else ++e;
+		}
+	}
+
 	// The scene's copy on `device`: flattened + uploaded the first time any device needs it, cloned device-to-device
 	// (NVLink peer copy) for every further device -- the host flattens ONCE whatever the number of GPUs.
 	const SceneEntry* SceneOn(const Scene* scene, int device)
@@ -252,24 +299,14 @@ namespace
 			const ImageHandle sky = scene->GetSkyPanorama();
 			if (sky != it->second.skyHandle || SkySignature(sky) != it->second.skySignature)
 			{
-				const bool prebuiltScene = false;
-				(void)prebuiltScene;
-				for (auto e = g_scenes.begin(); e != g_scenes.end();)
-				{
-					if (e->first.first == scene) { rt_scene_free(e->second.device); e = g_scenes.erase(e); }
-					else ++e;
-				}
+				DropSceneCopies(scene);
 				it = g_scenes.end();
 			}
 		}
 		// a statistics frame walks the reference topology, which plain uploads leave on the host: upload again with it
 		if (it != g_scenes.end() && g_collectStats && !it->second.referenceTree)
 		{
-			for (auto e = g_scenes.begin(); e != g_scenes.end();)
-			{
-				if (e->first.first == scene) { rt_scene_free(e->second.device); e = g_scenes.erase(e); }
-				else ++e;
-			}
+			DropSceneCopies(scene);
 			it = g_scenes.end();
 		}
 		if (it != g_scenes.end()) return &it->second;
@@ -315,6 +352,22 @@ namespace
 			(double)flat.HostBytes() / 1.0e6,
 			std::chrono::duration<double, std::milli>(t1 - t0).count(), std::chrono::duration<double, std::milli>(t2 - t1).count());
 		return &g_scenes.emplace(key, entry).first->second;
+	}
+
+	// the sun a frame of `scene` is rendered with: the Scene object's as it is now, or the stored one of a flattened-scene file
+	void FrameSun(const Scene* scene, float illuminance[3], float direction[3])
+	{
+		const auto pre = g_prebuilt.find(scene);
+		if (pre != g_prebuilt.end())
+		{
+			memcpy(illuminance, pre->second->desc.sunIlluminance, 12);
+			memcpy(direction, pre->second->desc.sunDirection, 12);
+			return;
+		}
+		vec3 i, d;
+		scene->GetSun(i, d);
+		illuminance[0] = i.x; illuminance[1] = i.y; illuminance[2] = i.z;
+		direction[0] = d.x; direction[1] = d.y; direction[2] = d.z;
 	}
 
 	void AddStats(RaylibB200Stats& st, const RtRenderStats& rs)
@@ -400,26 +453,11 @@ namespace RtGpu
 		return true;
 	}
 
-	RtRenderContext* AcquireContext()
-	{
-		std::lock_guard<std::recursive_mutex> lock(g_mutex);
-		if (DeviceCount() <= 0)
-		{
-			SetLastError("no CUDA device is available; this library renders on the GPU only (no CPU path)");
-			return nullptr;
-		}
-		return ContextOn(CurrentDevice());
-	}
-
 	const RtDeviceScene* AcquireScene(const Scene* scene, uint64_t* outCounts8)
 	{
 		std::lock_guard<std::recursive_mutex> lock(g_mutex);
 		if (!scene) { SetLastError("null scene handle"); return nullptr; }
-		if (DeviceCount() <= 0)
-		{
-			SetLastError("no CUDA device is available; this library renders on the GPU only (no CPU path)");
-			return nullptr;
-		}
+		if (DeviceCount() <= 0) { SetLastError(kNoDevice); return nullptr; }
 		const SceneEntry* entry = SceneOn(scene, CurrentDevice());
 		if (!entry) return nullptr;
 		if (outCounts8) memcpy(outCounts8, entry->counts, sizeof(entry->counts));
@@ -472,22 +510,17 @@ namespace RtGpu
 		}
 	}
 
-	bool Render(const RendererSettings* settings, const Scene* scene, const Camera* camera,
-	            Image2D* hostImage, void* deviceImage, void* deviceShard,
-	            uint32_t shardRank, uint32_t shardCount, uint32_t renderModeOverride, void* stream, bool pinHostImage,
-	            const SampleWindow* window)
+	bool Render(const RendererSettings* settings, const Scene* scene, const Camera* camera, FrameTarget target,
+	            uint32_t renderModeOverride)
 	{
-		std::lock_guard<std::recursive_mutex> lock(g_mutex);
-		const auto wall0 = std::chrono::steady_clock::now();
-		t_lastError.clear();
-		if (!settings || !scene || !camera) { SetLastError("Raylib_Render: null settings/scene/camera"); return false; }
-		if (settings->viewportWidth == 0 || settings->viewportHeight == 0) { SetLastError("Raylib_Render: empty viewport"); return false; }
-		if (settings->renderMode >= RAYLIB_RENDERMODE_MAX && renderModeOverride == 0) { SetLastError("Raylib_Render: invalid renderMode"); return false; }
-		if (DeviceCount() <= 0)
-		{
-			SetLastError("no CUDA device is available; this library renders on the GPU only (no CPU path)");
-			return false;
-		}
+		const Call call("Raylib_Render: ");
+		if (!settings || !scene || !camera) return call.Fail("null settings/scene/camera");
+		if (settings->viewportWidth == 0 || settings->viewportHeight == 0) return call.Fail("empty viewport");
+		if (settings->renderMode >= RAYLIB_RENDERMODE_MAX && renderModeOverride == 0) return call.Fail("invalid renderMode");
+		const int destinations = (target.hostImage != nullptr) + (target.deviceImage != nullptr) + (target.deviceShard != nullptr) +
+		                         (target.window != nullptr);
+		if (destinations != 1) return call.Fail("a frame needs exactly one destination");
+		if (!call.RequireDevice()) return false;
 		ResolveDevices();
 		const int primary = CurrentDevice();
 
@@ -512,33 +545,30 @@ namespace RtGpu
 		if (g_prebuilt.find(scene) == g_prebuilt.end())
 		{
 			// the sun as the Scene object holds it NOW (the reference reads it on every miss, renderer.cc:160-191)
-			vec3 illuminance, direction;
-			scene->GetSun(illuminance, direction);
 			params.lightingOverride = 1;
-			params.sunIlluminance[0] = illuminance.x; params.sunIlluminance[1] = illuminance.y; params.sunIlluminance[2] = illuminance.z;
-			params.sunDirection[0] = direction.x; params.sunDirection[1] = direction.y; params.sunDirection[2] = direction.z;
+			FrameSun(scene, params.sunIlluminance, params.sunDirection);
 		}
 
 		// ---- which devices render this frame -------------------------------------------------------------
 		// A whole frame (read back into a host image, or left in a row-major device image on the primary device) is spread over the
 		// active devices by interleaved 16x16 tiles (SURVEY 8e); shards, debug views and statistics frames stay on the primary device.
-		const uint64_t samples = window ? (uint64_t)(window->end - window->begin) : (uint64_t)std::max(1, params.samplesPerPixel);
+		const uint64_t samples = target.window ? (uint64_t)(target.window->end - target.window->begin) : (uint64_t)std::max(1, params.samplesPerPixel);
 		const uint64_t pixelSamples = (uint64_t)params.width * params.height * samples;
 		std::vector<int> devices(1, primary);
-		const bool wholeFrame = window || hostImage || (deviceImage && !deviceShard && shardCount <= 1);
+		const bool wholeFrame = target.window || target.hostImage || (target.deviceImage && target.shardCount <= 1);
 		if (wholeFrame && params.renderMode == 0u && !g_collectStats && !g_timeStages && g_devices.size() > 1 &&
 		    pixelSamples >= g_multiDeviceMinSamples)
 			devices = g_devices;
 		// the running sums of an installment live on the primary device: a device that cannot address them sits it out
-		if (window && devices.size() > 1)
+		if (target.window && devices.size() > 1)
 			for (size_t i = 1; i < devices.size(); ++i)
 				if (!PeerOk(devices[i], primary)) { devices.assign(1, primary); break; }
 		const uint32_t n = (uint32_t)devices.size();
 
 		// hostImage: always the whole frame; deviceShard / deviceImage: the tiles of (shardRank, shardCount)
-		if (hostImage) { shardRank = 0; shardCount = 1; }
-		if (shardCount == 0) shardCount = 1;
-		if (shardRank >= shardCount) { SetLastError("Raylib_Render: shardRank >= shardCount"); return false; }
+		if (target.hostImage) { target.shardRank = 0; target.shardCount = 1; }
+		if (target.shardCount == 0) target.shardCount = 1;
+		if (target.shardRank >= target.shardCount) return call.Fail("shardRank >= shardCount");
 
 		struct PerDevice
 		{
@@ -571,9 +601,9 @@ namespace RtGpu
 		void* imageBuffer = nullptr;
 		bool direct = true;
 		for (uint32_t i = 1; i < n; ++i) direct = direct && PeerOk(work[i].device, primary);
-		if (!deviceShard)
+		if (!target.deviceShard)
 		{
-			imageBuffer = window ? window->sums : deviceImage ? deviceImage : ScratchBuffer(primary, 1, imageBytes);
+			imageBuffer = target.window ? target.window->sums : target.deviceImage ? target.deviceImage : ScratchBuffer(primary, ScratchSlot::Image, imageBytes);
 			if (!imageBuffer) { SetLastError(std::string("device allocation failed: ") + rt_last_error()); return false; }
 		}
 		const uint64_t shardBytes = (uint64_t)rt_shard_tile_capacity(params.width, params.height, n) * RT_TILE_PIXELS * 16ull;
@@ -581,20 +611,20 @@ namespace RtGpu
 		{
 			PerDevice& w = work[i];
 			w.params = params;
-			w.params.shardRank = n > 1 ? i : shardRank;
-			w.params.shardCount = n > 1 ? n : shardCount;
-			if (deviceShard) w.shard = deviceShard;
+			w.params.shardRank = n > 1 ? i : target.shardRank;
+			w.params.shardCount = n > 1 ? n : target.shardCount;
+			if (target.deviceShard) w.shard = target.deviceShard;
 			else if (direct) w.params.imageOut = imageBuffer;
 			else
 			{
-				w.shard = ScratchBuffer(w.device, 0, shardBytes);
+				w.shard = ScratchBuffer(w.device, ScratchSlot::Shard, shardBytes);
 				if (!w.shard) { SetLastError(std::string("device allocation failed: ") + rt_last_error()); return false; }
 			}
 		}
 
 		// one host thread per device issues that device's launches (about ten thousand per 4K frame) and waits for it;
 		// they share nothing but the read-only camera block
-		auto renderOn = [&cam, window](PerDevice& w, void* onStream)
+		auto renderOn = [&cam, window = target.window](PerDevice& w, void* onStream)
 		{
 			w.rc = window ? rt_render_window(w.ctx, w.scene, &cam, &w.params, window->begin, window->end, window->sums, w.shard, onStream, &w.stats)
 			              : rt_render_shard(w.ctx, w.scene, &cam, &w.params, w.shard, onStream, &w.stats);
@@ -610,7 +640,7 @@ namespace RtGpu
 				worker->Submit([renderOn, w]() { renderOn(*w, nullptr); });
 				helpers.push_back(worker.get());
 			}
-			renderOn(work[0], n > 1 ? nullptr : stream);
+			renderOn(work[0], n > 1 ? nullptr : target.stream);
 			for (DeviceWorker* h : helpers) h->Wait();
 		}
 		for (const PerDevice& w : work)
@@ -618,7 +648,7 @@ namespace RtGpu
 
 		if (n > 1 && !direct)
 		{
-			void* gathered = ScratchBuffer(primary, 3, shardBytes * n);
+			void* gathered = ScratchBuffer(primary, ScratchSlot::Gather, shardBytes * n);
 			if (!gathered) { SetLastError(std::string("device allocation failed: ") + rt_last_error()); return false; }
 			for (uint32_t i = 0; i < n; ++i)
 				if (rt_copy_peer(primary, (char*)gathered + shardBytes * i, work[i].device, work[i].shard, shardBytes) != 0)
@@ -634,11 +664,11 @@ namespace RtGpu
 		}
 
 		uint64_t d2h = 0;
-		if (hostImage)
+		if (target.hostImage)
 		{
-			if (pinHostImage) PinHostImage(hostImage, imageBytes);
+			if (target.pinHostImage) PinHostImage(target.hostImage, imageBytes);
 			// Pixel is four packed floats, same as the device float4 image
-			if (rt_copy_to_host(primary, hostImage->MutablePixels(), imageBuffer, imageBytes, n > 1 ? nullptr : stream) != 0)
+			if (rt_copy_to_host(primary, target.hostImage->MutablePixels(), imageBuffer, imageBytes, n > 1 ? nullptr : target.stream) != 0)
 			{
 				SetLastError(std::string("device -> host copy failed: ") + rt_last_error());
 				return false;
@@ -649,12 +679,11 @@ namespace RtGpu
 		RaylibB200Stats st;
 		memset(&st, 0, sizeof(st));
 		for (const PerDevice& w : work) AddStats(st, w.stats);
-		st.totalMs = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - wall0).count();
 		st.h2dBytes = (sizeof(RtCamera) + sizeof(RtRenderParams)) * n;
 		st.d2hBytes = d2h;
 		st.device = (uint32_t)primary;
 		st.devicesUsed = n;
-		SetLastStats(st);
+		call.Report(st);
 		return true;
 	}
 }
@@ -663,14 +692,11 @@ namespace RtGpu
 {
 	bool RenderAux(const RendererSettings* settings, const Scene* scene, const Camera* camera, Image2D* albedoImage, Image2D* normalImage)
 	{
-		std::lock_guard<std::recursive_mutex> lock(g_mutex);
-		const auto wall0 = std::chrono::steady_clock::now();
-		t_lastError.clear();
-		if (!settings || !scene || !camera || !albedoImage || !normalImage) { SetLastError("RaylibB200_RenderAux: null argument"); return false; }
-		if (settings->viewportWidth == 0 || settings->viewportHeight == 0) { SetLastError("RaylibB200_RenderAux: empty viewport"); return false; }
+		const Call call("RaylibB200_RenderAux: ");
+		if (!settings || !scene || !camera || !albedoImage || !normalImage) return call.Fail("null argument");
+		if (settings->viewportWidth == 0 || settings->viewportHeight == 0) return call.Fail("empty viewport");
 		const RtDeviceScene* deviceScene = AcquireScene(scene);
-		if (!deviceScene) return false;
-		RtRenderContext* ctx = AcquireContext();
+		RtRenderContext* ctx = deviceScene ? ContextOn(CurrentDevice()) : nullptr;
 		if (!ctx) return false;
 		const int device = CurrentDevice();
 		const uint32_t W = settings->viewportWidth, H = settings->viewportHeight;
@@ -681,9 +707,9 @@ namespace RtGpu
 		RtFlattenCamera(camera, cam);
 		const uint64_t shardBytes = (uint64_t)rt_shard_tile_capacity(W, H, 1) * RT_TILE_PIXELS * 16ull;
 		const uint64_t imageBytes = (uint64_t)W * H * 16ull;
-		void* shardA = ScratchBuffer(device, 0, shardBytes);
-		void* shardB = ScratchBuffer(device, 2, shardBytes);
-		void* image = ScratchBuffer(device, 1, imageBytes);
+		void* shardA = ScratchBuffer(device, ScratchSlot::Shard, shardBytes);
+		void* shardB = ScratchBuffer(device, ScratchSlot::AuxShard, shardBytes);
+		void* image = ScratchBuffer(device, ScratchSlot::Image, imageBytes);
 		if (!shardA || !shardB || !image) { SetLastError(std::string("device allocation failed: ") + rt_last_error()); return false; }
 
 		RtRenderParams params;
@@ -714,36 +740,31 @@ namespace RtGpu
 		}
 		RaylibB200Stats st;
 		memset(&st, 0, sizeof(st));
-		st.rayQueries = rs.rayQueries; st.pixelSamples = rs.pixelSamples; st.deviceMs = rs.deviceMs;
-		st.totalMs = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - wall0).count();
+		AddStats(st, rs);
+		st.kernelLaunches += 2;      // the read-backs' k_assemble
 		st.h2dBytes = sizeof(RtCamera) + sizeof(RtRenderParams); st.d2hBytes = 2 * imageBytes;
-		st.kernelLaunches = rs.kernelLaunches + 2; st.device = (uint32_t)device;
-		SetLastStats(st);
+		st.device = (uint32_t)device;
+		call.Report(st);
 		return true;
 	}
 
 	bool PostProcessDevice(void* deviceImage, uint32_t width, uint32_t height, void* deviceOutArgb8, float* outMaxWhite, void* stream)
 	{
-		std::lock_guard<std::recursive_mutex> lock(g_mutex);
-		t_lastError.clear();
-		if (DeviceCount() <= 0) { SetLastError("no CUDA device is available; this library renders on the GPU only (no CPU path)"); return false; }
+		const Call call;
+		if (!call.RequireDevice()) return false;
 		if (rt_postprocess(CurrentDevice(), deviceImage, width, height, (uint32_t*)deviceOutArgb8, outMaxWhite, stream) != 0)
-		{
-			SetLastError(std::string("rt_postprocess: ") + rt_last_error());
-			return false;
-		}
+			return call.Fail(std::string("rt_postprocess: ") + rt_last_error());
 		return rt_stream_sync(CurrentDevice(), stream) == 0;
 	}
 
 	bool PostProcessHostImage(Image2D* hostImage)
 	{
-		std::lock_guard<std::recursive_mutex> lock(g_mutex);
-		t_lastError.clear();
-		if (!hostImage || hostImage->GetWidth() == 0 || hostImage->GetHeight() == 0) { SetLastError("RaylibB200_PostProcessGPU: empty image"); return false; }
-		if (DeviceCount() <= 0) { SetLastError("no CUDA device is available; this library renders on the GPU only (no CPU path)"); return false; }
+		const Call call("RaylibB200_PostProcessGPU: ");
+		if (!hostImage || hostImage->GetWidth() == 0 || hostImage->GetHeight() == 0) return call.Fail("empty image");
+		if (!call.RequireDevice()) return false;
 		const int device = CurrentDevice();
 		const uint64_t bytes = (uint64_t)hostImage->GetWidth() * hostImage->GetHeight() * 16ull;
-		void* image = ScratchBuffer(device, 1, bytes);
+		void* image = ScratchBuffer(device, ScratchSlot::Image, bytes);
 		if (!image) { SetLastError(std::string("device allocation failed: ") + rt_last_error()); return false; }
 		float maxWhite = 1.0f;
 		if (rt_copy_to_device(device, image, hostImage->MutablePixels(), bytes, nullptr) != 0 ||
@@ -763,9 +784,6 @@ namespace RtGpu
 
 namespace
 {
-	const int kDenoiseScratchSlot = 5;      // the filter's records (rt_denoise_scratch_bytes)
-	const int kDenoiseImageSlot = 6;        // device copies of a host call's images: colour, albedo, normal, output
-
 	// "" or why a guide image cannot go with a W x H colour image
 	std::string GuideSizeError(const Image2D* guide, const char* name, uint32_t width, uint32_t height, const char* against)
 	{
@@ -776,21 +794,17 @@ namespace
 
 	// Uploads the non-null host images of `images` into consecutive W x H float4 images of the slot buffer (which also
 	// holds the output, returned in *out); NULL stays NULL.
-	bool UploadDenoiseImages(const std::string& fn, int device, const Image2D* const images[3], uint64_t bytes, void* dev[3],
+	bool UploadDenoiseImages(const Call& call, int device, const Image2D* const images[3], uint64_t bytes, void* dev[3],
 	                         void** out, RaylibB200Stats& st)
 	{
-		char* base = (char*)ScratchBuffer(device, kDenoiseImageSlot, 4 * bytes);
-		if (!base) { RtGpu::SetLastError(fn + "device allocation failed: " + rt_last_error()); return false; }
+		char* base = (char*)ScratchBuffer(device, ScratchSlot::DenoiseImages, 4 * bytes);
+		if (!base) return call.Fail(std::string("device allocation failed: ") + rt_last_error());
 		for (int k = 0; k < 3; ++k)
 		{
 			dev[k] = nullptr;
 			if (!images[k]) continue;
 			dev[k] = base + k * bytes;
-			if (rt_copy_to_device(device, dev[k], images[k]->GetPixelArray().data(), bytes, nullptr) != 0)
-			{
-				RtGpu::SetLastError(fn + rt_last_error());
-				return false;
-			}
+			if (rt_copy_to_device(device, dev[k], images[k]->GetPixelArray().data(), bytes, nullptr) != 0) return call.Fail(rt_last_error());
 			st.h2dBytes += bytes;
 		}
 		*out = base + 3 * bytes;
@@ -798,14 +812,14 @@ namespace
 	}
 
 	// rt_denoise (n == 0) or rt_denoise_sums on device images of `device`; fills the device part of the statistics
-	bool RunDenoise(const std::string& fn, int device, const void* color, uint32_t n, const void* albedo, const void* normal,
+	bool RunDenoise(const Call& call, int device, const void* color, uint32_t n, const void* albedo, const void* normal,
 	                uint32_t width, uint32_t height, void* out, void* stream, RaylibB200Stats& st)
 	{
-		void* scratch = ScratchBuffer(device, kDenoiseScratchSlot, rt_denoise_scratch_bytes(width, height));
-		if (!scratch) { RtGpu::SetLastError(fn + "device allocation failed: " + rt_last_error()); return false; }
+		void* scratch = ScratchBuffer(device, ScratchSlot::DenoiseScratch, rt_denoise_scratch_bytes(width, height));
+		if (!scratch) return call.Fail(std::string("device allocation failed: ") + rt_last_error());
 		const int rc = n ? rt_denoise_sums(device, color, n, albedo, normal, width, height, scratch, out, stream, &st.deviceMs)
 		                 : rt_denoise(device, color, albedo, normal, width, height, scratch, out, stream, &st.deviceMs);
-		if (rc != 0) { RtGpu::SetLastError(fn + rt_denoise_last_error()); return false; }
+		if (rc != 0) return call.Fail(rt_denoise_last_error());
 		st.kernelLaunches = RT_DENOISE_LAUNCHES;
 		st.device = (uint32_t)device;
 		st.devicesUsed = 1;
@@ -813,18 +827,13 @@ namespace
 	}
 
 	// The result of a host call: read back into `out`, resized to W x H only now that the filter has run
-	bool ReadDenoised(const std::string& fn, int device, const void* image, uint32_t width, uint32_t height, Image2D* out, RaylibB200Stats& st)
+	bool ReadDenoised(const Call& call, int device, const void* image, uint32_t width, uint32_t height, Image2D* out, RaylibB200Stats& st)
 	{
 		if (out->GetWidth() != width || out->GetHeight() != height) out->Reallocate(width, height);
 		const uint64_t bytes = (uint64_t)width * height * 16ull;
-		if (rt_copy_to_host(device, out->MutablePixels(), image, bytes, nullptr) != 0) { RtGpu::SetLastError(fn + rt_last_error()); return false; }
+		if (rt_copy_to_host(device, out->MutablePixels(), image, bytes, nullptr) != 0) return call.Fail(rt_last_error());
 		st.d2hBytes += bytes;
 		return true;
-	}
-
-	double MsSince(std::chrono::steady_clock::time_point t0)
-	{
-		return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
 	}
 }
 
@@ -832,107 +841,108 @@ namespace RtGpu
 {
 	bool Denoise(const Image2D* color, const Image2D* albedo, const Image2D* normal, Image2D* out)
 	{
-		std::lock_guard<std::recursive_mutex> lock(g_mutex);
-		const auto wall0 = std::chrono::steady_clock::now();
-		t_lastError.clear();
-		const std::string fn = "RaylibB200_Denoise: ";
-		if (!color || !out) { SetLastError(fn + "null main or output image"); return false; }
+		const Call call("RaylibB200_Denoise: ");
+		if (!color || !out) return call.Fail("null main or output image");
 		const uint32_t W = color->GetWidth(), H = color->GetHeight();
-		if (W == 0 || H == 0 || (uint64_t)W * H >= (1ull << 31)) { SetLastError(fn + "the main image must be non-empty and below 2^31 pixels"); return false; }
+		if (W == 0 || H == 0 || (uint64_t)W * H >= (1ull << 31)) return call.Fail("the main image must be non-empty and below 2^31 pixels");
 		for (const std::string& why : { GuideSizeError(albedo, "albedo", W, H, "the main image"), GuideSizeError(normal, "normal", W, H, "the main image") })
-			if (!why.empty()) { SetLastError(fn + why); return false; }
-		if (DeviceCount() <= 0) { SetLastError("no CUDA device is available; this library renders on the GPU only (no CPU path)"); return false; }
+			if (!why.empty()) return call.Fail(why);
+		if (!call.RequireDevice()) return false;
 		const int device = CurrentDevice();
 		RaylibB200Stats st;
 		memset(&st, 0, sizeof(st));
 		const Image2D* images[3] = { color, albedo, normal };
 		void* dev[3];
 		void* image = nullptr;
-		if (!UploadDenoiseImages(fn, device, images, (uint64_t)W * H * 16ull, dev, &image, st) ||
-		    !RunDenoise(fn, device, dev[0], 0, dev[1], dev[2], W, H, image, nullptr, st) ||
-		    !ReadDenoised(fn, device, image, W, H, out, st))
+		if (!UploadDenoiseImages(call, device, images, (uint64_t)W * H * 16ull, dev, &image, st) ||
+		    !RunDenoise(call, device, dev[0], 0, dev[1], dev[2], W, H, image, nullptr, st) ||
+		    !ReadDenoised(call, device, image, W, H, out, st))
 			return false;
-		st.totalMs = MsSince(wall0);
-		SetLastStats(st);
+		call.Report(st);
 		return true;
 	}
 
 	bool DenoiseDevice(const void* color, const void* albedo, const void* normal, uint32_t width, uint32_t height, void* out, void* stream)
 	{
-		std::lock_guard<std::recursive_mutex> lock(g_mutex);
-		const auto wall0 = std::chrono::steady_clock::now();
-		t_lastError.clear();
-		const std::string fn = "RaylibB200_DenoiseDevice: ";
-		if (!color || !out) { SetLastError(fn + "null colour or output image"); return false; }
-		if (width == 0 || height == 0 || (uint64_t)width * height >= (1ull << 31)) { SetLastError(fn + "the image must be non-empty and below 2^31 pixels"); return false; }
+		const Call call("RaylibB200_DenoiseDevice: ");
+		if (!color || !out) return call.Fail("null colour or output image");
+		if (width == 0 || height == 0 || (uint64_t)width * height >= (1ull << 31)) return call.Fail("the image must be non-empty and below 2^31 pixels");
 		// the kernels read and write whole float4 pixels: a misaligned view (a sliced tensor) is refused here, not faulted on
 		for (const void* p : { color, albedo, normal, (const void*)out })
-			if ((uintptr_t)p % 16u != 0) { SetLastError(fn + "device images must be 16-byte aligned (RGBA float4 pixels)"); return false; }
-		if (DeviceCount() <= 0) { SetLastError("no CUDA device is available; this library renders on the GPU only (no CPU path)"); return false; }
+			if ((uintptr_t)p % 16u != 0) return call.Fail("device images must be 16-byte aligned (RGBA float4 pixels)");
+		if (!call.RequireDevice()) return false;
 		RaylibB200Stats st;
 		memset(&st, 0, sizeof(st));
-		if (!RunDenoise(fn, CurrentDevice(), color, 0, albedo, normal, width, height, out, stream, st)) return false;
-		st.totalMs = MsSince(wall0);
-		SetLastStats(st);
+		if (!RunDenoise(call, CurrentDevice(), color, 0, albedo, normal, width, height, out, stream, st)) return false;
+		call.Report(st);
 		return true;
 	}
 }
 
 // ---------------------------------------------------------------------------------------------
-// The traversal stage kernels on caller rays (RaylibB200_TraceRaysStaged, rt_trace_stage of rt_trace_stage.h)
+// Ray queries on caller rays: one closest-hit ray per thread (RaylibB200_TraceRays, rt_trace_closest) and the traversal stage
+// kernels of a render (RaylibB200_TraceRaysStaged, rt_trace_stage of rt_trace_stage.h).  Both use the current device's
+// render context, so both run under the state lock like a render does.
 
 namespace RtGpu
 {
+	bool TraceRays(const Scene* scene, const float* rays, int64_t numRays, float tMin, int32_t* outRank, float* outT)
+	{
+		const Call call;
+		const RtDeviceScene* ds = AcquireScene(scene);
+		RtRenderContext* ctx = ds ? ContextOn(CurrentDevice()) : nullptr;
+		if (!ctx) return false;
+		RtRenderStats rs;
+		memset(&rs, 0, sizeof(rs));      // rt_trace_closest leaves it untouched when there are no rays
+		if (rt_trace_closest(ctx, ds, rays, numRays, tMin, outRank, outT, &rs) != 0) return call.Fail(std::string("rt_trace_closest: ") + rt_last_error());
+		RaylibB200Stats st;
+		memset(&st, 0, sizeof(st));
+		AddStats(st, rs);
+		call.Report(st);
+		return true;
+	}
+
 	bool TraceRaysStaged(const Scene* scene, int mode, const float* rays, const uint32_t* order, int64_t numRays, float tMin,
 	                     const float* sunDirection, const RtStageSchedule& schedule, int32_t* outQueue, float* outHit,
 	                     uint32_t* outQueueCounts)
 	{
-		const auto wall0 = std::chrono::steady_clock::now();
-		t_lastError.clear();
-		const std::string fn = "RaylibB200_TraceRaysStaged: ";
-		if (!scene) { SetLastError(fn + "null scene"); return false; }
-		if (!rays || !order || !outQueue || !outHit) { SetLastError(fn + "null ray, order or output buffer"); return false; }
-		if (mode < RT_STAGE_EXTEND || mode > RT_STAGE_SHADOW) { SetLastError(fn + "unknown mode " + std::to_string(mode) + " (0..3)"); return false; }
-		if (numRays <= 0 || numRays >= ((int64_t)1 << 31)) { SetLastError(fn + "the ray count must be in [1, 2^31)"); return false; }
+		const Call call("RaylibB200_TraceRaysStaged: ");
+		if (!scene) return call.Fail("null scene");
+		if (!rays || !order || !outQueue || !outHit) return call.Fail("null ray, order or output buffer");
+		if (mode < RT_STAGE_EXTEND || mode > RT_STAGE_SHADOW) return call.Fail("unknown mode " + std::to_string(mode) + " (0..3)");
+		if (numRays <= 0 || numRays >= ((int64_t)1 << 31)) return call.Fail("the ray count must be in [1, 2^31)");
 		if (mode == RT_STAGE_SHADOW)
 		{
-			if (!sunDirection) { SetLastError(fn + "the any-hit mode needs a sun direction"); return false; }
+			if (!sunDirection) return call.Fail("the any-hit mode needs a sun direction");
 			bool finite = true, zero = true;
 			for (int i = 0; i < 3; ++i) { finite = finite && std::isfinite(sunDirection[i]); zero = zero && sunDirection[i] == 0.0f; }
-			if (!finite || zero) { SetLastError(fn + "the sun direction must be finite and non-zero"); return false; }
+			if (!finite || zero) return call.Fail("the sun direction must be finite and non-zero");
 		}
 		if (schedule.refillThreshold > 32u || schedule.walkThreshold > 32u || schedule.poolNodeThreshold > 32u ||
 		    schedule.poolRefill > 64u || schedule.gridCtas > 4096u)
-		{
-			SetLastError(fn + "scheduling out of range (refill, walk, pool node: 0..32; pool refill: 0..64; grid: 0..4096 CTAs)");
-			return false;
-		}
+			return call.Fail("scheduling out of range (refill, walk, pool node: 0..32; pool refill: 0..64; grid: 0..4096 CTAs)");
 		{
 			std::vector<uint8_t> seen((size_t)numRays, 0);
 			for (int64_t i = 0; i < numRays; ++i)
 			{
-				if ((int64_t)order[i] >= numRays || seen[order[i]]) { SetLastError(fn + "the order is not a permutation of 0..numRays-1"); return false; }
+				if ((int64_t)order[i] >= numRays || seen[order[i]]) return call.Fail("the order is not a permutation of 0..numRays-1");
 				seen[order[i]] = 1;
 			}
 		}
 		const RtDeviceScene* ds = AcquireScene(scene);
-		RtRenderContext* ctx = ds ? AcquireContext() : nullptr;
-		if (!ds || !ctx) return false;
+		RtRenderContext* ctx = ds ? ContextOn(CurrentDevice()) : nullptr;
+		if (!ctx) return false;
 		RtRenderStats rs;
 		if (rt_trace_stage(ctx, ds, mode, rays, order, numRays, tMin, sunDirection, &schedule, outQueue, outHit, outQueueCounts, &rs) != 0)
-		{
-			SetLastError(fn + rt_last_error());
-			return false;
-		}
+			return call.Fail(rt_last_error());
 		RaylibB200Stats st;
 		memset(&st, 0, sizeof(st));
 		AddStats(st, rs);
-		st.totalMs = MsSince(wall0);
 		st.device = (uint32_t)CurrentDevice();
 		st.devicesUsed = 1;
 		st.h2dBytes = (uint64_t)numRays * 36u;                                   // rays + order
 		st.d2hBytes = (uint64_t)numRays * (mode == RT_STAGE_SHADOW ? 16u : 36u);   // records or radiance (+ queues)
-		SetLastStats(st);
+		call.Report(st);
 		return true;
 	}
 }
@@ -982,7 +992,6 @@ struct RaylibB200Accumulator
 namespace
 {
 	const uint32_t kMaxAccumSamples = 1u << 24;       // every count up to here is exact as the float divisor
-	const char* kNoDevice = "no CUDA device is available; this library renders on the GPU only (no CPU path)";
 
 	struct AccumFileHeader
 	{
@@ -1005,22 +1014,6 @@ namespace
 		sum.Add(&b, sizeof(b));
 		sum.Add(sums, (size_t)sumBytes);
 		return sum.h;
-	}
-
-	// the sun a frame of `scene` is rendered with: the Scene object's as it is now, or the stored one of a flattened-scene file
-	void FrameSun(const Scene* scene, float illuminance[3], float direction[3])
-	{
-		const auto pre = g_prebuilt.find(scene);
-		if (pre != g_prebuilt.end())
-		{
-			memcpy(illuminance, pre->second->desc.sunIlluminance, 12);
-			memcpy(direction, pre->second->desc.sunDirection, 12);
-			return;
-		}
-		vec3 i, d;
-		scene->GetSun(i, d);
-		illuminance[0] = i.x; illuminance[1] = i.y; illuminance[2] = i.z;
-		direction[0] = d.x; direction[1] = d.y; direction[2] = d.z;
 	}
 
 	bool SceneFingerprint(const Scene* scene, int device, uint64_t* out)
@@ -1055,9 +1048,9 @@ namespace
 		return fields;
 	}
 
-	RaylibB200Accumulator* NewAccumulator(uint32_t width, uint32_t height, const char* fn)
+	RaylibB200Accumulator* NewAccumulator(const Call& call, uint32_t width, uint32_t height)
 	{
-		if (rt_device_count() <= 0) { RtGpu::SetLastError(kNoDevice); return nullptr; }
+		if (!call.RequireDevice()) return nullptr;
 		ResolveDevices();
 		std::unique_ptr<RaylibB200Accumulator> acc(new RaylibB200Accumulator);
 		memset(&acc->binding, 0, sizeof(acc->binding));
@@ -1066,7 +1059,7 @@ namespace
 		const uint64_t bytes = (uint64_t)width * height * 16ull;
 		if (rt_device_alloc(acc->device, bytes, &acc->sums) != 0 || rt_device_zero(acc->device, acc->sums, bytes) != 0)
 		{
-			RtGpu::SetLastError(std::string(fn) + "device allocation failed: " + rt_last_error());
+			call.Fail(std::string("device allocation failed: ") + rt_last_error());
 			if (acc->sums) rt_device_free(acc->device, acc->sums);
 			return nullptr;
 		}
@@ -1078,14 +1071,13 @@ namespace RtGpu
 {
 	RaylibB200Accumulator* AccumulatorCreate(uint32_t width, uint32_t height)
 	{
-		std::lock_guard<std::recursive_mutex> lock(g_mutex);
-		t_lastError.clear();
+		const Call call("RaylibB200_AccumulatorCreate: ");
 		if (width == 0 || height == 0 || (uint64_t)width * height >= (1ull << 31))
 		{
-			SetLastError("RaylibB200_AccumulatorCreate: size must be non-empty and below 2^31 pixels");
+			call.Fail("size must be non-empty and below 2^31 pixels");
 			return nullptr;
 		}
-		return NewAccumulator(width, height, "RaylibB200_AccumulatorCreate: ");
+		return NewAccumulator(call, width, height);
 	}
 
 	void AccumulatorDestroy(RaylibB200Accumulator* acc)
@@ -1098,14 +1090,9 @@ namespace RtGpu
 
 	bool AccumulatorReset(RaylibB200Accumulator* acc)
 	{
-		std::lock_guard<std::recursive_mutex> lock(g_mutex);
-		t_lastError.clear();
-		if (!acc) { SetLastError("RaylibB200_AccumulatorReset: null accumulator"); return false; }
-		if (rt_device_zero(acc->device, acc->sums, (uint64_t)acc->width * acc->height * 16ull) != 0)
-		{
-			SetLastError(std::string("RaylibB200_AccumulatorReset: ") + rt_last_error());
-			return false;
-		}
+		const Call call("RaylibB200_AccumulatorReset: ");
+		if (!acc) return call.Fail("null accumulator");
+		if (rt_device_zero(acc->device, acc->sums, (uint64_t)acc->width * acc->height * 16ull) != 0) return call.Fail(rt_last_error());
 		acc->samples = 0;
 		acc->bound = false;
 		memset(&acc->binding, 0, sizeof(acc->binding));
@@ -1116,21 +1103,16 @@ namespace RtGpu
 
 	bool RenderAccumulate(const RendererSettings* settings, const Scene* scene, const Camera* camera, RaylibB200Accumulator* acc, uint32_t samples)
 	{
-		std::lock_guard<std::recursive_mutex> lock(g_mutex);
-		t_lastError.clear();
-		const std::string fn = "RaylibB200_RenderAccumulate: ";
-		if (!settings || !scene || !camera || !acc) { SetLastError(fn + "null argument"); return false; }
-		if (samples == 0) { SetLastError(fn + "an installment renders at least one sample"); return false; }
-		if (settings->renderMode != 0u) { SetLastError(fn + "only renderMode 0 (path tracing) accumulates"); return false; }
-		if ((uint64_t)acc->samples + samples > kMaxAccumSamples) { SetLastError(fn + "more than 2^24 samples per pixel"); return false; }
-		if (DeviceCount() <= 0) { SetLastError(kNoDevice); return false; }
+		const Call call("RaylibB200_RenderAccumulate: ");
+		if (!settings || !scene || !camera || !acc) return call.Fail("null argument");
+		if (samples == 0) return call.Fail("an installment renders at least one sample");
+		if (settings->renderMode != 0u) return call.Fail("only renderMode 0 (path tracing) accumulates");
+		if ((uint64_t)acc->samples + samples > kMaxAccumSamples) return call.Fail("more than 2^24 samples per pixel");
+		if (!call.RequireDevice()) return false;
 		ResolveDevices();
 		const int primary = g_devices[0];
 		if (primary != acc->device)
-		{
-			SetLastError(fn + "the accumulator lives on GPU " + std::to_string(acc->device) + ", the first active device is GPU " + std::to_string(primary));
-			return false;
-		}
+			return call.Fail("the accumulator lives on GPU " + std::to_string(acc->device) + ", the first active device is GPU " + std::to_string(primary));
 
 		RtAccumBinding b;
 		memset(&b, 0, sizeof(b));
@@ -1141,25 +1123,21 @@ namespace RtGpu
 		RtFlattenCamera(camera, b.camera);
 		FrameSun(scene, b.sunIlluminance, b.sunDirection);
 		if (b.width != acc->width || b.height != acc->height)
-		{
-			SetLastError(fn + "viewport " + std::to_string(b.width) + "x" + std::to_string(b.height) + " differs from the accumulator's " +
-			             std::to_string(acc->width) + "x" + std::to_string(acc->height));
-			return false;
-		}
+			return call.Fail("viewport " + std::to_string(b.width) + "x" + std::to_string(b.height) + " differs from the accumulator's " +
+			                 std::to_string(acc->width) + "x" + std::to_string(acc->height));
 		if (!SceneFingerprint(scene, primary, &b.sceneFingerprint)) return false;
 		if (acc->bound)
 		{
 			const std::string fields = BindingDifference(acc->binding, b);
 			if (!fields.empty())
-			{
-				SetLastError(fn + "the accumulated image's " + fields + (fields.find(',') == std::string::npos ? " differs" : " differ") +
-				             " from this installment's; Reset the accumulator to start a new image");
-				return false;
-			}
+				return call.Fail("the accumulated image's " + fields + (fields.find(',') == std::string::npos ? " differs" : " differ") +
+				                 " from this installment's; Reset the accumulator to start a new image");
 		}
 
 		const SampleWindow window = { acc->samples, acc->samples + samples, acc->sums };
-		if (!Render(settings, scene, camera, nullptr, nullptr, nullptr, 0, 1, 0, nullptr, false, &window)) return false;
+		FrameTarget target;
+		target.window = &window;
+		if (!Render(settings, scene, camera, target)) return false;
 		acc->binding = b;
 		acc->bound = true;
 		acc->samples += samples;
@@ -1168,101 +1146,78 @@ namespace RtGpu
 
 	bool AccumulatorResolve(RaylibB200Accumulator* acc, Image2D* hostImage, void* deviceImage, void* stream)
 	{
-		std::lock_guard<std::recursive_mutex> lock(g_mutex);
-		t_lastError.clear();
-		const std::string fn = "RaylibB200_AccumulatorResolve: ";
-		if (!acc || (!hostImage && !deviceImage)) { SetLastError(fn + "null argument"); return false; }
-		if (acc->samples == 0) { SetLastError(fn + "the accumulator holds no samples"); return false; }
+		const Call call("RaylibB200_AccumulatorResolve: ");
+		if (!acc || (!hostImage && !deviceImage)) return call.Fail("null argument");
+		if (acc->samples == 0) return call.Fail("the accumulator holds no samples");
 		const uint64_t count = (uint64_t)acc->width * acc->height, bytes = count * 16ull;
 		if (deviceImage)
 		{
 			if (rt_resolve(acc->device, acc->sums, (uint32_t)count, acc->samples, deviceImage, nullptr, nullptr, stream) != 0)
-			{
-				SetLastError(fn + rt_last_error());
-				return false;
-			}
+				return call.Fail(rt_last_error());
 			return true;
 		}
 		if (hostImage->GetWidth() != acc->width || hostImage->GetHeight() != acc->height) hostImage->Reallocate(acc->width, acc->height);
-		void* image = ScratchBuffer(acc->device, 1, bytes);
-		if (!image) { SetLastError(fn + "device allocation failed: " + rt_last_error()); return false; }
+		void* image = ScratchBuffer(acc->device, ScratchSlot::Image, bytes);
+		if (!image) return call.Fail(std::string("device allocation failed: ") + rt_last_error());
 		if (rt_resolve(acc->device, acc->sums, (uint32_t)count, acc->samples, image, nullptr, nullptr, nullptr) != 0 ||
 		    rt_copy_to_host(acc->device, hostImage->MutablePixels(), image, bytes, nullptr) != 0)
-		{
-			SetLastError(fn + rt_last_error());
-			return false;
-		}
+			return call.Fail(rt_last_error());
 		return true;
 	}
 
 	bool AccumulatorDenoise(RaylibB200Accumulator* acc, const Image2D* albedo, const Image2D* normal, Image2D* out)
 	{
-		std::lock_guard<std::recursive_mutex> lock(g_mutex);
-		const auto wall0 = std::chrono::steady_clock::now();
-		t_lastError.clear();
-		const std::string fn = "RaylibB200_AccumulatorDenoise: ";
-		if (!acc || !out) { SetLastError(fn + "null accumulator or output image"); return false; }
-		if (acc->samples < 2) { SetLastError(fn + "the variance needs at least 2 samples per pixel"); return false; }
+		const Call call("RaylibB200_AccumulatorDenoise: ");
+		if (!acc || !out) return call.Fail("null accumulator or output image");
+		if (acc->samples < 2) return call.Fail("the variance needs at least 2 samples per pixel");
 		const uint32_t W = acc->width, H = acc->height;
 		for (const std::string& why : { GuideSizeError(albedo, "albedo", W, H, "the accumulator"), GuideSizeError(normal, "normal", W, H, "the accumulator") })
-			if (!why.empty()) { SetLastError(fn + why); return false; }
+			if (!why.empty()) return call.Fail(why);
 		RaylibB200Stats st;
 		memset(&st, 0, sizeof(st));
 		const Image2D* images[3] = { nullptr, albedo, normal };
 		void* dev[3];
 		void* image = nullptr;
-		if (!UploadDenoiseImages(fn, acc->device, images, (uint64_t)W * H * 16ull, dev, &image, st) ||
-		    !RunDenoise(fn, acc->device, acc->sums, acc->samples, dev[1], dev[2], W, H, image, nullptr, st) ||
-		    !ReadDenoised(fn, acc->device, image, W, H, out, st))
+		if (!UploadDenoiseImages(call, acc->device, images, (uint64_t)W * H * 16ull, dev, &image, st) ||
+		    !RunDenoise(call, acc->device, acc->sums, acc->samples, dev[1], dev[2], W, H, image, nullptr, st) ||
+		    !ReadDenoised(call, acc->device, image, W, H, out, st))
 			return false;
-		st.totalMs = MsSince(wall0);
-		SetLastStats(st);
+		call.Report(st);
 		return true;
 	}
 
 	bool AccumulatorRead(RaylibB200Accumulator* acc, float* rgba)
 	{
-		std::lock_guard<std::recursive_mutex> lock(g_mutex);
-		t_lastError.clear();
-		if (!acc || !rgba) { SetLastError("RaylibB200_AccumulatorRead: null argument"); return false; }
-		if (rt_copy_to_host(acc->device, rgba, acc->sums, (uint64_t)acc->width * acc->height * 16ull, nullptr) != 0)
-		{
-			SetLastError(std::string("RaylibB200_AccumulatorRead: ") + rt_last_error());
-			return false;
-		}
+		const Call call("RaylibB200_AccumulatorRead: ");
+		if (!acc || !rgba) return call.Fail("null argument");
+		if (rt_copy_to_host(acc->device, rgba, acc->sums, (uint64_t)acc->width * acc->height * 16ull, nullptr) != 0) return call.Fail(rt_last_error());
 		return true;
 	}
 
 	bool AccumulatorNoise(RaylibB200Accumulator* acc, float* perPixel, double* mean)
 	{
-		std::lock_guard<std::recursive_mutex> lock(g_mutex);
-		t_lastError.clear();
-		const std::string fn = "RaylibB200_AccumulatorNoise: ";
-		if (!acc) { SetLastError(fn + "null accumulator"); return false; }
-		if (acc->samples < 2) { SetLastError(fn + "the noise figure needs at least 2 samples per pixel"); return false; }
+		const Call call("RaylibB200_AccumulatorNoise: ");
+		if (!acc) return call.Fail("null accumulator");
+		if (acc->samples < 2) return call.Fail("the noise figure needs at least 2 samples per pixel");
 		const uint64_t count = (uint64_t)acc->width * acc->height;
 		float* noise = nullptr;
-		if (perPixel && !(noise = (float*)ScratchBuffer(acc->device, 4, count * 4ull))) { SetLastError(fn + "device allocation failed: " + rt_last_error()); return false; }
+		if (perPixel && !(noise = (float*)ScratchBuffer(acc->device, ScratchSlot::Noise, count * 4ull)))
+			return call.Fail(std::string("device allocation failed: ") + rt_last_error());
 		double total = 0.0;
 		if (rt_resolve(acc->device, acc->sums, (uint32_t)count, acc->samples, nullptr, noise, mean ? &total : nullptr, nullptr) != 0 ||
 		    (perPixel && rt_copy_to_host(acc->device, perPixel, noise, count * 4ull, nullptr) != 0))
-		{
-			SetLastError(fn + rt_last_error());
-			return false;
-		}
+			return call.Fail(rt_last_error());
 		if (mean) *mean = total / (double)count;
 		return true;
 	}
 
 	bool AccumulatorSave(const RaylibB200Accumulator* acc, const char* path)
 	{
-		std::lock_guard<std::recursive_mutex> lock(g_mutex);
-		t_lastError.clear();
-		const std::string fn = "RaylibB200_AccumulatorSave: ";
-		if (!acc || !path || !*path) { SetLastError(fn + "null accumulator or empty path"); return false; }
+		const Call call("RaylibB200_AccumulatorSave: ");
+		if (!acc || !path || !*path) return call.Fail("null accumulator or empty path");
 		const uint64_t sumBytes = (uint64_t)acc->width * acc->height * 16ull;
 		std::vector<float> sums((size_t)(sumBytes / 4));
-		if (rt_copy_to_host(acc->device, sums.data(), acc->sums, sumBytes, nullptr) != 0) { SetLastError(fn + rt_last_error()); return false; }
+		if (rt_copy_to_host(acc->device, sums.data(), acc->sums, sumBytes, nullptr) != 0) return call.Fail(rt_last_error());
 		AccumFileHeader h;
 		memset(&h, 0, sizeof(h));
 		memcpy(h.magic, "RTACCUM1", 8);
@@ -1271,21 +1226,19 @@ namespace RtGpu
 		h.checksum = AccumFileChecksum(h, acc->binding, sums.data(), sumBytes);
 		const std::string tmp = std::string(path) + ".tmp";
 		FILE* f = fopen(tmp.c_str(), "wb");
-		if (!f) { SetLastError(fn + "cannot create " + tmp); return false; }
+		if (!f) return call.Fail("cannot create " + tmp);
 		bool ok = fwrite(&h, 1, sizeof(h), f) == sizeof(h) && fwrite(&acc->binding, 1, sizeof(acc->binding), f) == sizeof(acc->binding) &&
 		          fwrite(sums.data(), 1, (size_t)sumBytes, f) == (size_t)sumBytes;
 		ok = (fclose(f) == 0) && ok;
-		if (!ok || rename(tmp.c_str(), path) != 0) { remove(tmp.c_str()); SetLastError(fn + "write failed: " + path); return false; }
+		if (!ok || rename(tmp.c_str(), path) != 0) { remove(tmp.c_str()); return call.Fail(std::string("write failed: ") + path); }
 		return true;
 	}
 
 	RaylibB200Accumulator* AccumulatorLoad(const char* path)
 	{
-		std::lock_guard<std::recursive_mutex> lock(g_mutex);
-		t_lastError.clear();
-		const std::string fn = std::string("RaylibB200_AccumulatorLoad: ") + (path ? path : "(null)") + ": ";
+		const Call call(std::string("RaylibB200_AccumulatorLoad: ") + (path ? path : "(null)") + ": ");
 		FILE* f = path ? fopen(path, "rb") : nullptr;
-		if (!f) { SetLastError(fn + "cannot open"); return nullptr; }
+		if (!f) { call.Fail("cannot open"); return nullptr; }
 		AccumFileHeader h;
 		RtAccumBinding b;
 		std::vector<float> sums;
@@ -1313,12 +1266,12 @@ namespace RtGpu
 			}
 		}
 		fclose(f);
-		if (!why.empty()) { SetLastError(fn + why); return nullptr; }
-		RaylibB200Accumulator* acc = NewAccumulator(h.width, h.height, fn.c_str());
+		if (!why.empty()) { call.Fail(why); return nullptr; }
+		RaylibB200Accumulator* acc = NewAccumulator(call, h.width, h.height);
 		if (!acc) return nullptr;
 		if (rt_copy_to_device(acc->device, acc->sums, sums.data(), (uint64_t)sums.size() * 4ull, nullptr) != 0)
 		{
-			SetLastError(fn + rt_last_error());
+			call.Fail(rt_last_error());
 			AccumulatorDestroy(acc);
 			return nullptr;
 		}
@@ -1333,11 +1286,7 @@ void RtForgetScene(const Scene* scene)
 {
 	std::lock_guard<std::recursive_mutex> lock(g_mutex);
 	g_prebuilt.erase(scene);
-	for (auto it = g_scenes.begin(); it != g_scenes.end();)
-	{
-		if (it->first.first == scene) { rt_scene_free(it->second.device); it = g_scenes.erase(it); }
-		else ++it;
-	}
+	DropSceneCopies(scene);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1354,7 +1303,10 @@ void Renderer::RenderScene(const RendererSettings* settings, const Scene* world,
 	if (settings->viewportWidth != outImage->GetWidth() || settings->viewportHeight != outImage->GetHeight())
 		outImage->Reallocate(settings->viewportWidth, settings->viewportHeight);
 
-	if (!RtGpu::Render(settings, world, camera, outImage, nullptr, nullptr, 0, 1, 0, nullptr, RtIsLibraryImage(outImage)))
+	RtGpu::FrameTarget target;
+	target.hostImage = outImage;
+	target.pinHostImage = RtIsLibraryImage(outImage);
+	if (!RtGpu::Render(settings, world, camera, target))
 	{
 		LOG("Raylib_Render FAILED: %s", RtGpu::LastError());
 		return;

@@ -35,6 +35,8 @@ namespace RtGpu
 	void SetPipes(uint32_t pipes);
 	void SetFusedPass(uint32_t mode);
 
+	// The message of every call that needs a device when there is none.
+	constexpr const char* kNoDevice = "no CUDA device is available; this library renders on the GPU only (no CPU path)";
 	void SetLastError(const std::string& message);
 	const char* LastError();
 	void SetLastStats(const RaylibB200Stats& stats);
@@ -42,7 +44,6 @@ namespace RtGpu
 
 	// Flatten + upload (once per scene and device). nullptr on failure (LastError says why).
 	const RtDeviceScene* AcquireScene(const Scene* scene, uint64_t* outCounts8 = nullptr);
-	RtRenderContext* AcquireContext();
 	// A scene whose flattened form was read from disk (RaylibB200_LoadFlattenedScene): AcquireScene uploads it as is.
 	void AdoptPrebuilt(const Scene* scene, std::shared_ptr<RtFlatScene> flat);
 	std::shared_ptr<RtFlatScene> Prebuilt(const Scene* scene);
@@ -52,12 +53,21 @@ namespace RtGpu
 	// primary device): rt_render_window of rt_progressive.h.
 	struct SampleWindow { uint32_t begin, end; void* sums; };
 
-	// Shared implementation of every render entry point.  Exactly one of hostImage / deviceImage /
-	// deviceShard / window is non-null.
-	bool Render(const RendererSettings* settings, const Scene* scene, const Camera* camera,
-	            Image2D* hostImage, void* deviceImage, void* deviceShard,
-	            uint32_t shardRank, uint32_t shardCount, uint32_t renderModeOverride, void* stream, bool pinHostImage = false,
-	            const SampleWindow* window = nullptr);
+	// Where Render puts a frame: exactly one of hostImage / deviceImage / deviceShard / window is set.
+	struct FrameTarget
+	{
+		Image2D* hostImage = nullptr;            // the whole frame, read back; pinHostImage page-locks its storage first
+		bool pinHostImage = false;
+		void* deviceImage = nullptr;             // row-major W x H float4 on the primary device
+		void* deviceShard = nullptr;             // tile-major shard buffer
+		uint32_t shardRank = 0, shardCount = 1;  // the tiles deviceImage / deviceShard receive
+		const SampleWindow* window = nullptr;    // added to an accumulator's running sums
+		void* stream = nullptr;                  // cudaStream_t of a one-device frame
+	};
+
+	// Shared implementation of every render entry point.  renderModeOverride != 0 replaces settings->renderMode.
+	bool Render(const RendererSettings* settings, const Scene* scene, const Camera* camera, FrameTarget target,
+	            uint32_t renderModeOverride = 0);
 
 	// Progressive rendering (RaylibB200_Accumulator*, include/raylib_b200.h)
 	RaylibB200Accumulator* AccumulatorCreate(uint32_t width, uint32_t height);
@@ -87,6 +97,8 @@ namespace RtGpu
 	bool Denoise(const Image2D* color, const Image2D* albedo, const Image2D* normal, Image2D* out);
 	bool DenoiseDevice(const void* color, const void* albedo, const void* normal, uint32_t width, uint32_t height, void* out, void* stream);
 
+	// One k_trace_rays launch on caller rays: per ray the leaf rank and t of its closest hit (rt_trace_closest).
+	bool TraceRays(const Scene* scene, const float* rays, int64_t numRays, float tMin, int32_t* outRank, float* outT);
 	// One launch of a traversal stage kernel (k_extend, k_extend_pool, k_shadow) on caller rays in a caller order
 	// (rt_trace_stage of rt_trace_stage.h).  Arguments are checked before a device is used.
 	bool TraceRaysStaged(const Scene* scene, int mode, const float* rays, const uint32_t* order, int64_t numRays, float tMin,

@@ -477,8 +477,11 @@ int32_t RaylibB200_RenderShard(const RendererSettings* settings, SceneHandle sce
 	uint32_t shardRank, uint32_t shardCount, void* deviceShardOut, void* cudaStream)
 {
 	if (!deviceShardOut || shardCount == 0 || shardRank >= shardCount) { RtGpu::SetLastError("RaylibB200_RenderShard: bad shard arguments"); return 0; }
-	return RtGpu::Render(settings, (const Scene*)scene, (const Camera*)camera, nullptr, nullptr, deviceShardOut,
-		shardRank, shardCount, 0, cudaStream) ? 1 : 0;
+	RtGpu::FrameTarget target;
+	target.deviceShard = deviceShardOut;
+	target.shardRank = shardRank; target.shardCount = shardCount;
+	target.stream = cudaStream;
+	return RtGpu::Render(settings, (const Scene*)scene, (const Camera*)camera, target) ? 1 : 0;
 }
 
 // ---- shared frame: every rank renders its tiles straight into one row-major image (no shard buffers, no gather) ----
@@ -486,8 +489,11 @@ int32_t RaylibB200_RenderShardToFrame(const RendererSettings* settings, SceneHan
 	uint32_t shardRank, uint32_t shardCount, void* deviceFrame, void* cudaStream)
 {
 	if (!deviceFrame || shardCount == 0 || shardRank >= shardCount) { RtGpu::SetLastError("RaylibB200_RenderShardToFrame: bad shard arguments"); return 0; }
-	return RtGpu::Render(settings, (const Scene*)scene, (const Camera*)camera, nullptr, deviceFrame, nullptr,
-		shardRank, shardCount, 0, cudaStream) ? 1 : 0;
+	RtGpu::FrameTarget target;
+	target.deviceImage = deviceFrame;
+	target.shardRank = shardRank; target.shardCount = shardCount;
+	target.stream = cudaStream;
+	return RtGpu::Render(settings, (const Scene*)scene, (const Camera*)camera, target) ? 1 : 0;
 }
 
 void* RaylibB200_FrameCreate(uint32_t width, uint32_t height, unsigned char* outIpcHandle64)
@@ -565,7 +571,10 @@ int32_t RaylibB200_RenderToDevice(const RendererSettings* settings, SceneHandle 
 	void* deviceImageOut, void* cudaStream)
 {
 	if (!deviceImageOut) { RtGpu::SetLastError("RaylibB200_RenderToDevice: null output"); return 0; }
-	return RtGpu::Render(settings, (const Scene*)scene, (const Camera*)camera, nullptr, deviceImageOut, nullptr, 0, 1, 0, cudaStream) ? 1 : 0;
+	RtGpu::FrameTarget target;
+	target.deviceImage = deviceImageOut;
+	target.stream = cudaStream;
+	return RtGpu::Render(settings, (const Scene*)scene, (const Camera*)camera, target) ? 1 : 0;
 }
 
 int32_t RaylibB200_RenderAux(const RendererSettings* settings, SceneHandle scene, CameraHandle camera,
@@ -600,7 +609,7 @@ int32_t RaylibB200_ImageGetRGBA(ImageHandle imageHandle, float* outRgba)
 int32_t RaylibB200_LibmEval(int32_t fn, const float* x, const float* y, float* out, uint64_t count)
 {
 	if (!x || !out || fn < 0 || fn > 9) { RtGpu::SetLastError("RaylibB200_LibmEval: bad arguments"); return 0; }
-	if (RtGpu::DeviceCount() <= 0) { RtGpu::SetLastError("no CUDA device is available; this library renders on the GPU only (no CPU path)"); return 0; }
+	if (RtGpu::DeviceCount() <= 0) { RtGpu::SetLastError(RtGpu::kNoDevice); return 0; }
 	if (rt_libm_eval(RtGpu::CurrentDevice(), fn, x, y, out, count) != 0) { RtGpu::SetLastError(std::string("rt_libm_eval: ") + rt_last_error()); return 0; }
 	return 1;
 }
@@ -619,23 +628,7 @@ int32_t RaylibB200_DenoiseDevice(const void* color, const void* albedo, const vo
 
 int32_t RaylibB200_TraceRays(SceneHandle scene, const float* rays, int64_t numRays, float tMin, int32_t* outRank, float* outT)
 {
-	const RtDeviceScene* ds = RtGpu::AcquireScene((const Scene*)scene);
-	RtRenderContext* ctx = ds ? RtGpu::AcquireContext() : nullptr;
-	if (!ds || !ctx) return 0;
-	RtRenderStats rs;
-	if (rt_trace_closest(ctx, ds, rays, numRays, tMin, outRank, outT, &rs) != 0)
-	{
-		RtGpu::SetLastError(std::string("rt_trace_closest: ") + rt_last_error());
-		return 0;
-	}
-	RaylibB200Stats st;
-	memset(&st, 0, sizeof(st));
-	st.rayQueries = rs.rayQueries; st.boxTests = rs.boxTests; st.triTests = rs.triTests; st.sphereTests = rs.sphereTests;
-	st.nodeVisits = rs.nodeVisits; st.deviceMs = rs.deviceMs; st.kernelLaunches = 1;
-	st.gateTests = rs.gateTests; st.cubeTests = rs.cubeTests;
-	st.refBoxTests = rs.refBoxTests; st.refTriTests = rs.refTriTests; st.refSphereTests = rs.refSphereTests; st.statRays = rs.statRays;
-	RtGpu::SetLastStats(st);
-	return 1;
+	return RtGpu::TraceRays((const Scene*)scene, rays, numRays, tMin, outRank, outT) ? 1 : 0;
 }
 
 int32_t RaylibB200_TraceRaysStaged(SceneHandle scene, int32_t mode, const float* rays, const uint32_t* order, int64_t numRays,
@@ -652,8 +645,10 @@ int32_t RaylibB200_PrimaryHits(const RendererSettings* settings, SceneHandle sce
 	if (!settings || !outRank || !outT) { RtGpu::SetLastError("RaylibB200_PrimaryHits: null argument"); return 0; }
 	const size_t n = (size_t)settings->viewportWidth * settings->viewportHeight;
 	Image2D scratch(settings->viewportWidth, settings->viewportHeight, 0x0);
+	RtGpu::FrameTarget target;
+	target.hostImage = &scratch;
 	// internal render mode 100: pixel = (t, bit pattern of the leaf rank, bu, bv)
-	if (!RtGpu::Render(settings, (const Scene*)scene, (const Camera*)camera, &scratch, nullptr, nullptr, 0, 1, 100u, nullptr)) return 0;
+	if (!RtGpu::Render(settings, (const Scene*)scene, (const Camera*)camera, target, 100u)) return 0;
 	const std::vector<Pixel>& px = scratch.GetPixelArray();
 	for (size_t i = 0; i < n; ++i)
 	{

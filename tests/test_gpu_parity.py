@@ -165,8 +165,9 @@ def test_reference_work_counters_match_oracle(gpu):
         info = gpu.create_demo(cfg, int(g["size"]))
         try:
             # plain uploads leave the reference topology on the host: without statistics the counters stay zero ...
+            gpu.lib.RaylibB200_SetDevice(-1)                # a refused call leaves a message; a successful query clears it
             gpu.trace_rays(info.scene, g["rays"], info.settings.rayTMin)
-            assert gpu.last_stats().refBoxTests == 0
+            assert gpu.last_stats().refBoxTests == 0 and gpu.last_error() == ""
             # ... and asking for statistics uploads the scene again, with it
             gpu.lib.RaylibB200_SetCollectStats(1)
             gpu.trace_rays(info.scene, g["rays"], info.settings.rayTMin)
